@@ -9,7 +9,8 @@ One "step" = one pass of pileup -> candidate select -> window gather -> PileupMo
   N > 1   BASELINE.json configs[3]: the whole-genome-shaped 3.1 Gb input (chr1-22,X,Y,M lengths) at 30x, cut into regions
           with 16-bp halos, LPT-assigned to the N GPUs (STRONG scaling, the north-star split), through the product's
           sharded path; a weak-scaling line (one 100 Mb contig per rank) is reported as the secondary key "weak"
-  value  device-resident inputs, CUDA-event timed, max over ranks
+  value  device-resident inputs, CUDA-event timed, max over ranks; --dump-outputs DIR writes what the last timed step
+         returned (see dump_outputs) so that two builds can be compared on the same seeded inputs
   e2e    same work through the host-buffer API: pinned host arrays -> H2D -> kernels -> VCF text on the GPU -> D2H of the
          text (N > 1: every rank writes its segments of ONE ordered VCF file; only counts / batch heads are all-reduced)
 """
@@ -50,6 +51,8 @@ def parse_args():
     ap.add_argument("--no-selfcheck", action="store_true")
     ap.add_argument("--no-fast-mode", action="store_true", help="skip the secondary NSNP_PREC_F16X1 measurement")
     ap.add_argument("--write-vcf", action="store_true", help="N > 1: also place the text segments into ONE file on /dev/shm inside the timed region")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned (rank 0's regions) as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -196,6 +199,29 @@ def region_slices(reads, regions, cfg, dev, alg):
     return out
 
 
+DUMP_SITES = 1 << 16             # sites sampled by --dump-outputs: ~15 MB of .npy files
+
+
+def dump_outputs(out_dir, outputs):
+    """--dump-outputs: what RegionRunner.run_device returned to the caller in the last timed step, for comparing two builds
+    output for output.  outputs: [(pos0, gt, zy, rec)] per region, in region order.  Writes region_sites (site count of
+    every region) and, for a sample of DUMP_SITES sites drawn with a fixed seed from the concatenation of all regions,
+    site_index (index into that concatenation), pos0 (0-based contig position), gt [k,21] and zy [k,3] (probabilities)
+    and records [k,32] (the bytes of the compact site records).  Integers are stored exactly as float64 / float32."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    pos0, gt, zy, rec = (torch.cat([o[i] for o in outputs]) for i in range(4))
+    n = pos0.shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(n, min(n, DUMP_SITES), replace=False))
+    ti = torch.from_numpy(idx).to(pos0.device)
+    arrays = {"region_sites": np.array([o[0].shape[0] for o in outputs], np.float64), "site_index": idx.astype(np.float64),
+              "pos0": pos0[ti].cpu().numpy().astype(np.float64), "gt": gt[ti].cpu().numpy(), "zy": zy[ti].cpu().numpy(),
+              "records": rec[ti].cpu().numpy().astype(np.float32)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main_ours(args):
     import ctypes as C
     import hashlib
@@ -252,12 +278,17 @@ def main_ours(args):
         rd = cigar16(rd)                                       # host hand-off ships uint16 CIGAR words (every length < 4096 here)
         return PackedReads(*[None if getattr(rd, f) is None else getattr(rd, f).cpu().pin_memory() for f in FIELDS])
 
-    def time_device(work, steps, timer=None, profile=False):
-        """work: [(Region, device reads, device ref)].  Returns (ms_total, sites of one step, t_begin, t_end)."""
-        def step(tm=None):
+    def time_device(work, steps, timer=None, profile=False, keep=None):
+        """work: [(Region, device reads, device ref)].  Returns (ms_total, sites of one step, t_begin, t_end).
+        keep: a list that receives device copies of (pos0, gt, zy, rec) of every region of the last timed step (the runner
+        reuses its buffers from region to region)."""
+        def step(tm=None, keep=None):
             n = 0
             for rg, rd, rf in work:
-                n += runner.run_device(rd, rf, rg, tm).n
+                o = runner.run_device(rd, rf, rg, tm)
+                n += o.n
+                if keep is not None:
+                    keep.append((o.pos0.clone(), o.gt.clone(), o.zy.clone(), o.rec.clone()))
             return n
         for _ in range(W):
             n_sites = step()
@@ -268,8 +299,8 @@ def main_ours(args):
         barrier()
         t_begin = time.time()
         e0.record()
-        for _ in range(steps):
-            n_sites = step(timer)
+        for i in range(steps):
+            n_sites = step(timer, keep if i == steps - 1 else None)
         e1.record()
         barrier()
         return e0.elapsed_time(e1), n_sites, t_begin, time.time()
@@ -301,7 +332,7 @@ def main_ours(args):
     sampler.start()
 
     # ================================================================ one 100 Mb contig per rank (N = 1 headline; N > 1: "weak")
-    def contig_workload(steps, with_e2e, with_selfcheck, alg_acc):
+    def contig_workload(steps, with_e2e, with_selfcheck, alg_acc, keep=None):
         L = int(args.contig_mb * 1e6)
         cfg = synth_cfg(args, rank, L)
         ref, reads = generate_device(cfg, dev)
@@ -311,7 +342,7 @@ def main_ours(args):
         torch.cuda.empty_cache()
         work = [(rg, rd, ref) for rg, rd in zip(regions, dev_regions)]
         timer = StageTimer(True)
-        ms_total, n_sites, t_begin, t_end = time_device(work, steps, timer, profile=True)
+        ms_total, n_sites, t_begin, t_end = time_device(work, steps, timer, profile=True, keep=keep)
         res = {"cfg": cfg, "regions": regions, "ms_total": ms_total, "n_sites": n_sites, "t": (t_begin, t_end), "timer": timer, "e2e": None}
         kms = (C.c_double * len(_lib.PROF_SLOTS))(); kln = (C.c_int64 * len(_lib.PROF_SLOTS))()
         _lib.check(lib.nsnp_profile_read(kms, kln))
@@ -417,7 +448,7 @@ def main_ours(args):
         return res
 
     # ================================================================ genome-shaped strong scaling (N > 1)
-    def genome_workload(steps):
+    def genome_workload(steps, keep=None):
         contigs = [(n, max(2000, int(L * args.genome_scale))) for n, L in GRCH38]
         regions = plan_regions(contigs, int(args.region_mb * 1e6))
         mine = assign_lpt(regions, world)[rank]
@@ -435,7 +466,7 @@ def main_ours(args):
         torch.cuda.synchronize()
         t_gen = time.perf_counter() - t_gen
         timer = StageTimer(True)
-        ms_total, n_sites, t_begin, t_end = time_device(work, steps, timer, profile=True)
+        ms_total, n_sites, t_begin, t_end = time_device(work, steps, timer, profile=True, keep=keep)
         kms = (C.c_double * len(_lib.PROF_SLOTS))(); kln = (C.c_int64 * len(_lib.PROF_SLOTS))()
         _lib.check(lib.nsnp_profile_read(kms, kln))
         lib.nsnp_profile_enable(0)
@@ -470,12 +501,16 @@ def main_ours(args):
                 os.unlink(out_path)
         return res
 
+    outputs = [] if args.dump_outputs and rank == 0 else None
     if world == 1:
-        main_res = contig_workload(K, not args.no_e2e, not args.no_selfcheck and not args.no_e2e, alg)
+        main_res = contig_workload(K, not args.no_e2e, not args.no_selfcheck and not args.no_e2e, alg, keep=outputs)
         scaling = "weak"
     else:
-        main_res = genome_workload(K)
+        main_res = genome_workload(K, keep=outputs)
         scaling = "strong"
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
+        del outputs
     clocks = sampler.stop(*main_res["t"])
     if world > 1 and not args.no_weak:
         wk = contig_workload(max(1, min(K, 2)), not args.no_e2e, False, {"pileup": 0.0, "n_bases": 0, "n_cigar": 0, "n_reads": 0})

@@ -3,21 +3,17 @@
   * our PredictDataset('.pd') through DataLoader(batch_size=1000, shuffle=False, num_workers=0 / 4) collates to the 4-tuple
     PileupModel/predict.py:45-49 unpacks (tuple[str], LongTensor[N], LongTensor[N], IntTensor[N,33,18]) with the reference's
     batch boundaries;
-  * (build container only) the REFERENCE's predict.predict runs unmodified with `predict.PredictDataset` replaced by ours, a
-    `.pd.bin` path (predict.py:215 lists *.bin) resolved through the `.pd` text, and a stub model returning the golden
-    probabilities: the VCF is byte-equal to the golden file the all-reference run produced.
+  * the predict loop (restated in oracle/s2_restate.py, pinned to the reference Python by tests/test_oracle_pinning.py) over
+    the `.pd.bin` path predict.py:215 lists, resolved through the `.pd` text, with our PredictDataset and a stub model
+    returning the golden probabilities: the VCF is byte-equal to the golden file the all-reference run produced.
 """
 import os
 import sys
-import types
-from pathlib import Path
 
 import numpy as np
 import pytest
 
 from conftest import GOLDEN
-
-REF = Path("/root/reference/PileupModel")
 
 
 @pytest.fixture()
@@ -53,41 +49,22 @@ def test_dataset_collates_like_the_reference(pd_dir, small_case, workers):
     assert seen == n
 
 
-@pytest.mark.skipif(not REF.exists(), reason="the reference checkout is only present in the build container")
-def test_reference_predict_loop_with_our_dataset(pd_dir, tmp_path):
+def test_reference_predict_loop_with_our_dataset(pd_dir, monkeypatch):
     import torch
-    for name, body in (("ranger", {"Ranger": type("Ranger", (), {})}),
-                       ("tables", None)):
-        if body is not None:
-            m = types.ModuleType(name); m.__dict__.update(body); sys.modules[name] = m
-    tb = types.ModuleType("tables"); tb.Filters = type("Filters", (), {"__init__": lambda self, *a, **k: None})
-    sys.modules["tables"] = tb                                  # only so that the reference's dataset.py imports
-    sys.path.insert(0, str(REF))
-    try:
-        import predict as ref_predict
-        from nanosnp_b200 import dataset as ours
-        real_tables = sys.modules.pop("tables")                 # our PredictDataset must take its no-PyTables route
-        sys.modules["tables"] = None
-        ref_predict.PredictDataset = ours.PredictDataset        # the one-line swap of INTEGRATION.md option 2
-        z = np.load(GOLDEN / "s2_small.npz")
-
-        class GoldenModel:                                      # stands in for LSTMNetwork: returns the reference's own probabilities
-            def __init__(self):
-                self.k = 0
-            def eval(self):
-                return self
-            def predict(self, x):
-                n = x.shape[0]
-                assert x.dtype == torch.float32 and tuple(x.shape[1:]) == (33, 18)
-                g, y = z["gt"][self.k:self.k + n], z["zy"][self.k:self.k + n]
-                self.k += n
-                return torch.from_numpy(g), torch.from_numpy(y)
-
-        out = str(tmp_path / "swap.vcf")
-        paths = [str(pd_dir / "bin_predict_data" / f) for f in os.listdir(pd_dir / "bin_predict_data") if f.endswith(".bin")]   # predict.py:215
-        ref_predict.predict(GoldenModel(), paths, str(GOLDEN / "s2_small.fai"), 1000, out, torch.device("cpu"))
-        assert open(out, "rb").read() == (GOLDEN / "s2_small.vcf").read_bytes()
-    finally:
-        sys.path.remove(str(REF))
-        for mod in ("predict", "model", "dataset", "options", "utils", "optim", "tables", "ranger"):
-            sys.modules.pop(mod, None)
+    from torch.utils.data import DataLoader
+    from nanosnp_b200.dataset import PredictDataset
+    from oracle.s2_restate import vcf_header, vcf_records
+    monkeypatch.setitem(sys.modules, "tables", None)            # our PredictDataset must take its no-PyTables route
+    z = np.load(GOLDEN / "s2_small.npz")
+    text = vcf_header((GOLDEN / "s2_small.fai").read_text().splitlines())           # predict.py:13-27
+    k = 0
+    paths = [str(pd_dir / "bin_predict_data" / f) for f in os.listdir(pd_dir / "bin_predict_data") if f.endswith(".bin")]   # predict.py:215
+    for path in paths:
+        for names, pos, refb, x in DataLoader(PredictDataset(path), batch_size=1000, shuffle=False):       # predict.py:43-45
+            x = x.type(torch.FloatTensor)                                                               # predict.py:49
+            n = x.shape[0]
+            assert x.dtype == torch.float32 and tuple(x.shape[1:]) == (33, 18)
+            text += vcf_records(names, pos.numpy(), refb.numpy(), x.numpy(), z["gt"][k:k + n], z["zy"][k:k + n])
+            k += n
+    assert k == len(z["gt"])
+    assert text.encode() == (GOLDEN / "s2_small.vcf").read_bytes()
