@@ -31,7 +31,7 @@ extern "C" {
 #define NSNP_E_INVALID       -1   /* bad argument (null pointer, negative size, unsorted reads ...) */
 #define NSNP_E_CUDA          -2   /* a CUDA runtime call failed; see nsnp_last_error() */
 #define NSNP_E_WORKSPACE     -3   /* caller workspace too small */
-#define NSNP_E_OVERFLOW      -4   /* a device-side capacity was exceeded (> 16383 reads over one 1024-bp tile, indel slab full) */
+#define NSNP_E_OVERFLOW      -4   /* a device-side capacity was exceeded (> 16383 reads over one 1024-bp tile, candidate buffer) */
 #define NSNP_E_NO_DEVICE     -5   /* no CUDA device: there is deliberately no CPU fallback */
 #define NSNP_E_UNSUPPORTED   -6   /* e.g. a CIGAR with P pads or unmerged adjacent I I / D D ops (nsnp_bam_fill merges them) */
 

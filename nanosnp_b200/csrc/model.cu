@@ -247,23 +247,35 @@ static const int64_t kChunkSites = [] { const char* v = getenv("NSNP_CHUNK_WAVES
 // enough to flip an argmax only where the two best classes of a head are closer than that.  Every site whose top-2 margin is
 // below kX1Margin in EITHER head is therefore run again through the three-pass path (its result replaces the single-pass
 // one), so genotype / zygosity calls are those of NSNP_PREC_F16X3; the other sites keep probabilities within the stated 5e-3.
+// That error bound holds for ordinary counts.  The single pass drops the low bits of a count above 2048 (fp16 holds every
+// integer up to 2048), and the errors grow with the counts: deep windows (chrM, collapsed repeats) reach |dp| ~ 1e-2 without a
+// flip.  Sites whose window holds such a count are re-evaluated as well.
 constexpr float kX1Margin = 0.02f;           // > 6x the largest single-pass error observed
+constexpr float kX1ExactCount = 2048.f;
 constexpr int kX1Cap = 4096;                 // re-evaluated sites per call (expected: ~0.07 % of the sites); beyond it
                                              // nsnp_model_f16x1_reevaluated reports the overflow
 struct X1Work { int32_t* cnt; int32_t* idx; int32_t* pos_low; float* gt_low; float* zy_low; int32_t* x_low; };
 constexpr size_t kX1FixedBytes = 256 + (size_t)kX1Cap * (4 + 4 + 24 * 4);
 constexpr size_t kX1WindowBytes = (size_t)kX1Cap * kT * kF * 4;
 
+// one warp per site: the lanes scan the site's window (int32 or float32 rows, or its row span of the count tensor when pos is given)
 __global__ void x1_margin_kernel(const float* __restrict__ gt, const float* __restrict__ zy, int64_t n, const int32_t* __restrict__ n_dev,
-                                 float tau, int32_t* __restrict__ cnt, int32_t* __restrict__ idx)
+                                 float tau, const int32_t* __restrict__ x, const float* __restrict__ xf, const int32_t* __restrict__ pos,
+                                 int64_t pos_bias, int32_t* __restrict__ cnt, int32_t* __restrict__ idx)
 {
-    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n || (n_dev && i >= *n_dev)) return;
+    const int64_t i = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (i >= n || (n_dev && i >= *n_dev)) return;           // warp-uniform
+    const int64_t w0 = pos ? ((int64_t)pos[i] - pos_bias) * kF : i * kT * kF;
+    bool deep = false;
+    for (int j = lane; j < kT * kF; j += 32) deep |= !(fabsf(x ? (float)x[w0 + j] : xf[w0 + j]) <= kX1ExactCount);
+    deep = __any_sync(0xffffffffu, deep);
+    if (lane != 0) return;
     float a = -1.f, b = -1.f;
     for (int k = 0; k < 21; ++k) { const float v = gt[i * 21 + k]; if (v > a) { b = a; a = v; } else if (v > b) b = v; }
     float c = -1.f, d = -1.f;
     for (int k = 0; k < 3; ++k) { const float v = zy[i * 3 + k]; if (v > c) { d = c; c = v; } else if (v > d) d = v; }
-    if (!(a - b >= tau) || !(c - d >= tau)) {                 // also catches NaN
+    if (deep || !(a - b >= tau) || !(c - d >= tau)) {         // also catches NaN
         const int k = atomicAdd(cnt, 1);
         if (k < kX1Cap) idx[k] = (int32_t)i;
     }
@@ -465,7 +477,8 @@ static int model_forward(const void* blob_dev, const int32_t* x_i32_dev, const f
     if (x1) {
         // low-margin sites -> one three-pass batch of kX1Cap sites (layer-0 buffer and h16 of the main pass are free again)
         const X1Work w = x1_carve(workspace_dev, n);
-        x1_margin_kernel<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(gt_prob_dev, zy_prob_dev, n, n <= ch ? n_dev : nullptr, kX1Margin, w.cnt, w.idx);
+        x1_margin_kernel<<<(unsigned)((n + 7) / 8), 256, 0, stream>>>(gt_prob_dev, zy_prob_dev, n, n <= ch ? n_dev : nullptr, kX1Margin,
+                                                                     x_i32_dev, x_f32_dev, pos_dev, pos_bias, w.cnt, w.idx);
         x1_gather_kernel<<<kX1Cap, 128, 0, stream>>>(w.cnt, w.idx, pos_dev, pos_dev ? nullptr : x_i32_dev, x_f32_dev, w.pos_low, w.x_low);
         if (int e = cuda_status("x1 margin / gather kernels")) return e;
         const int32_t* xi_low = pos_dev ? x_i32_dev : (x_i32_dev ? w.x_low : nullptr);

@@ -16,6 +16,7 @@
 //       - epilogue: prefix sums -> 18 channels + AF gate (IEEE double, tensor_maker.cpp:195-228)
 //         -> rows staged in shared memory -> coalesced 16-byte stores of the int32 [T][18] block.
 #include <stdlib.h>
+#include <type_traits>
 #include "common.cuh"
 
 namespace nsnp {
@@ -246,7 +247,7 @@ struct TileSmem {
     int32_t  thr_snp[kGateTab], thr_indel[kGateTab];   // smallest count c with (double)c / den >= min_af
     int32_t  rlist[T];                                  // >= kReadList; reused as per-warp walk lists (T / warps each)
     int32_t  warp_tot[T / 128][4];
-    int32_t  n_rlist, next_task, n_events, tile, ref_has_x;
+    int32_t  n_rlist, next_task, n_events, tile, ref_has_x, sub_end;
 };
 
 struct ReadMeta { int32_t rpos; int32_t rend; int32_t strand; int64_t c0, c1, sbase; };
@@ -259,9 +260,11 @@ __device__ __forceinline__ ReadMeta load_meta(const nsnp_reads_t& rd, const Work
 
 // All coordinates are 32-bit: contig positions are int32 (BAM), query offsets are < 2^31; only the absolute base index
 // of the packed sequence array needs 64 bits (added last).
-template <int T>
+// kEvOnly: the re-walk of a tile whose indel events overflowed the slab (see pileup_tile_kernel): only the chained events
+// anchored in [elo, ehi) are recorded, no counter is touched.  The first walk passes elo = ts, ehi = te.
+template <int T, bool kEvOnly>
 __device__ __forceinline__ void process_read(TileSmem<T>& sm, const nsnp_reads_t& rd, const Workspace& ws, Event* slab,
-                                             int r, const ReadMeta& meta, int ts, int te, bool deep, int32_t* status)
+                                             int r, const ReadMeta& meta, int ts, int te, int elo, int ehi, bool deep, int32_t* status)
 {
     const int lane = lane_id();
     const int rpos = meta.rpos;
@@ -275,15 +278,15 @@ __device__ __forceinline__ void process_read(TileSmem<T>& sm, const nsnp_reads_t
     const int32_t* ckq = ws.ck_q + ((c0 >> kCkShift) + r);
     // the read's reference span [rpos, rend): two boundary increments per read and tile.  Aligned depth = span depth
     // minus deletion depth (minus reference skips, which close and reopen the span below): prefix sums in the epilogue.
-    if (lane == 0) atomicAdd(&sm.ms[max(rpos - ts, 0)], sinc);
-    if (lane == 1 && meta.rend < te) atomicSub(&sm.ms[meta.rend - ts], sinc);
-    // last chunk whose first op starts at or before the tile start (32-ary search over the checkpoints)
+    if (!kEvOnly && lane == 0) atomicAdd(&sm.ms[max(rpos - ts, 0)], sinc);
+    if (!kEvOnly && lane == 1 && meta.rend < te) atomicSub(&sm.ms[meta.rend - ts], sinc);
+    // last chunk whose first op starts at or before the window start (32-ary search over the checkpoints)
     int lo = 0, hi = nchunks;
-    if (rpos < ts) {
+    if (rpos < elo) {
         while (hi - lo > 1) {
             const int step = (hi - lo + 31) >> 5;
             const int c = lo + lane * step;
-            const bool le = c < hi && __ldg(ckr + c) <= ts;
+            const bool le = c < hi && __ldg(ckr + c) <= elo;
             const int cnt = __popc(__ballot_sync(0xffffffffu, le));      // monotone: lanes 0..cnt-1 are true, cnt >= 1
             lo = lo + (cnt - 1) * step;
             hi = min(hi, lo + step);
@@ -297,7 +300,7 @@ __device__ __forceinline__ void process_read(TileSmem<T>& sm, const nsnp_reads_t
     int64_t cgp = c0 + ((int64_t)chunk << kCkShift);
     int left = (int)(c1 - c0) - (chunk << kCkShift);                             // ops from this chunk to the end of the read
     uint32_t cg_next = lane < left ? ld_cigar(rd, cgp + lane) : 6u;               // software-pipelined CIGAR loads
-    for (; left > 0 && R <= te; left -= 32, cgp += 32) {
+    for (; left > 0 && R <= ehi; left -= 32, cgp += 32) {
         const uint32_t cg = cg_next;
         cg_next = (32 + lane < left) ? ld_cigar(rd, cgp + 32 + lane) : 6u;
         const int op = cg & 15, len = cg >> 4;                          // 6 = pad: consumes nothing
@@ -323,14 +326,14 @@ __device__ __forceinline__ void process_read(TileSmem<T>& sm, const nsnp_reads_t
         // have their own byte counters; everything else is chained per position and grouped exactly in the epilogue.
         const int anchor = rs - 1;
         const bool isins = op == 1;
-        const bool ev = (isins || isdel) && len <= NSNP_MAX_INDEL && rs > rpos && anchor >= ts && anchor < te;
+        const bool ev = (isins || isdel) && len <= NSNP_MAX_INDEL && rs > rpos && anchor >= elo && anchor < ehi;
         const int64_t gq = sbase + qs;                                   // absolute base index of an inserted sequence
         const bool ins1 = ev && isins && len == 1 && !deep;
         // '*' / '#' depth: a counted 1- or 2-base deletion anchored inside the tile is covered by its fast counter (the
         // epilogue adds D1[p-1] + D2[p-1] + D2[p-2]); every other deletion -- longer, leading, anchored in the previous
         // tile, or any in a deep tile -- marks its clipped span with two boundary deltas
         const bool fastdel = ev && isdel && len <= 2 && !deep;
-        if (isdel && a < b && !fastdel) {
+        if (!kEvOnly && isdel && a < b && !fastdel) {
             atomicAdd(&sm.ds[a - ts], sinc);
             if (b < te) atomicSub(&sm.ds[b - ts], sinc);
         }
@@ -339,9 +342,9 @@ __device__ __forceinline__ void process_read(TileSmem<T>& sm, const nsnp_reads_t
         if (ev) {
             const int cls = (isdel ? 2 : 0) + strand;
             const int ap = anchor - ts;
-            atomicAdd(&sm.cnt4[ap], 1u << (8 * cls));
+            if (!kEvOnly) atomicAdd(&sm.cnt4[ap], deep ? 1u : 1u << (8 * cls));
             if (fastdel) {
-                atomicAdd(&sm.dfast[ap], 1u << (8 * (2 * strand + len - 1)));
+                if (!kEvOnly) atomicAdd(&sm.dfast[ap], 1u << (8 * (2 * strand + len - 1)));
             } else if (!ins1) {
                 const int e = atomicAdd(&sm.n_events, 1);
                 if (e < ws.slab_cap) {
@@ -350,12 +353,12 @@ __device__ __forceinline__ void process_read(TileSmem<T>& sm, const nsnp_reads_t
                     evr.info = (uint32_t)len | ((uint32_t)cls << 8);
                     evr.seq = (uint64_t)gq;
                     slab[e] = evr;
-                } else {
+                } else if (kEvOnly) {
                     dev_fail(status, DEV_E_INDEL_SLAB, sm.tile);
                 }
             }
         }
-        if (op == 3 && a < b) {                                          // reference skip: covered, nothing counted
+        if (!kEvOnly && op == 3 && a < b) {                                          // reference skip: covered, nothing counted
             atomicSub(&sm.ms[a - ts], sinc);                             // close the span over the skip, reopen after it
             if (b < te) atomicAdd(&sm.ms[b - ts], sinc);
             for (int p = a; p < b; ++p) atomicOr(&sm.skipcov[(p - ts) >> 5], 1u << ((p - ts) & 31));
@@ -363,7 +366,7 @@ __device__ __forceinline__ void process_read(TileSmem<T>& sm, const nsnp_reads_t
 
         // ---- phase 2: mismatch detection, one lane per 16-base word of any aligned run of this chunk.  The words of
         //      all 32 ops are flattened (warp scan) so long runs do not leave the other lanes idle. ----
-        const int n = (aligned && a < b) ? (b - a) : 0;
+        const int n = (!kEvOnly && aligned && a < b) ? (b - a) : 0;
         const int nw = (n + 15) >> 4;
         const int winc = warp_incl_scan(nw);
         const int W = __shfl_sync(0xffffffffu, winc, 31);
@@ -407,7 +410,7 @@ __device__ __forceinline__ void process_read(TileSmem<T>& sm, const nsnp_reads_t
         }
         if (ins1) {                                                      // 1-base insertion: fast counter, or the chain when the base is N
             if (!inbit) {
-                atomicAdd(&sm.ifast[strand][anchor - ts], 1u << (8 * ((iword >> (2 * (int)(gq & 15))) & 3u)));
+                if (!kEvOnly) atomicAdd(&sm.ifast[strand][anchor - ts], 1u << (8 * ((iword >> (2 * (int)(gq & 15))) & 3u)));
             } else {
                 const int e = atomicAdd(&sm.n_events, 1);
                 if (e < ws.slab_cap) {
@@ -416,7 +419,7 @@ __device__ __forceinline__ void process_read(TileSmem<T>& sm, const nsnp_reads_t
                     evr.info = 1u | ((uint32_t)strand << 8);
                     evr.seq = (uint64_t)gq;
                     slab[e] = evr;
-                } else {
+                } else if (kEvOnly) {
                     dev_fail(status, DEV_E_INDEL_SLAB, sm.tile);
                 }
             }
@@ -459,9 +462,9 @@ __device__ __forceinline__ void count_mismatches(TileSmem<T>& sm, uint32_t* __re
     }
 }
 
-template <int T>
+template <int T, bool kEvOnly>
 __device__ __forceinline__ void process_read2(TileSmem<T>& sm, const nsnp_reads_t& rd, const Workspace& ws, Event* slab,
-                                              int r, const ReadMeta& meta, int ts, int te, bool deep, int32_t* status)
+                                              int r, const ReadMeta& meta, int ts, int te, int elo, int ehi, bool deep, int32_t* status)
 {
     const int lane = lane_id();
     const int rpos = meta.rpos;
@@ -472,14 +475,14 @@ __device__ __forceinline__ void process_read2(TileSmem<T>& sm, const nsnp_reads_
     const bool ref_has_x = sm.ref_has_x != 0;                       // tile-uniform
     const int32_t* ckr = ws.ck_ref + ((meta.c0 >> kCkShift) + r);
     const int32_t* ckq = ws.ck_q + ((meta.c0 >> kCkShift) + r);
-    if (lane == 0) atomicAdd(&sm.ms[max(rpos - ts, 0)], sinc);
-    if (lane == 1 && meta.rend < te) atomicSub(&sm.ms[meta.rend - ts], sinc);
+    if (!kEvOnly && lane == 0) atomicAdd(&sm.ms[max(rpos - ts, 0)], sinc);
+    if (!kEvOnly && lane == 1 && meta.rend < te) atomicSub(&sm.ms[meta.rend - ts], sinc);
     int lo = 0, hi = nchunks;
-    if (rpos < ts) {
+    if (rpos < elo) {
         while (hi - lo > 1) {
             const int step = (hi - lo + 31) >> 5;
             const int c = lo + lane * step;
-            const bool le = c < hi && __ldg(ckr + c) <= ts;
+            const bool le = c < hi && __ldg(ckr + c) <= elo;
             const int cnt = __popc(__ballot_sync(0xffffffffu, le));
             lo = lo + (cnt - 1) * step;
             hi = min(hi, lo + step);
@@ -498,7 +501,7 @@ __device__ __forceinline__ void process_read2(TileSmem<T>& sm, const nsnp_reads_
     int left = n_ops - (chunk << kCkShift);
     uint32_t nx0 = 2 * lane < left ? ld_cigar(rd, cgp + 2 * lane) : 6u;
     uint32_t nx1 = 2 * lane + 1 < left ? ld_cigar(rd, cgp + 2 * lane + 1) : 6u;
-    for (; left > 0 && R <= te; left -= 64, cgp += 64) {
+    for (; left > 0 && R <= ehi; left -= 64, cgp += 64) {
         const uint32_t cgv[2] = {nx0, nx1};
         nx0 = (64 + 2 * lane < left) ? ld_cigar(rd, cgp + 64 + 2 * lane) : 6u;
         nx1 = (65 + 2 * lane < left) ? ld_cigar(rd, cgp + 65 + 2 * lane) : 6u;
@@ -523,7 +526,7 @@ __device__ __forceinline__ void process_read2(TileSmem<T>& sm, const nsnp_reads_
             const int op = cgv[s] & 15, len = cgv[s] >> 4, rs = rsv[s], qs = qsv[s];
             const int a = max(rs, ts), b = min(rs + len, te);                 // clipped reference span
             // ---- aligned run: bit-parallel mismatch detection, this lane's own run, 16 bases per step ----
-            const int n = (((kAlnOps >> op) & 1u) && a < b) ? (b - a) : 0;
+            const int n = (!kEvOnly && ((kAlnOps >> op) & 1u) && a < b) ? (b - a) : 0;
             const int pa = a - ts;
             const int qa = qs + (a - rs) + sb_lo;                            // offset (bases) from the read's first seq word
             if (n > 0) {
@@ -555,19 +558,20 @@ __device__ __forceinline__ void process_read2(TileSmem<T>& sm, const nsnp_reads_
             const bool isins = op == 1, isdel = op == 2;
             if (isins || isdel) {
                 const int anchor = rs - 1;
-                const bool ev = len <= NSNP_MAX_INDEL && rs > rpos && anchor >= ts && anchor < te;
+                const bool ev = len <= NSNP_MAX_INDEL && rs > rpos && anchor >= elo && anchor < ehi;
                 const bool fastdel = ev && isdel && len <= 2 && !deep;
-                if (isdel && a < b && !fastdel) {
+                if (!kEvOnly && isdel && a < b && !fastdel) {
                     atomicAdd(&sm.ds[a - ts], sinc);
                     if (b < te) atomicSub(&sm.ds[b - ts], sinc);
                 }
                 if (ev) {
                     const int cls = (isdel ? 2 : 0) + strand;
                     const int ap = anchor - ts;
-                    atomicAdd(&sm.cnt4[ap], 1u << (8 * cls));
+                    // deep tiles count chained events per position in the whole word (the classes come from the chain walk)
+                    if (!kEvOnly) atomicAdd(&sm.cnt4[ap], deep ? 1u : 1u << (8 * cls));
                     bool chain = true;
                     if (fastdel) {
-                        atomicAdd(&sm.dfast[ap], 1u << (8 * (2 * strand + len - 1)));
+                        if (!kEvOnly) atomicAdd(&sm.dfast[ap], 1u << (8 * (2 * strand + len - 1)));
                         chain = false;
                     } else if (isins && len == 1 && !deep) {                  // 1-base insertion: fast counter unless the base is N
                         const int qi1 = qs + sb_lo;
@@ -575,7 +579,7 @@ __device__ __forceinline__ void process_read2(TileSmem<T>& sm, const nsnp_reads_
                         const int qn = qs + nb_lo;
                         const uint32_t inbit = nmr ? (__ldg(nmr + (qn >> 5)) >> (qn & 31)) & 1u : 0u;
                         if (!inbit) {
-                            atomicAdd(&sm.ifast[strand][ap], 1u << (8 * ((iword >> (2 * (qi1 & 15))) & 3u)));
+                            if (!kEvOnly) atomicAdd(&sm.ifast[strand][ap], 1u << (8 * ((iword >> (2 * (qi1 & 15))) & 3u)));
                             chain = false;
                         }
                     }
@@ -587,12 +591,12 @@ __device__ __forceinline__ void process_read2(TileSmem<T>& sm, const nsnp_reads_
                             evr.info = (uint32_t)len | ((uint32_t)cls << 8);
                             evr.seq = (uint64_t)(meta.sbase + qs);
                             slab[e] = evr;
-                        } else {
+                        } else if (kEvOnly) {
                             dev_fail(status, DEV_E_INDEL_SLAB, sm.tile);
                         }
                     }
                 }
-            } else if (op == 3 && a < b) {                                    // reference skip: covered, nothing counted
+            } else if (!kEvOnly && op == 3 && a < b) {                                    // reference skip: covered, nothing counted
                 atomicSub(&sm.ms[a - ts], sinc);
                 if (b < te) atomicAdd(&sm.ms[b - ts], sinc);
                 for (int p = a; p < b; ++p) atomicOr(&sm.skipcov[(p - ts) >> 5], 1u << ((p - ts) & 31));
@@ -696,34 +700,39 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
         // count is known before any read is processed only when the candidates fit one round; otherwise assume deep:
         // then every indel event is chained and counted by the walk (16-bit results).
         bool deep = rhi - rlo > kReadList;
-        for (int rb = rlo; rb < rhi; rb += kReadList) {
-            __syncthreads();
-            if (tid == 0) { sm.n_rlist = 0; sm.next_task = 0; }
-            __syncthreads();
-            for (int r = rb + tid; r < min(rhi, rb + kReadList); r += kThreads) {
-                // overlap test; a read that merely starts at te has no anchor inside the tile
-                if (rd.pos[r] < te && ws.rend[r] > ts) sm.rlist[atomicAdd(&sm.n_rlist, 1)] = r;
+        // one walk over the reads that overlap [elo, ehi): the whole tile first; events-only re-walks of anchor sub-ranges
+        // (kEv) when the tile's chained indel events overflowed the slab
+        auto walk = [&](const int elo, const int ehi, auto ev_tag) {
+            constexpr bool kEv = decltype(ev_tag)::value;
+            for (int rb = rlo; rb < rhi; rb += kReadList) {
+                __syncthreads();
+                if (tid == 0) { sm.n_rlist = 0; sm.next_task = 0; }
+                __syncthreads();
+                for (int r = rb + tid; r < min(rhi, rb + kReadList); r += kThreads) {
+                    // overlap test; a read that merely starts at ehi has no anchor inside the window
+                    if (rd.pos[r] < ehi && ws.rend[r] > elo) sm.rlist[atomicAdd(&sm.n_rlist, 1)] = r;
+                }
+                __syncthreads();
+                const int nr = sm.n_rlist;
+                if (!kEv) { n_overlap += nr; deep = deep || nr > 255; }
+                // dynamic read -> warp assignment; the NEXT read's metadata is fetched before the current one is processed
+                auto grab = [&]() { int t = 0; if (lane == 0) t = atomicAdd(&sm.next_task, 1); return __shfl_sync(0xffffffffu, t, 0); };
+                int t = grab();
+                ReadMeta meta = {};
+                int r = 0;
+                if (t < nr) { r = sm.rlist[t]; meta = load_meta(rd, ws, r); }
+                while (t < nr) {
+                    const int tn = grab();
+                    ReadMeta mnext = {};
+                    int rn = 0;
+                    if (tn < nr) { rn = sm.rlist[tn]; mnext = load_meta(rd, ws, rn); }
+                    if (V == 2) process_read2<T, kEv>(sm, rd, ws, slab, r, meta, ts, te, elo, ehi, deep, status);
+                    else process_read<T, kEv>(sm, rd, ws, slab, r, meta, ts, te, elo, ehi, deep, status);
+                    t = tn; r = rn; meta = mnext;
+                }
             }
-            __syncthreads();
-            const int nr = sm.n_rlist;
-            n_overlap += nr;
-            deep = deep || nr > 255;
-            // dynamic read -> warp assignment; the NEXT read's metadata is fetched before the current one is processed
-            auto grab = [&]() { int t = 0; if (lane == 0) t = atomicAdd(&sm.next_task, 1); return __shfl_sync(0xffffffffu, t, 0); };
-            int t = grab();
-            ReadMeta meta = {};
-            int r = 0;
-            if (t < nr) { r = sm.rlist[t]; meta = load_meta(rd, ws, r); }
-            while (t < nr) {
-                const int tn = grab();
-                ReadMeta mnext = {};
-                int rn = 0;
-                if (tn < nr) { rn = sm.rlist[tn]; mnext = load_meta(rd, ws, rn); }
-                if (V == 2) process_read2<T>(sm, rd, ws, slab, r, meta, ts, te, deep, status);
-                else process_read<T>(sm, rd, ws, slab, r, meta, ts, te, deep, status);
-                t = tn; r = rn; meta = mnext;
-            }
-        }
+        };
+        walk(ts, te, std::false_type{});
         __syncthreads();
         if (tid == 0 && n_overlap > kMaxOverlap) dev_fail(status, DEV_E_DEPTH, (int)(ts & 0x7fffffff));
 
@@ -766,8 +775,9 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
         //      the positions {warp*32 + lane + 256*k}: it first COMPACTS the positions that need a walk into a list
         //      (ballot ranks), then walks them one per lane, so the walk runs with full lanes and the channel epilogue
         //      below stays straight-line and convergent.  Results per position (u16 pairs):
-        //      cnt4 <- tot I | i << 16,  head <- tot D | d << 16,  dfast <- max I | i << 16,  ifast[0] <- max D | d << 16. ----
-        {
+        //      cnt4 <- tot I | i << 16,  head <- tot D | d << 16,  dfast <- max I | i << 16,  ifast[0] <- max D | d << 16.
+        //      Positions [plo, phi) only: all of them, or one anchor sub-range of an overflowed tile. ----
+        auto indel_channels = [&](const int plo, const int phi) {
             // per-class (I i D d) sum and maximum of the fast group counters, as bytes of one word each
             auto fast_stats = [](uint32_t dfv, uint32_t if0, uint32_t if1, uint32_t& fsum, uint32_t& fmax) {
                 auto sum4 = [](uint32_t x) { const uint32_t t = (x & 0x00FF00FFu) + ((x >> 8) & 0x00FF00FFu); return (t + (t >> 16)) & 0x3FFu; };
@@ -784,10 +794,11 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
                 uint32_t fsum, fmax;
                 fast_stats(sm.dfast[p], sm.ifast[0][p], sm.ifast[1][p], fsum, fmax);
                 const uint32_t oth = __vsub4(c4, fsum);            // chained events per class
-                const bool need = p < tn && (deep ? sm.head[p] != kNoEvent : ((oth + 0x7E7E7E7Eu) & 0x80808080u) != 0u);   // some byte >= 2
+                const bool inr = p >= plo && p < phi;
+                const bool need = inr && p < tn && (deep ? sm.head[p] != kNoEvent : ((oth + 0x7E7E7E7Eu) & 0x80808080u) != 0u);   // some byte >= 2
                 const uint32_t bal = __ballot_sync(0xffffffffu, need);
                 if (need) wl[nlist + __popc(bal & ((1u << lane) - 1u))] = p;
-                else {
+                else if (inr) {
                     const uint32_t mx = __vmaxu4(fmax, oth);       // a class with <= 1 chained event: that event is its own group
                     sm.cnt4[p] = (c4 & 0xFFu) | ((c4 & 0xFF00u) << 8); sm.head[p] = ((c4 >> 16) & 0xFFu) | ((c4 >> 24) << 16);
                     sm.dfast[p] = (mx & 0xFFu) | ((mx & 0xFF00u) << 8); sm.ifast[0][p] = ((mx >> 16) & 0xFFu) | ((mx >> 24) << 16);
@@ -856,6 +867,37 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
                 sm.dfast[p] = (uint32_t)mxs[0] | ((uint32_t)mxs[1] << 16); sm.ifast[0][p] = (uint32_t)mxs[2] | ((uint32_t)mxs[3] << 16);
             }
             __syncwarp();
+        };
+        if (sm.n_events <= ws.slab_cap) {
+            indel_channels(0, T);
+        } else {
+            // The slab held only the first slab_cap chained events of this tile (the rest were not linked).  Re-walk the
+            // reads once per anchor sub-range whose events fit the slab, each time rebuilding the chains of that range
+            // and reducing them.  cnt4 bounds the chained events per position: in a deep tile it counts exactly them, else
+            // its byte sum counts every event.  One position holds at most two events per read (an insertion and a
+            // deletion after it), so with <= kMaxOverlap reads a single position always fits.  Tiles that fit never get here.
+            for (int i = tid; i < T; i += kThreads) sm.head[i] = kNoEvent;
+            for (int alo = 0; alo < tn;) {
+                __syncthreads();                            // heads reset / previous sub-range reduced, read list free
+                if (tid == 0) {
+                    int64_t acc = 0;
+                    int p = alo;
+                    for (; p < tn; ++p) {
+                        const uint32_t c4 = sm.cnt4[p];
+                        const int64_t w = deep ? (int64_t)c4 : (int64_t)((c4 & 0xFFu) + ((c4 >> 8) & 0xFFu) + ((c4 >> 16) & 0xFFu) + (c4 >> 24));
+                        if (acc + w > ws.slab_cap && p > alo) break;
+                        acc += w;
+                    }
+                    sm.sub_end = p;
+                    sm.n_events = 0;
+                }
+                __syncthreads();
+                const int ahi = sm.sub_end;
+                walk(ts + alo, ts + ahi, std::true_type{});
+                __syncthreads();
+                indel_channels(alo, ahi);
+                alo = ahi;
+            }
         }
 
         // ---- epilogue: 18 channels + gate per position, rows stored straight from registers.  Warp-private positions:
