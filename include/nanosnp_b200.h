@@ -209,6 +209,19 @@ int nsnp_hap_model_pack_weights(const nsnp_hap_weights_t* w, void* host_blob, si
 size_t nsnp_hap_model_workspace_bytes(int64_t n);
 int nsnp_hap_model_forward(const void* blob_dev, const float* xp_dev, const float* xh_dev, int64_t n, float* gt_prob_dev, float* zy_prob_dev,
                            void* workspace_dev, size_t workspace_bytes, void* stream);
+/* Opt-in tensor-core version of nsnp_hap_model_forward (csrc/haplotype_tc.cu): same inputs and outputs, its own packed blob and
+ * workspace.  Precision f16x3: tcgen05 MMAs with hi/lo split operands (three MMAs per product), fp32 accumulation -- tf32 hi/lo
+ * for the layer-0 input channels (unbounded feature values), fp16 hi/lo for h and the layer outputs.  Probabilities stay within
+ * 5e-5 of a float64 evaluation of the network, as NSNP_PREC_F16X3 does for the PileupModel; nsnp_hap_model_forward (fp32) stays
+ * the parity reference.  A site's result does not depend on the batch it is in. */
+size_t nsnp_hap_model_tc_blob_bytes(void);
+int nsnp_hap_model_tc_pack_weights(const nsnp_hap_weights_t* w, void* host_blob, size_t blob_bytes);
+size_t nsnp_hap_model_tc_workspace_bytes(int64_t n);
+int nsnp_hap_model_tc_forward(const void* blob_dev, const float* xp_dev, const float* xh_dev, int64_t n, float* gt_prob_dev, float* zy_prob_dev,
+                              void* workspace_dev, size_t workspace_bytes, void* stream);
+/* test aid, like nsnp_debug_lstm_tc_gates: the layer-0 gate pre-activations (input part + bias, h = 0) of the FIRST step of one
+ * (encoder 0 pileup / 1 haplotype, direction), [m][1024] in PyTorch gate order.  x_dev: that encoder's features [m][105][L]. */
+int nsnp_debug_hap_tc_gates(const void* blob_dev, const float* x_dev, int encoder, int dir, float* gates_out_dev, int64_t m, void* stream);
 
 /* ---- BASELINE configs[4]: HaplotypeModel s4, read x position matrices (csrc/hap_groups.cu) -----------------------------
  * Replaces single_group_pileup_haplotype_feature (HaplotypeModel/create_pileup_haplotype.py:23-216): the two pysam pileup

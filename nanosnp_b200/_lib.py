@@ -102,6 +102,11 @@ SYMBOLS = {
     "nsnp_hap_model_pack_weights": (C.c_int, [C.POINTER(HapWeights), _P, _SZ]),
     "nsnp_hap_model_workspace_bytes": (_SZ, [_I64]),
     "nsnp_hap_model_forward": (C.c_int, [_P, _P, _P, _I64, _P, _P, _P, _SZ, _P]),
+    "nsnp_hap_model_tc_blob_bytes": (_SZ, []),
+    "nsnp_hap_model_tc_pack_weights": (C.c_int, [C.POINTER(HapWeights), _P, _SZ]),
+    "nsnp_hap_model_tc_workspace_bytes": (_SZ, [_I64]),
+    "nsnp_hap_model_tc_forward": (C.c_int, [_P, _P, _P, _I64, _P, _P, _P, _SZ, _P]),
+    "nsnp_debug_hap_tc_gates": (C.c_int, [_P, _P, C.c_int, C.c_int, _P, _I64, _P]),
     "nsnp_hap_checkpoint_count": (_I64, [_I64, _I64]),
     "nsnp_hap_read_ends": (C.c_int, [C.POINTER(Reads), _P, _P, _P]),
     "nsnp_hap_group_matrices": (C.c_int, [C.POINTER(Reads), _P, _P, _P, _P, _P, _P, _P, _P, _I64, _I32, _I32, _I32, _P, _P, _P, _P, _P, _P]),

@@ -14,7 +14,7 @@ from pathlib import Path
 ROOT = Path(__file__).resolve().parent
 CSRC = ROOT / "csrc"
 LIB = ROOT / "libnanosnp_b200.so"
-SOURCES = ["api.cu", "synth.cu", "pileup.cu", "select.cu", "model.cu", "model_tc.cu", "vcf.cu", "vcf_dev.cu", "bam.cu", "bam_stream.cu", "record.cu", "haplotype.cu", "hap_groups.cu"]
+SOURCES = ["api.cu", "synth.cu", "pileup.cu", "select.cu", "model.cu", "model_tc.cu", "vcf.cu", "vcf_dev.cu", "bam.cu", "bam_stream.cu", "record.cu", "haplotype.cu", "haplotype_tc.cu", "hap_groups.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

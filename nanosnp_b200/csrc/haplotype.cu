@@ -9,9 +9,10 @@
 //                        kernel (h W_hh^T tile + projected input -> LSTM cell update in the epilogue: the packed weight rows
 //                        interleave the four gates of a unit, so one thread holds i, f, g, o of its unit).  The last layer only
 //                        runs the steps its centre output needs.  This path sees the few low-QUAL sites of a sample
-//                        (~0.34 GFLOP/site); a tcgen05 version along the lines of model_tc.cu is the next step (DESIGN.md).
+//                        (~0.32 GFLOP/site) and is the parity reference of the opt-in tensor-core path
+//                        (nsnp_hap_model_tc_forward, haplotype_tc.cu), which runs its tail through sgemm_nt_kernel / heads_kernel.
 #include <math.h>
-#include "common.cuh"
+#include "hap_common.cuh"
 
 namespace nsnp {
 namespace {
@@ -210,6 +211,21 @@ inline size_t carve_ws(void* base, int64_t n, Ws* w) {
 }
 
 }  // namespace
+
+// the fp32 tail kernels, for the tensor-core path (haplotype_tc.cu)
+int hap_sgemm_nt(const float* A, int64_t lda, const float* B, const float* bias, float* C, int64_t ldc, int64_t M, int N, int K, int act_tanh,
+                 cudaStream_t st)
+{
+    sgemm_nt_kernel<<<dim3((unsigned)((N + 63) / 64), (unsigned)((M + 63) / 64)), 256, 0, st>>>(A, lda, B, bias, C, ldc, M, N, K, act_tanh);
+    return cuda_status("sgemm_nt_kernel");
+}
+
+int hap_heads(const float* hid, const float* gw, const float* gb, const float* zw, const float* zb, float* gt, float* zy, int64_t n, cudaStream_t st)
+{
+    heads_kernel<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(hid, gw, gb, zw, zb, gt, zy, n);
+    return cuda_status("heads_kernel");
+}
+
 }  // namespace nsnp
 
 using namespace nsnp;

@@ -23,6 +23,7 @@ import torch
 from . import _lib
 from .pipeline import require_cuda
 
+PRECISIONS = ("fp32", "f16x3")
 GT10 = ["AA", "AC", "AG", "AT", "CC", "CG", "CT", "GG", "GT", "TT"]                 # HaplotypeModel/options.py:8-17
 _ENC = ("pileup_encoder", "haplotype_encoder")
 
@@ -43,9 +44,15 @@ def required_keys():
 
 
 class LSTMNetwork:
-    """model_dev.LSTMNetwork for inference: same constructor / load_state_dict / predict; the forward pass is csrc/haplotype.cu."""
+    """model_dev.LSTMNetwork for inference: same constructor / load_state_dict / predict; the forward pass is csrc/haplotype.cu.
 
-    def __init__(self, config=None):
+    precision "fp32" (default, the parity reference): fp32 FFMA.  "f16x3": tcgen05 tensor cores (csrc/haplotype_tc.cu), hi/lo
+    split operands with three MMAs per product and fp32 accumulation; probabilities within 5e-5 of a float64 evaluation."""
+
+    def __init__(self, config=None, precision: str = "fp32"):
+        if precision not in PRECISIONS:
+            raise ValueError(f"precision must be one of {PRECISIONS}, got {precision!r}")
+        self.precision = precision
         m = getattr(config, "model", None) if config is not None else None
         if m is not None:
             dims = (m.pileup_dim, m.haplotype_dim, m.pileup_length, m.haplotype_length, m.hidden_size, m.lstm_layers, m.gt_num_class, m.zy_num_class)
@@ -93,9 +100,10 @@ class LSTMNetwork:
         for name, field in (("dense", "dense"), ("genotype_layer", "gt"), ("zygosity_layer", "zy")):
             setattr(w, field + "_w", s[f"forward_layer.{name}.weight"].ctypes.data)
             setattr(w, field + "_b", s[f"forward_layer.{name}.bias"].ctypes.data)
-        nbytes = self.lib.nsnp_hap_model_blob_bytes()
+        tc = self.precision == "f16x3"
+        nbytes = (self.lib.nsnp_hap_model_tc_blob_bytes if tc else self.lib.nsnp_hap_model_blob_bytes)()
         host = np.zeros(nbytes, np.uint8)
-        _lib.check(self.lib.nsnp_hap_model_pack_weights(C.byref(w), host.ctypes.data, nbytes))
+        _lib.check((self.lib.nsnp_hap_model_tc_pack_weights if tc else self.lib.nsnp_hap_model_pack_weights)(C.byref(w), host.ctypes.data, nbytes))
         self._blob = torch.from_numpy(host).to(self.device)
 
     def predict(self, pileup_x: torch.Tensor, haplotype_x: torch.Tensor):
@@ -107,12 +115,14 @@ class LSTMNetwork:
         assert tuple(px.shape[1:]) == (105, 33) and tuple(hx.shape) == (n, 105, 11)
         gt = torch.empty((n, 10), dtype=torch.float32, device=self.device)
         zy = torch.empty((n, 3), dtype=torch.float32, device=self.device)
-        need = self.lib.nsnp_hap_model_workspace_bytes(n)
+        tc = self.precision == "f16x3"
+        need = (self.lib.nsnp_hap_model_tc_workspace_bytes if tc else self.lib.nsnp_hap_model_workspace_bytes)(n)
         if self._ws is None or self._ws.numel() < need:
             self._ws = torch.empty(need, dtype=torch.uint8, device=self.device)
+        forward = self.lib.nsnp_hap_model_tc_forward if tc else self.lib.nsnp_hap_model_forward
         with torch.cuda.device(self.device):
-            _lib.check(self.lib.nsnp_hap_model_forward(self._blob.data_ptr(), px.data_ptr(), hx.data_ptr(), n, gt.data_ptr(), zy.data_ptr(),
-                                                       self._ws.data_ptr(), self._ws.numel(), _stream(self.device)))
+            _lib.check(forward(self._blob.data_ptr(), px.data_ptr(), hx.data_ptr(), n, gt.data_ptr(), zy.data_ptr(),
+                               self._ws.data_ptr(), self._ws.numel(), _stream(self.device)))
         return gt, zy
 
 
@@ -260,11 +270,13 @@ def main(argv=None):
     ap.add_argument("-output", required=True)
     ap.add_argument("-batch_size", type=int, default=1000)
     ap.add_argument("--no_cuda", action="store_true")
+    ap.add_argument("--precision", choices=PRECISIONS, default="fp32",
+                    help="fp32: FFMA parity path (default); f16x3: tensor cores, hi/lo split operands, within 5e-5 of float64")
     opt = ap.parse_args(argv)
     if opt.no_cuda:
         raise SystemExit("nanosnp_b200.haplotype: --no_cuda is not supported (no CPU fallback)")
     config = AttrDict(yaml.load(open(opt.config), Loader=yaml.FullLoader))
-    net = LSTMNetwork(config).to("cuda")
+    net = LSTMNetwork(config, precision=opt.precision).to("cuda")
     net.load_state_dict(torch.load(opt.model_path, map_location="cpu"))
     predict(net, opt.bin_paths, opt.reference_path, opt.batch_size, config.model.pileup_length, config.model.haplotype_length, opt.output, "cuda")
 

@@ -1,6 +1,7 @@
 #!/usr/bin/env python
 """BASELINE configs[4] measurement: HaplotypeModel s4 (read matrices) + s5 (features, model) on one synthetic contig.
-usage: tools/hap_bench.py [mb] [coverage] [reps]   -> one JSON line (groups/s per stage, device-timed)"""
+usage: tools/hap_bench.py [mb] [coverage] [reps]   -> one JSON line (groups/s per stage, device-timed; the model at both
+precisions, fp32 and the tensor-core f16x3, timed alternately after warm-up)"""
 import json
 import os
 import sys
@@ -56,10 +57,29 @@ def feats():
             G.frequency_features(gm.hap[0][:, :d], gm.hap[2][:, :d], gm.hap[3][:, :d], gm.hap[1][:, :d], href, dev))
 (xp, xh), ms_feat, _ = timed(feats)
 from oracle.hap_restate import HaplotypeModelOracle          # weights only (random init: the checkpoint is not shipped)
-net = G.LSTMNetwork().to(dev); net.load_state_dict(HaplotypeModelOracle(seed=1).state_dict())
-_, ms_model, _ = timed(lambda: net.predict(xp, xh))
+sd = HaplotypeModelOracle(seed=1).state_dict()
+net = G.LSTMNetwork().to(dev); net.load_state_dict(sd)
+net_tc = G.LSTMNetwork(precision="f16x3").to(dev); net_tc.load_state_dict(sd)
+# both precisions in the same run: warm up each, then alternate the timed calls
+(g32, z32), (gtc, ztc) = net.predict(xp, xh), net_tc.predict(xp, xh)
+ms32, mstc = [], []
+for _ in range(reps):
+    ms32.append(timed(lambda: net.predict(xp, xh))[1]); mstc.append(timed(lambda: net_tc.predict(xp, xh))[1])
+ms_model, ms_tc = min(ms32), min(mstc)
+dp = max(float((gtc - g32).abs().max()), float((ztc - z32).abs().max()))
+# pruned multiply-adds per site: every LSTM step the model needs (the last layer stops at the centre) plus the tail
+mac = sum(steps * 2 * 1024 * (in_dim + 256) for Lx in (33, 11) for steps, in_dim in ((Lx, 105), (Lx, 512), (Lx // 2 + 1, 512)))
+mac += 2 * 256 * 512 + 256 * 512 + 13 * 256
+try:
+    import subprocess
+    power = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", "0"], capture_output=True, text=True).stdout.strip()
+except OSError:
+    power = "unknown"
 out = {"workload": f"synthetic {mb} Mb contig at {cov}x, HP tags + qualities random, 1 site / kb, QUAL<19 candidates", "reads": n,
        "groups": int(len(groups)), "groups_out": int(G_), "rows_cap": int(gm.hap[0].shape[1]), "mean_depth": float(gm.depth.mean()),
        "s4_matrices_ms": ms_mat, "s4_matrices_wall_ms": wall_mat, "s5_features_ms": ms_feat, "s5_model_ms": ms_model,
-       "groups_per_s_s4": G_ / (wall_mat * 1e-3), "groups_per_s_s4_s5": G_ / ((wall_mat + ms_feat + ms_model) * 1e-3)}
+       "groups_per_s_s4": G_ / (wall_mat * 1e-3), "groups_per_s_s4_s5": G_ / ((wall_mat + ms_feat + ms_model) * 1e-3),
+       "s5_model_tc_ms": ms_tc, "tc_speedup": ms_model / ms_tc, "mac_per_site_pruned": mac,
+       "tflops_fp32": 2 * mac * G_ / (ms_model * 1e-3) / 1e12, "tflops_tc": 2 * mac * G_ / (ms_tc * 1e-3) / 1e12,
+       "max_abs_dp_tc_vs_fp32": dp, "gpu": torch.cuda.get_device_name(dev), "power_limit": power}
 print(json.dumps(out))
