@@ -123,6 +123,31 @@ int nsnp_select_candidates(const int32_t* counts_dev, uint8_t* flags_dev, const 
                            int recompute_gate, int32_t* pos_dev, int64_t capacity, int32_t* n_dev,
                            void* workspace_dev, size_t workspace_bytes, int32_t* status_dev, void* stream);
 
+/* ---- s1, steps A and B restricted to target intervals ------------------------------------------------
+ * An extension of this library with no reference counterpart (NanoSNP calls whole contigs).
+ * targets: n_targets half-open [start, end) int32 pairs in contig coordinates, in HOST memory, non-empty,
+ * ascending and disjoint (adjacent is allowed), inside [region_start, region_start + region_len); anything
+ * else returns NSNP_E_INVALID.  The library copies them to its workspace and derives on the device
+ *   - pileup: the tiles holding any position of [start - 16, end + 16); only those are computed.  Flags of
+ *     every other position are written as 0 and their count rows are left unwritten.  Count rows and flags
+ *     of computed positions equal those of nsnp_pileup_counts on the same reads.  The read pre-pass and the
+ *     depth cap still run over every read passed.
+ *   - select: a position is a candidate iff it is one of nsnp_select_candidates AND lies in an interval.
+ * n_targets == 0 is valid: no tile is computed, no site is selected.
+ */
+size_t nsnp_pileup_targets_workspace_bytes(int64_t n_reads, int64_t n_cigar, int64_t region_len, int64_t n_targets);
+int nsnp_pileup_counts_targets(const nsnp_reads_t* reads_dev, const uint8_t* ref_dev, int64_t contig_len,
+                               int64_t region_start, int64_t region_len, const int32_t* targets, int64_t n_targets,
+                               const nsnp_params_t* params, int32_t* counts_dev, uint8_t* flags_dev,
+                               void* workspace_dev, size_t workspace_bytes, int32_t* status_dev, void* stream);
+size_t nsnp_select_targets_workspace_bytes(int64_t region_len, int64_t n_targets);
+int nsnp_select_candidates_targets(const int32_t* counts_dev, uint8_t* flags_dev, const uint8_t* ref_dev,
+                                   int64_t contig_len, int64_t region_start, int64_t region_len,
+                                   int64_t emit_start, int64_t emit_end, const int32_t* targets, int64_t n_targets,
+                                   const nsnp_params_t* params, int recompute_gate, int32_t* pos_dev, int64_t capacity,
+                                   int32_t* n_dev, void* workspace_dev, size_t workspace_bytes, int32_t* status_dev,
+                                   void* stream);
+
 /* ---- s1, step C: window gather ------------------------------------------------------------------
  * Replaces the ring-buffer window emit (main.cpp:220-251), DNA_CreatePredictData
  * (make_predict_data/main.cpp:76-127) and make_bin_predict_data.py:35-55: writes position_matrix
@@ -370,6 +395,11 @@ int32_t nsnp_bam_next_contig(nsnp_bam_reader_t* r, const int8_t* want, int64_t* 
 /* reads of ref_id that start before `end` and overlap [beg, end) (needs the .bai); returns ref_id or -2 */
 int32_t nsnp_bam_fetch(nsnp_bam_reader_t* r, int32_t ref_id, int64_t beg, int64_t end, int64_t* n_reads, int64_t* n_cigar,
                        int64_t* n_bases_padded);
+/* reads of ref_id that overlap any of the n ranges [beg, end) (int64 pairs, ascending and disjoint; needs the .bai), each
+ * once, in file order.  Seeks through the linear index only when a range's first offset lies past what is already inflated,
+ * so each needed BGZF block is inflated once.  Returns ref_id or -2. */
+int32_t nsnp_bam_fetch_ranges(nsnp_bam_reader_t* r, int32_t ref_id, const int64_t* ranges, int64_t n, int64_t* n_reads,
+                              int64_t* n_cigar, int64_t* n_bases_padded);
 int nsnp_bam_take(nsnp_bam_reader_t* r, int32_t* pos, uint16_t* flag, uint8_t* mapq, int64_t* cigar_off, uint32_t* cigar,
                   int64_t* seq_off, uint8_t* seq2, uint8_t* nmask, int32_t* any_n);
 /* HaplotypeModel s4 inputs: with keep != 0 the reader also keeps, for every record it decodes from then on, the base

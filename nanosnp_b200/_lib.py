@@ -87,6 +87,11 @@ SYMBOLS = {
     "nsnp_pileup_counts": (C.c_int, [C.POINTER(Reads), _P, _I64, _I64, _I64, C.POINTER(Params), _P, _P, _P, _SZ, _P, _P]),
     "nsnp_select_workspace_bytes": (_SZ, [_I64]),
     "nsnp_select_candidates": (C.c_int, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, C.POINTER(Params), C.c_int, _P, _I64, _P, _P, _SZ, _P, _P]),
+    "nsnp_pileup_targets_workspace_bytes": (_SZ, [_I64, _I64, _I64, _I64]),
+    "nsnp_pileup_counts_targets": (C.c_int, [C.POINTER(Reads), _P, _I64, _I64, _I64, _P, _I64, C.POINTER(Params), _P, _P, _P, _SZ, _P, _P]),
+    "nsnp_select_targets_workspace_bytes": (_SZ, [_I64, _I64]),
+    "nsnp_select_candidates_targets": (C.c_int, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _P, _I64, C.POINTER(Params), C.c_int, _P, _I64, _P,
+                                                 _P, _SZ, _P, _P]),
     "nsnp_gather_windows": (C.c_int, [_P, _P, _I64, _I64, _P, _P, _I64, _P, _P, _P, _P]),
     "nsnp_model_blob_bytes": (_SZ, []),
     "nsnp_model_pack_weights": (C.c_int, [C.POINTER(ModelWeights), _P, _SZ]),
@@ -139,6 +144,7 @@ SYMBOLS = {
     "nsnp_bam_inflated_bytes": (_I64, [_P]),
     "nsnp_bam_next_contig": (_I32, [_P, _P, _P, _P, _P]),
     "nsnp_bam_fetch": (_I32, [_P, _I32, _I64, _I64, _P, _P, _P]),
+    "nsnp_bam_fetch_ranges": (_I32, [_P, _I32, _P, _I64, _P, _P, _P]),
     "nsnp_bam_take": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     "nsnp_bam_keep_aux": (C.c_int, [_P, C.c_int]),
     "nsnp_bam_take_aux": (C.c_int, [_P, _P, _P, _P]),

@@ -169,6 +169,18 @@ class BamReader:
         return self._take(n.value, nc.value, nb.value)
 
 
+    def fetch_ranges(self, ref_id: int, ranges) -> PackedReads:
+        """Reads of one reference that overlap any of the ascending, disjoint [beg, end) ranges, each once, in file order
+        (needs the .bai).  Each needed BGZF block is inflated once: the reader walks on between close ranges and seeks
+        through the linear index past gaps."""
+        rg = np.ascontiguousarray(np.asarray(ranges, dtype=np.int64).reshape(-1, 2))
+        n = C.c_int64(0); nc = C.c_int64(0); nb = C.c_int64(0)
+        rid = self.lib.nsnp_bam_fetch_ranges(self.h, int(ref_id), rg.ctypes.data, len(rg), C.byref(n), C.byref(nc), C.byref(nb))
+        if rid < 0:
+            raise ValueError(self.lib.nsnp_last_error().decode())
+        return self._take(n.value, nc.value, nb.value)
+
+
 def read_bam(path: str, contigs=None, threads: int = 0) -> Tuple[List[Tuple[str, int]], Dict[str, PackedReads]]:
     """Returns (reference list, {contig: PackedReads}) for the requested contigs (default: all with reads).  Convenience
     for small files: callers that must bound memory iterate BamReader.contigs() / fetch() instead."""

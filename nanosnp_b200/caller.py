@@ -22,8 +22,9 @@ def _pinned(reads: PackedReads) -> PackedReads:
 
 
 def call_contig(runner: RegionRunner, reads: PackedReads, ref: np.ndarray, contig: str, sink, batch_size: int = 1000,
-                region_len: int = 12_500_000, n_threads: int = 0, regions=None) -> dict:
-    """reads: numpy PackedReads of one contig (coordinate sorted).  Writes VCF records to `sink` (binary file-like)."""
+                region_len: int = 12_500_000, n_threads: int = 0, regions=None, targets=None) -> dict:
+    """reads: numpy PackedReads of one contig (coordinate sorted).  Writes VCF records to `sink` (binary file-like).
+    targets: optional per-region intervals, aligned with `regions` (shard.plan_target_units)."""
     L = int(len(ref))
     ref_dev = torch.from_numpy(np.ascontiguousarray(ref)).to(runner.device)
     regions = regions if regions is not None else plan_regions([(contig, L)], region_len)
@@ -49,15 +50,16 @@ def call_contig(runner: RegionRunner, reads: PackedReads, ref: np.ndarray, conti
         else:
             asm.add(res["pos0"].numpy(), res["refbase"].numpy(), res["gt"].numpy(), res["zy"].numpy(), res["cov8"].numpy())
         return None
-    n = runner.run_host_many(host_regions, regions, ref_dev, host_outs, consume)
+    n = runner.run_host_many(host_regions, regions, ref_dev, host_outs, consume, targets)
     nbytes = asm.close()
     return {"sites": n, "vcf_bytes": nbytes, "regions": len(regions)}
 
 
 def call_contig_text(runner: RegionRunner, reads: PackedReads, ref: np.ndarray, contig: str, sink, batch_size: int = 1000,
-                     region_len: int = 12_500_000, regions=None, region_reads=None) -> dict:
+                     region_len: int = 12_500_000, regions=None, region_reads=None, targets=None) -> dict:
     """call_contig with the VCF text assembled on the GPU (csrc/vcf_dev.cu): the host only writes the bytes.
-    region_reads: optional ready-made per-region PackedReads (e.g. BamReader.fetch); else `reads` is sliced."""
+    region_reads: optional ready-made per-region PackedReads (e.g. BamReader.fetch); else `reads` is sliced.
+    targets: optional per-region intervals, aligned with `regions` (shard.plan_target_units)."""
     from .vcf_text import GpuVcfText
     L = int(len(ref))
     ref_dev = torch.from_numpy(np.ascontiguousarray(ref)).to(runner.device)
@@ -73,7 +75,7 @@ def call_contig_text(runner: RegionRunner, reads: PackedReads, ref: np.ndarray, 
         nbytes[0] += len(mv)
         if sink is not None:
             sink.write(mv)
-    n = runner.run_host_text(host_regions, regions, ref_dev, gen, write)
+    n = runner.run_host_text(host_regions, regions, ref_dev, gen, write, targets)
     return {"sites": n, "vcf_bytes": nbytes[0], "regions": len(regions)}
 
 

@@ -430,9 +430,10 @@ int64_t nsnp_bam_inflated_bytes(const nsnp_bam_reader_t* r) { return r ? r->infl
 // shared record loop: decodes records of reference `ref` with pos < end whose reference span reaches beyond beg.
 // ref < 0: take the reference of the first wanted record.  Stops (without consuming) at the first record of another
 // reference or with pos >= end.  Returns the reference decoded, -1 at end of file, -2 on corruption.
-static int32_t decode_run(nsnp_bam_reader* r, int32_t ref, const int8_t* want, int64_t beg, int64_t end)
+// append: keep the records already decoded (nsnp_bam_fetch_ranges)
+static int32_t decode_run(nsnp_bam_reader* r, int32_t ref, const int8_t* want, int64_t beg, int64_t end, bool append = false)
 {
-    r->clear_arrays();
+    if (!append) r->clear_arrays();
     bool err = false;
     int32_t cur_ref = ref;
     for (;;) {
@@ -511,6 +512,39 @@ int32_t nsnp_bam_fetch(nsnp_bam_reader_t* r, int32_t ref_id, int64_t beg, int64_
         // records of earlier references cannot appear after this offset; skip reads that end before the window
         rid = decode_run(r, ref_id, nullptr, beg, end);
         if (rid == -2) return -2;
+    }
+    if (n_reads) *n_reads = (int64_t)r->pos.size();
+    if (n_cigar) *n_cigar = (int64_t)r->cigar.size();
+    if (n_bases_padded) *n_bases_padded = r->n_bases;
+    return ref_id;
+}
+
+int32_t nsnp_bam_fetch_ranges(nsnp_bam_reader_t* r, int32_t ref_id, const int64_t* ranges, int64_t n, int64_t* n_reads,
+                              int64_t* n_cigar, int64_t* n_bases_padded)
+{
+    if (!r || ref_id < 0 || ref_id >= (int32_t)r->ref_names.size()) { nsnp::set_error(NSNP_E_INVALID, "nsnp_bam_fetch_ranges: bad reference id"); return -2; }
+    if (!r->has_bai) { nsnp::set_error(NSNP_E_UNSUPPORTED, "nsnp_bam_fetch_ranges needs a .bai index next to the BAM"); return -2; }
+    if (n < 0 || (n > 0 && !ranges)) { nsnp::set_error(NSNP_E_INVALID, "nsnp_bam_fetch_ranges: bad range list"); return -2; }
+    for (int64_t k = 0; k < n; ++k)
+        if (ranges[2 * k] < 0 || ranges[2 * k + 1] <= ranges[2 * k] || (k && ranges[2 * k] < ranges[2 * k - 1])) {
+            nsnp::set_error(NSNP_E_INVALID, "nsnp_bam_fetch_ranges: range %lld is empty, unsorted or overlapping", (long long)k);
+            return -2;
+        }
+    r->clear_arrays();
+    if (r->bai[ref_id].has) {
+        const auto& io = r->bai[ref_id].ioff;
+        for (int64_t k = 0; k < n; ++k) {
+            const int64_t beg = ranges[2 * k], end = ranges[2 * k + 1];
+            uint64_t v = 0;
+            const size_t w = (size_t)(beg >> 14);
+            if (w < io.size()) v = io[w];
+            if (v == 0) { for (size_t j = std::min(w, io.size()); j-- > 0;) if (io[j]) { v = io[j]; break; } }
+            if (v == 0) v = r->bai[ref_id].first;
+            // Records are consumed in file order, so none is decoded twice.  Blocks before next_block are inflated (or being
+            // inflated) already: walk on from the current record, skipping those that end before the range.  Seek only past them.
+            if (k == 0 || (size_t)(v >> 16) >= r->next_block) r->seek(v);
+            if (decode_run(r, ref_id, nullptr, beg, end, true) == -2) return -2;
+        }
     }
     if (n_reads) *n_reads = (int64_t)r->pos.size();
     if (n_cigar) *n_cigar = (int64_t)r->cigar.size();

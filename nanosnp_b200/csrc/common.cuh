@@ -59,4 +59,19 @@ __host__ __device__ __forceinline__ int nt4(uint8_t c) {
     }
 }
 
+// Target intervals of nsnp_pileup_counts_targets / nsnp_select_candidates_targets: n half-open [start, end) int32 pairs in
+// contig coordinates (host memory), non-empty, ascending and disjoint (adjacent allowed), inside [lo, hi).
+inline int check_targets(const char* fn, const int32_t* iv, int64_t n, int64_t lo, int64_t hi) {
+    if (n < 0 || (n > 0 && !iv)) return set_error(NSNP_E_INVALID, "%s: bad interval list", fn);
+    int64_t prev = lo;
+    for (int64_t k = 0; k < n; ++k) {
+        const int64_t s = iv[2 * k], e = iv[2 * k + 1];
+        if (s < prev || e <= s || e > hi)
+            return set_error(NSNP_E_INVALID, "%s: interval %lld [%lld,%lld) is empty, unsorted, overlapping or outside [%lld,%lld)", fn,
+                             (long long)k, (long long)s, (long long)e, (long long)lo, (long long)hi);
+        prev = e;
+    }
+    return NSNP_OK;
+}
+
 }  // namespace nsnp

@@ -42,6 +42,10 @@ struct Workspace {
     int32_t* cap_heap;    // [n_reads] min-heap of the slow path
     Event*   slabs;       // [n_ctas][slab_cap]
     int64_t  slab_cap;
+    // target intervals (nsnp_pileup_counts_targets); tile_list == nullptr: every tile of the region, in ticket order
+    int32_t* targets;     // [2 * n_targets] copied from the host
+    int32_t* tile_diff;   // [n_tiles + 1] boundary deltas of the listed tile ranges
+    int32_t* tile_list;   // [n_tiles] ascending tile indices, count in counters[6]
 };
 
 // CIGAR words: BAM's u32 (len << 4 | op), or the same values as u16 when every length is below 4096 (nsnp_reads.cigar_bits = 16:
@@ -658,7 +662,10 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
 
     for (;;) {
         __syncthreads();                                    // previous tile fully written, smem reusable
-        if (tid == 0) sm.tile = atomicAdd(&ws.counters[0], 1);
+        if (tid == 0) {
+            const int k = atomicAdd(&ws.counters[0], 1);
+            sm.tile = ws.tile_list == nullptr ? k : k < *(volatile int32_t*)&ws.counters[6] ? ws.tile_list[k] : n_tiles;
+        }
         __syncthreads();
         const int tile = sm.tile;
         if (tile >= n_tiles) break;
@@ -963,6 +970,47 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
     }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Tile list of a targeted call: the tiles holding any position of [start - 16, end + 16) of some interval, ascending.
+// One block, no per-interval launch: boundary deltas per interval (tile ranges of neighbouring intervals may overlap),
+// then a running sum and an ordered compaction over the tiles.  Count -> counters[6].
+__global__ void __launch_bounds__(1024) tile_list_kernel(Workspace ws, int n_iv, int64_t region_start, int64_t region_len,
+                                                         int tile_shift, int n_tiles)
+{
+    __shared__ int wtot[2][32];
+    __shared__ int carry[2];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    for (int i = tid; i <= n_tiles; i += 1024) ws.tile_diff[i] = 0;
+    if (tid < 2) carry[tid] = 0;
+    __syncthreads();
+    for (int k = tid; k < n_iv; k += 1024) {
+        const int64_t a = max((int64_t)ws.targets[2 * k] - NSNP_FLANK, region_start) - region_start;
+        const int64_t b = min((int64_t)ws.targets[2 * k + 1] + NSNP_FLANK, region_start + region_len) - region_start;
+        if (a < b) { atomicAdd(&ws.tile_diff[a >> tile_shift], 1); atomicSub(&ws.tile_diff[((b - 1) >> tile_shift) + 1], 1); }
+    }
+    __syncthreads();
+    for (int base = 0; base < n_tiles; base += 1024) {
+        const int i = base + tid;
+        const int d = i < n_tiles ? ws.tile_diff[i] : 0;
+        const int di = warp_incl_scan(d);
+        if (lane == 31) wtot[0][warp] = di;
+        __syncthreads();
+        int run = carry[0] + di;
+        for (int w = 0; w < warp; ++w) run += wtot[0][w];
+        const bool listed = i < n_tiles && run > 0;
+        const uint32_t bal = __ballot_sync(0xffffffffu, listed);
+        if (lane == 0) wtot[1][warp] = __popc(bal);
+        __syncthreads();
+        int off = carry[1] + __popc(bal & ((1u << lane) - 1u));
+        for (int w = 0; w < warp; ++w) off += wtot[1][w];
+        if (listed) ws.tile_list[off] = i;
+        __syncthreads();
+        if (tid == 1023) { carry[0] = run; carry[1] = off + (listed ? 1 : 0); }
+        __syncthreads();
+    }
+    if (tid == 0) ws.counters[6] = carry[1];
+}
+
 int tile_shift_for(int64_t region_len) {                                    // T = 1024 (default) or 2048 (NSNP_PILEUP_TILE=2048)
     (void)region_len;
     static int shift = 0;
@@ -979,7 +1027,9 @@ static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; 
 static constexpr int kMaxCtas = kNumSMs * 4;
 static constexpr int64_t kSlabCapMax = 32768;
 
-static void carve(void* base, int64_t n_reads, int64_t n_cigar, int64_t region_len, int tile_shift, Workspace* w, size_t* total) {
+// n_targets < 0: no target areas (the layout of nsnp_pileup_counts)
+static void carve(void* base, int64_t n_reads, int64_t n_cigar, int64_t region_len, int tile_shift, Workspace* w, size_t* total,
+                  int64_t n_targets = -1) {
     const int64_t n_slots = (n_cigar >> kCkShift) + n_reads + 2;
     const int64_t n_tiles = (region_len + (1 << tile_shift) - 1) >> tile_shift;
     int64_t cap = n_cigar < kSlabCapMax ? n_cigar : kSlabCapMax; if (cap < 64) cap = 64;
@@ -995,20 +1045,20 @@ static void carve(void* base, int64_t n_reads, int64_t n_cigar, int64_t region_l
     w->cap_heap = (int32_t*)take((size_t)(n_reads + 1) * 4);
     w->slabs = (Event*)take((size_t)kMaxCtas * (size_t)cap * sizeof(Event));
     w->slab_cap = cap;
+    w->targets = w->tile_diff = w->tile_list = nullptr;
+    if (n_targets >= 0) {
+        w->targets = (int32_t*)take((size_t)(2 * n_targets + 2) * 4);
+        w->tile_diff = (int32_t*)take((size_t)(n_tiles + 1) * 4);
+        w->tile_list = (int32_t*)take((size_t)(n_tiles + 1) * 4);
+    }
     *total = off;
 }
 
-extern "C" {
-
-size_t nsnp_pileup_workspace_bytes(int64_t n_reads, int64_t n_cigar, int64_t region_len) {
-    Workspace w; size_t total = 0;
-    carve(nullptr, n_reads < 0 ? 0 : n_reads, n_cigar < 0 ? 0 : n_cigar, region_len < 0 ? 0 : region_len, tile_shift_for(region_len), &w, &total);
-    return total;
-}
-
-int nsnp_pileup_counts(const nsnp_reads_t* reads, const uint8_t* ref_dev, int64_t contig_len, int64_t region_start,
-                       int64_t region_len, const nsnp_params_t* params, int32_t* counts_dev, uint8_t* flags_dev,
-                       void* workspace_dev, size_t workspace_bytes, int32_t* status_dev, void* stream_)
+// targets == nullptr && n_targets < 0: the whole region (nsnp_pileup_counts)
+static int pileup_counts(const nsnp_reads_t* reads, const uint8_t* ref_dev, int64_t contig_len, int64_t region_start,
+                         int64_t region_len, const int32_t* targets, int64_t n_targets, const nsnp_params_t* params,
+                         int32_t* counts_dev, uint8_t* flags_dev, void* workspace_dev, size_t workspace_bytes,
+                         int32_t* status_dev, void* stream_)
 {
     cudaStream_t stream = (cudaStream_t)stream_;
     if (!reads || !params || !ref_dev || !counts_dev || !flags_dev || !status_dev || !workspace_dev)
@@ -1024,18 +1074,29 @@ int nsnp_pileup_counts(const nsnp_reads_t* reads, const uint8_t* ref_dev, int64_
         return set_error(NSNP_E_INVALID, "nsnp_pileup_counts: seq2/nmask must be 4-byte and counts 16-byte aligned");
     if (reads->n_reads > 0x7fffffff - 1) return set_error(NSNP_E_UNSUPPORTED, "more than 2^31 reads in one call");
     if (contig_len > 0x7fffffff - 4096) return set_error(NSNP_E_UNSUPPORTED, "contig longer than 2^31 - 4096 (BAM positions are int32)");
+    if (n_targets >= 0) {
+        if (int e = check_targets("nsnp_pileup_counts_targets", targets, n_targets, region_start, region_start + region_len)) return e;
+    }
     if (nsnp_device_count() == 0) return set_error(NSNP_E_NO_DEVICE, "no CUDA device (there is no CPU fallback)");
     if (region_len == 0) return NSNP_OK;
 
     const int tile_shift = tile_shift_for(region_len);
     Workspace w; size_t need = 0;
-    carve(workspace_dev, reads->n_reads, reads->n_cigar, region_len, tile_shift, &w, &need);
+    carve(workspace_dev, reads->n_reads, reads->n_cigar, region_len, tile_shift, &w, &need, n_targets);
     if (need > workspace_bytes) return set_error(NSNP_E_WORKSPACE, "pileup workspace: need %zu bytes, have %zu", need, workspace_bytes);
     const int n_tiles = (int)((region_len + (1 << tile_shift) - 1) >> tile_shift);
 
     cudaMemsetAsync(w.tile_lo, 0x7f, (size_t)(n_tiles + 1) * 4, stream);
     cudaMemsetAsync(w.tile_hi, 0, (size_t)(n_tiles + 1) * 4, stream);
     cudaMemsetAsync(w.counters, 0, 64, stream);
+    if (n_targets >= 0) {
+        // unlisted tiles: flags zero, count rows left unwritten (nothing reads them)
+        cudaMemsetAsync(flags_dev, 0, (size_t)region_len, stream);
+        if (n_targets > 0)
+            cudaMemcpyAsync(w.targets, targets, (size_t)n_targets * 8, cudaMemcpyHostToDevice, stream);
+        tile_list_kernel<<<1, 1024, 0, stream>>>(w, (int)n_targets, region_start, region_len, tile_shift, n_tiles);
+        if (int e = cuda_status("tile_list_kernel")) return e;
+    }
     if (reads->n_reads > 0) {
         const int64_t warps = reads->n_reads;
         int blocks = (int)((warps + 7) / 8); if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
@@ -1072,6 +1133,39 @@ int nsnp_pileup_counts(const nsnp_reads_t* reads, const uint8_t* ref_dev, int64_
         if (int e = cuda_status("pileup_tile_kernel")) return e;
     }
     return NSNP_OK;
+}
+
+extern "C" {
+
+size_t nsnp_pileup_workspace_bytes(int64_t n_reads, int64_t n_cigar, int64_t region_len) {
+    Workspace w; size_t total = 0;
+    carve(nullptr, n_reads < 0 ? 0 : n_reads, n_cigar < 0 ? 0 : n_cigar, region_len < 0 ? 0 : region_len, tile_shift_for(region_len), &w, &total);
+    return total;
+}
+
+int nsnp_pileup_counts(const nsnp_reads_t* reads, const uint8_t* ref_dev, int64_t contig_len, int64_t region_start,
+                       int64_t region_len, const nsnp_params_t* params, int32_t* counts_dev, uint8_t* flags_dev,
+                       void* workspace_dev, size_t workspace_bytes, int32_t* status_dev, void* stream)
+{
+    return pileup_counts(reads, ref_dev, contig_len, region_start, region_len, nullptr, -1, params, counts_dev, flags_dev,
+                         workspace_dev, workspace_bytes, status_dev, stream);
+}
+
+size_t nsnp_pileup_targets_workspace_bytes(int64_t n_reads, int64_t n_cigar, int64_t region_len, int64_t n_targets) {
+    Workspace w; size_t total = 0;
+    carve(nullptr, n_reads < 0 ? 0 : n_reads, n_cigar < 0 ? 0 : n_cigar, region_len < 0 ? 0 : region_len, tile_shift_for(region_len), &w, &total,
+          n_targets < 0 ? 0 : n_targets);
+    return total;
+}
+
+int nsnp_pileup_counts_targets(const nsnp_reads_t* reads, const uint8_t* ref_dev, int64_t contig_len, int64_t region_start,
+                               int64_t region_len, const int32_t* targets, int64_t n_targets, const nsnp_params_t* params,
+                               int32_t* counts_dev, uint8_t* flags_dev, void* workspace_dev, size_t workspace_bytes,
+                               int32_t* status_dev, void* stream)
+{
+    if (n_targets < 0) return set_error(NSNP_E_INVALID, "nsnp_pileup_counts_targets: negative interval count");
+    return pileup_counts(reads, ref_dev, contig_len, region_start, region_len, targets, n_targets, params, counts_dev, flags_dev,
+                         workspace_dev, workspace_bytes, status_dev, stream);
 }
 
 }  // extern "C"

@@ -19,7 +19,24 @@ struct SelArgs {
     const uint8_t* flags;      // [region_len]
     int64_t region_start, region_len;
     int64_t emit_start, emit_end;      // contig coordinates
+    const int32_t* targets;            // nullptr, or n_targets sorted disjoint [start, end) pairs (contig coordinates)
+    int n_targets;
 };
+
+// target bits of the 8 positions [c0, c0 + 8): binary search for the first interval ending after c0, then at most 8 more
+// (intervals are non-empty and disjoint)
+__device__ __forceinline__ uint32_t target_mask8(const SelArgs& a, int64_t c0) {
+    int lo = 0, hi = a.n_targets;
+    while (lo < hi) { const int mid = (lo + hi) >> 1; if (__ldg(a.targets + 2 * mid + 1) > c0) hi = mid; else lo = mid + 1; }
+    uint32_t t = 0;
+    for (int k = lo; k < a.n_targets; ++k) {
+        const int64_t s = __ldg(a.targets + 2 * k), e = __ldg(a.targets + 2 * k + 1);
+        if (s >= c0 + 8) break;
+        const int b0 = (int)(max(s, c0) - c0), b1 = (int)(min(e, c0 + 8) - c0);
+        t |= ((1u << (b1 - b0)) - 1u) << b0;
+    }
+    return t;
+}
 
 // 8-bit candidate mask of positions [seg0 + 8*tid, +8): bit j set <=> site
 __device__ __forceinline__ uint32_t cand_mask8(const SelArgs& a, int64_t seg0, uint32_t* covw /* smem, (kSeg+64)/32 + 2 words */) {
@@ -63,6 +80,7 @@ __device__ __forceinline__ uint32_t cand_mask8(const SelArgs& a, int64_t seg0, u
         const uint32_t hi = (covw[(b >> 5) + 1] >> (b & 31)) & 1u;
         if (lo == 0xFFFFFFFFu && hi) m |= 1u << j;
     }
+    if (a.targets && m) m &= target_mask8(a, a.region_start + i0);
     return m;
 }
 
@@ -219,10 +237,14 @@ size_t nsnp_select_workspace_bytes(int64_t region_len) {
     return (size_t)(n_seg + 1) * 4 + 256;
 }
 
-int nsnp_select_candidates(const int32_t* counts_dev, uint8_t* flags_dev, const uint8_t* ref_dev, int64_t contig_len,
-                           int64_t region_start, int64_t region_len, int64_t emit_start, int64_t emit_end,
-                           const nsnp_params_t* params, int recompute_gate, int32_t* pos_dev, int64_t capacity,
-                           int32_t* n_dev, void* workspace_dev, size_t workspace_bytes, int32_t* status_dev, void* stream_)
+}  // extern "C"
+
+// targets == nullptr && n_targets < 0: every position of the emit range (nsnp_select_candidates)
+static int select_candidates(const int32_t* counts_dev, uint8_t* flags_dev, const uint8_t* ref_dev, int64_t contig_len,
+                             int64_t region_start, int64_t region_len, int64_t emit_start, int64_t emit_end,
+                             const int32_t* targets, int64_t n_targets, const nsnp_params_t* params, int recompute_gate,
+                             int32_t* pos_dev, int64_t capacity, int32_t* n_dev, void* workspace_dev, size_t workspace_bytes,
+                             int32_t* status_dev, void* stream_)
 {
     cudaStream_t stream = (cudaStream_t)stream_;
     if (!flags_dev || !pos_dev || !n_dev || !workspace_dev || !status_dev || !params)
@@ -230,22 +252,57 @@ int nsnp_select_candidates(const int32_t* counts_dev, uint8_t* flags_dev, const 
     if (recompute_gate && (!counts_dev || !ref_dev)) return set_error(NSNP_E_INVALID, "nsnp_select_candidates: recompute_gate needs counts and ref");
     if (region_start < 0 || region_len < 0 || region_start + region_len > contig_len || capacity < 0)
         return set_error(NSNP_E_INVALID, "nsnp_select_candidates: bad region");
-    if (workspace_bytes < nsnp_select_workspace_bytes(region_len)) return set_error(NSNP_E_WORKSPACE, "select workspace too small");
+    if (n_targets >= 0) {
+        if (int e = check_targets("nsnp_select_candidates_targets", targets, n_targets, region_start, region_start + region_len)) return e;
+    }
+    const size_t ws_need = n_targets >= 0 ? nsnp_select_targets_workspace_bytes(region_len, n_targets) : nsnp_select_workspace_bytes(region_len);
+    if (workspace_bytes < ws_need) return set_error(NSNP_E_WORKSPACE, "select workspace too small");
     if (nsnp_device_count() == 0) return set_error(NSNP_E_NO_DEVICE, "no CUDA device (there is no CPU fallback)");
-    if (region_len == 0 || emit_end <= emit_start) { cudaMemsetAsync(n_dev, 0, 4, stream); return cuda_status("memset n"); }
+    if (region_len == 0 || emit_end <= emit_start || n_targets == 0) { cudaMemsetAsync(n_dev, 0, 4, stream); return cuda_status("memset n"); }
     if (recompute_gate) {
         int blocks = (int)((region_len + 255) / 256); if (blocks > kNumSMs * 16) blocks = kNumSMs * 16;
         regate_kernel<<<blocks, 256, 0, stream>>>(counts_dev, flags_dev, ref_dev, region_start, region_len, *params);
         if (int e = cuda_status("regate_kernel")) return e;
     }
     ProfScope prof(NSNP_PROF_SELECT, stream);
-    SelArgs a{flags_dev, region_start, region_len, emit_start, emit_end};
+    SelArgs a{flags_dev, region_start, region_len, emit_start, emit_end, nullptr, 0};
     const int n_seg = (int)((region_len + kSeg - 1) / kSeg);
     int32_t* seg = (int32_t*)workspace_dev;
+    if (n_targets > 0) {                        // the interval copy sits behind the segment counts
+        int32_t* iv = (int32_t*)((char*)workspace_dev + nsnp_select_workspace_bytes(region_len));
+        cudaMemcpyAsync(iv, targets, (size_t)n_targets * 8, cudaMemcpyHostToDevice, stream);
+        a.targets = iv; a.n_targets = (int)n_targets;
+    }
     select_count_kernel<<<n_seg, kSelThreads, 0, stream>>>(a, seg);
     select_scan_kernel<<<1, 1024, 0, stream>>>(seg, n_seg, n_dev, capacity, status_dev);
     select_write_kernel<<<n_seg, kSelThreads, 0, stream>>>(a, seg, pos_dev, capacity);
     return cuda_status("select kernels");
+}
+
+extern "C" {
+
+int nsnp_select_candidates(const int32_t* counts_dev, uint8_t* flags_dev, const uint8_t* ref_dev, int64_t contig_len,
+                           int64_t region_start, int64_t region_len, int64_t emit_start, int64_t emit_end,
+                           const nsnp_params_t* params, int recompute_gate, int32_t* pos_dev, int64_t capacity,
+                           int32_t* n_dev, void* workspace_dev, size_t workspace_bytes, int32_t* status_dev, void* stream)
+{
+    return select_candidates(counts_dev, flags_dev, ref_dev, contig_len, region_start, region_len, emit_start, emit_end, nullptr, -1,
+                             params, recompute_gate, pos_dev, capacity, n_dev, workspace_dev, workspace_bytes, status_dev, stream);
+}
+
+size_t nsnp_select_targets_workspace_bytes(int64_t region_len, int64_t n_targets) {
+    return nsnp_select_workspace_bytes(region_len) + (size_t)(n_targets < 0 ? 0 : n_targets) * 8 + 256;
+}
+
+int nsnp_select_candidates_targets(const int32_t* counts_dev, uint8_t* flags_dev, const uint8_t* ref_dev, int64_t contig_len,
+                                   int64_t region_start, int64_t region_len, int64_t emit_start, int64_t emit_end,
+                                   const int32_t* targets, int64_t n_targets, const nsnp_params_t* params, int recompute_gate,
+                                   int32_t* pos_dev, int64_t capacity, int32_t* n_dev, void* workspace_dev, size_t workspace_bytes,
+                                   int32_t* status_dev, void* stream)
+{
+    if (n_targets < 0) return set_error(NSNP_E_INVALID, "nsnp_select_candidates_targets: negative interval count");
+    return select_candidates(counts_dev, flags_dev, ref_dev, contig_len, region_start, region_len, emit_start, emit_end, targets,
+                             n_targets, params, recompute_gate, pos_dev, capacity, n_dev, workspace_dev, workspace_bytes, status_dev, stream);
 }
 
 int nsnp_gather_windows(const int32_t* counts_dev, const uint8_t* ref_dev, int64_t region_start, int64_t region_len,

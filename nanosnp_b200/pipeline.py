@@ -42,6 +42,14 @@ class RegionResult:
     zy: Optional[torch.Tensor]  # float32 [n,3]
 
 
+def _intervals(targets) -> np.ndarray:
+    """[k, 2] int32 host copy of target intervals (the library checks order, overlap and range)."""
+    a = np.asarray(targets)
+    if a.size and (a.min() < np.iinfo(np.int32).min or a.max() > np.iinfo(np.int32).max):
+        raise _lib.NsnpError(_lib.E_INVALID, "target interval outside the int32 contig coordinates")
+    return np.ascontiguousarray(a.reshape(-1, 2), dtype=np.int32)
+
+
 class PileupEngine:
     """One engine per GPU / process.  Buffers are grown on demand and reused across regions."""
 
@@ -65,7 +73,9 @@ class PileupEngine:
 
     # -- s1 step A ---------------------------------------------------------------------------------
     def pileup_counts(self, reads: PackedReads, ref: torch.Tensor, region_start: int = 0, region_len: Optional[int] = None,
-                      counts: Optional[torch.Tensor] = None, flags: Optional[torch.Tensor] = None):
+                      counts: Optional[torch.Tensor] = None, flags: Optional[torch.Tensor] = None, targets: Optional[np.ndarray] = None):
+        """targets: optional [k, 2] sorted disjoint [start, end) contig intervals: only the tiles holding a position within 16 bp
+        of an interval are computed; every other position gets flags 0 and an unwritten count row."""
         contig_len = int(ref.shape[0])
         if region_len is None:
             region_len = contig_len - region_start
@@ -74,6 +84,15 @@ class PileupEngine:
         if flags is None:
             flags = torch.empty(region_len, dtype=torch.uint8, device=self.device)
         st = reads.as_struct()
+        if targets is not None:
+            iv = _intervals(targets)
+            ws = self._workspace("pileup", self.lib.nsnp_pileup_targets_workspace_bytes(st.n_reads, st.n_cigar, region_len, len(iv)))
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.nsnp_pileup_counts_targets(C.byref(st), ref.data_ptr(), contig_len, region_start, region_len,
+                                                               iv.ctypes.data, len(iv), C.byref(self.params), counts.data_ptr(),
+                                                               flags.data_ptr(), ws.data_ptr(), ws.numel(), self.status.data_ptr(),
+                                                               _stream(self.device)))
+            return counts, flags
         need = self.lib.nsnp_pileup_workspace_bytes(st.n_reads, st.n_cigar, region_len)
         ws = self._workspace("pileup", need)
         with torch.cuda.device(self.device):
@@ -85,12 +104,22 @@ class PileupEngine:
     # -- s1 step B ---------------------------------------------------------------------------------
     def select(self, flags: torch.Tensor, ref: torch.Tensor, region_start: int, emit_start: int, emit_end: int,
                capacity: int, counts: Optional[torch.Tensor] = None, recompute_gate: bool = False,
-               pos: Optional[torch.Tensor] = None, n_dev: Optional[torch.Tensor] = None):
+               pos: Optional[torch.Tensor] = None, n_dev: Optional[torch.Tensor] = None, targets: Optional[np.ndarray] = None):
+        """targets: optional [k, 2] sorted disjoint [start, end) contig intervals: only sites inside them are selected."""
         region_len = int(flags.shape[0])
         if pos is None:
             pos = torch.empty(max(capacity, 1), dtype=torch.int32, device=self.device)
         if n_dev is None:
             n_dev = torch.zeros(1, dtype=torch.int32, device=self.device)
+        if targets is not None:
+            iv = _intervals(targets)
+            ws = self._workspace("select", self.lib.nsnp_select_targets_workspace_bytes(region_len, len(iv)))
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.nsnp_select_candidates_targets(
+                    0 if counts is None else counts.data_ptr(), flags.data_ptr(), ref.data_ptr(), int(ref.shape[0]), region_start,
+                    region_len, emit_start, emit_end, iv.ctypes.data, len(iv), C.byref(self.params), int(recompute_gate), pos.data_ptr(),
+                    capacity, n_dev.data_ptr(), ws.data_ptr(), ws.numel(), self.status.data_ptr(), _stream(self.device)))
+            return pos, n_dev
         ws = self._workspace("select", self.lib.nsnp_select_workspace_bytes(region_len))
         with torch.cuda.device(self.device):
             _lib.check(self.lib.nsnp_select_candidates(0 if counts is None else counts.data_ptr(), flags.data_ptr(), ref.data_ptr(),

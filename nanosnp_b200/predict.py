@@ -12,6 +12,7 @@ from __future__ import annotations
 import argparse
 import ctypes as C
 import os
+import sys
 
 import numpy as np
 import torch
@@ -61,26 +62,35 @@ def _read_inputs(testing_paths, only=None):
                 yield contig, reads, None, -1
 
 
-def _region_reads(reads, reader, rid, regions):
+def _region_reads(reads, reader, rid, regions, targets=None):
+    """Reads of each region: fetched through the .bai (with targets: only the reads near the unit's intervals), else the
+    contiguous slice of the in-memory reads that can overlap the region's computed span."""
     from .reads import max_reference_span, slice_reads
-    from .shard import read_range_for_region
+    from .shard import fetch_ranges, read_range_for_region
     if reader is not None:
+        if targets is not None:
+            return [reader.fetch_ranges(rid, fetch_ranges(rg, iv)) for rg, iv in zip(regions, targets)]
         return [reader.fetch(rid, rg.start, rg.end) for rg in regions]
     span = max_reference_span(reads) + 1
     return [slice_reads(reads, *read_range_for_region(reads.pos, span, rg)) for rg in regions]
 
 
-def predict(model: LSTMNetwork, testing_paths, reference_index_file, batch_size, output_file, device, reference=None, region_len=12_500_000):
+def predict(model: LSTMNetwork, testing_paths, reference_index_file, batch_size, output_file, device, reference=None, region_len=12_500_000,
+            targets=None):
     """predict.py:37-195.  `.pd` text files: windows -> model -> records.  Read inputs (`.bam`, `.reads.npz`): the whole
     s1 + s2 path incl. the VCF text runs on the GPU region by region (caller.call_contig_text); under torchrun every rank
     computes and formats its LPT share of the regions and writes its own segments of the one output file
-    (caller.write_sharded_vcf)."""
+    (caller.write_sharded_vcf).
+    targets: None (every position), or contig -> merged [k, 2] 0-based [start, end) intervals (targets.build_targets): only
+    sites inside them are called, and the GPU computes only the pileup tiles near them.  The VCF is the one the reference
+    writes from `.pd` files holding only those sites (batches are consecutive kept sites)."""
     import io
     from .caller import call_contig_text, write_sharded_vcf, _pinned
     from .dataset import load_fasta
     from .pipeline import PileupEngine
     from .runner import RegionRunner
-    from .shard import assign_lpt, plan_regions
+    from .shard import assign_lpt, listed_tiles, plan_regions, plan_target_units
+    from .targets import in_targets
     runner = None
     fasta = None
 
@@ -106,8 +116,12 @@ def predict(model: LSTMNetwork, testing_paths, reference_index_file, batch_size,
         fasta = load_fasta(reference)
         with open(reference_index_file) as f:
             contigs = [(l.split()[0], int(l.split()[1])) for l in f if l.strip()]
-        regions = plan_regions(contigs, region_len)
-        mine = assign_lpt(regions, world)[rank]
+        if targets is None:
+            regions, unit_iv = plan_regions(contigs, region_len), None
+            mine = assign_lpt(regions, world)[rank]
+        else:
+            regions, unit_iv = plan_target_units(contigs, targets, region_len)
+            mine = assign_lpt(regions, world, [len(listed_tiles(rg, iv)) for rg, iv in zip(regions, unit_iv)])[rank]
         need = {regions[i].contig for i in mine}
         index_of = {name: ci for ci, (name, _) in enumerate(contigs)}
         recs = {}
@@ -119,11 +133,12 @@ def predict(model: LSTMNetwork, testing_paths, reference_index_file, batch_size,
             if not idx:
                 continue
             rgs = [regions[i] for i in idx]
-            host = [_pinned(r) for r in _region_reads(reads, reader, rid, rgs)]
+            ivs = None if unit_iv is None else [unit_iv[i] for i in idx]
+            host = [_pinned(r) for r in _region_reads(reads, reader, rid, rgs, ivs)]
             ref_dev = torch.from_numpy(np.ascontiguousarray(fasta[contig])).to(device)
             r = get_runner()
-            for i, rg, hr in zip(idx, rgs, host):
-                out = r.run_device(r.upload(hr), ref_dev, rg)
+            for k, (i, rg, hr) in enumerate(zip(idx, rgs, host)):
+                out = r.run_device(r.upload(hr), ref_dev, rg, targets=None if ivs is None else ivs[k])
                 recs[i] = out.rec.clone()                    # records stay on this GPU until the text is made
         for i in mine:
             recs.setdefault(i, torch.zeros((0, 32), dtype=torch.uint8, device=device))
@@ -141,6 +156,13 @@ def predict(model: LSTMNetwork, testing_paths, reference_index_file, batch_size,
                 names = dataset.contig_names
                 if any(nm != names[0] for nm in names):
                     raise NotImplementedError("one predict-data file must hold one contig (as make_predict_data.sh writes them)")
+                if targets is not None:                       # POS is 1-based
+                    keep = in_targets(np.asarray(dataset.positions, np.int64) - 1, targets.get(names[0]))
+                    if not keep.any():
+                        continue
+                    dataset.position_matrix = np.ascontiguousarray(dataset.position_matrix[keep])
+                    dataset.positions = np.asarray(dataset.positions)[keep]
+                    dataset.reference_bases = np.asarray(dataset.reference_bases)[keep]
                 x = torch.from_numpy(dataset.position_matrix).to(device)
                 gt, zy = model.predict(x)
                 cov8 = x[:, 16, COV_CHANNELS].to(torch.float32)
@@ -151,14 +173,17 @@ def predict(model: LSTMNetwork, testing_paths, reference_index_file, batch_size,
             if reference is None:
                 raise ValueError("read inputs need the reference FASTA")
             fasta = load_fasta(reference)
-            for contig, reads, reader, rid in _read_inputs(read_paths):
+            for contig, reads, reader, rid in _read_inputs(read_paths, None if targets is None else set(targets)):
                 if contig not in fasta:
                     if reader is not None:
                         continue                              # an indexed BAM lists every @SQ; only contigs of the FASTA are called
                     raise KeyError(f"contig {contig} is not in the reference")
-                regions = plan_regions([(contig, len(fasta[contig]))], region_len)
+                if targets is None:
+                    regions, unit_iv = plan_regions([(contig, len(fasta[contig]))], region_len), None
+                else:
+                    regions, unit_iv = plan_target_units([(contig, len(fasta[contig]))], targets, region_len)
                 call_contig_text(get_runner(), reads, fasta[contig], contig, fwriter, batch_size, region_len, regions,
-                                 _region_reads(reads, reader, rid, regions))
+                                 _region_reads(reads, reader, rid, regions, unit_iv), unit_iv)
         model._forward().reevaluated()                          # f16x1: raises if a region had more low-margin sites than are re-run
 
 
@@ -174,6 +199,9 @@ def main(argv=None):
     parser.add_argument("--precision", default="f16x3", choices=["fp32", "f16x3", "f16x1"],
                         help="f16x1: single-pass tensor-core LSTM, low-margin sites re-evaluated in f16x3 (same calls, QUAL may move by ~0.06)")
     parser.add_argument("--region_len", type=int, default=12_500_000, help="positions per GPU work unit (read inputs)")
+    parser.add_argument("--bed", default=None, help="call only inside these intervals (BED: 0-based, half-open; first three fields)")
+    parser.add_argument("--region", action="append", default=[],
+                        help="call only inside CTG or CTG:START-END (1-based, inclusive); repeatable, combines with --bed")
     opt = parser.parse_args(argv)
     if opt.no_cuda:
         raise SystemExit("nanosnp_b200.predict: --no_cuda is not supported (no CPU fallback); use the reference's predict.py on CPU")
@@ -207,8 +235,15 @@ def main(argv=None):
     else:
         testing_paths = sorted(opt.data + "/" + f for f in os.listdir(opt.data) if f.endswith((".pd", ".reads.npz", ".bam")))
     assert os.path.exists(opt.reference + ".fai"), "reference index file does not exist."
+    targets = None
+    if opt.bed is not None or opt.region:
+        from .targets import build_targets
+        with open(opt.reference + ".fai") as f:
+            contigs = [(l.split()[0], int(l.split()[1])) for l in f if l.strip()]
+        quiet = int(os.environ.get("RANK", "0")) != 0                   # report skipped intervals once, not once per rank
+        targets = build_targets(contigs, opt.bed, opt.region, report=None if quiet else sys.stderr)
     predict(pred_model, testing_paths, opt.reference + ".fai", opt.batch_size, opt.output, device, reference=opt.reference,
-            region_len=opt.region_len)
+            region_len=opt.region_len, targets=targets)
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
         import torch.distributed as dist
         dist.barrier()

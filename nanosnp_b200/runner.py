@@ -87,21 +87,25 @@ class RegionRunner:
             self._bufs[key] = t
         return t[:n].view(*shape)
 
-    def run_device(self, reads: PackedReads, ref: torch.Tensor, region: Region, timer: Optional[StageTimer] = None) -> RegionOutput:
+    def run_device(self, reads: PackedReads, ref: torch.Tensor, region: Region, timer: Optional[StageTimer] = None,
+                   targets: Optional[np.ndarray] = None) -> RegionOutput:
+        """targets: the unit's [k, 2] sorted disjoint [start, end) intervals (contig coordinates, inside the emit span), or None
+        for every position of the region.  With targets only the tiles near them are computed and only sites inside them
+        are kept; the launch count does not depend on k."""
         eng = self.eng
         rlen = region.length
         timer = timer or StageTimer(False)
         counts = self._buf("counts", (rlen, _lib.CHANNELS), torch.int32)
         flags = self._buf("flags", (rlen,), torch.uint8)
         timer.start("pileup")
-        eng.pileup_counts(reads, ref, region.start, rlen, counts=counts, flags=flags)
+        eng.pileup_counts(reads, ref, region.start, rlen, counts=counts, flags=flags, targets=targets)
         timer.stop()
-        self.launches += 2 if reads.n_reads else 1
+        self.launches += (2 if reads.n_reads else 1) + (targets is not None)
         cap = max(1024, region.emit_end - region.emit_start)
         pos = self._buf("pos", (cap,), torch.int32)
         n_dev = self._buf("n", (1,), torch.int32)
         timer.start("select")
-        eng.select(flags, ref, region.start, region.emit_start, region.emit_end, cap, pos=pos, n_dev=n_dev)
+        eng.select(flags, ref, region.start, region.emit_start, region.emit_end, cap, pos=pos, n_dev=n_dev, targets=targets)
         timer.stop()
         self.launches += 3
         if self.blocking_sync:
@@ -154,10 +158,11 @@ class RegionRunner:
         return RegionOutput(n, pos[:n], refbase, cov8, gt, zy, x if self.keep_windows else None)
 
     # ---- host-buffer mode, pipelined: H2D of region k+1 and D2H of region k-1 overlap the kernels of region k ----
-    def run_host_many(self, host_regions, regions, ref: torch.Tensor, host_outs, consume=None):
+    def run_host_many(self, host_regions, regions, ref: torch.Tensor, host_outs, consume=None, targets=None):
         """host_regions: PackedReads of pinned host tensors, one per region; host_outs: two dicts of pinned result
         buffers (double buffered).  consume(k, result_dict) is called on the host once region k's results have landed
-        (e.g. VCF formatting); it runs while the GPU works on later regions.  Returns the total site count."""
+        (e.g. VCF formatting); it runs while the GPU works on later regions.  targets: optional per-region intervals (run_device).
+        Returns the total site count."""
         dev = self.device
         main = torch.cuda.current_stream(dev)
         if not hasattr(self, "_copy_streams"):
@@ -198,7 +203,7 @@ class RegionRunner:
                     raise RuntimeError("pipeline order")
                 start_upload(k + 1)
             main.wait_event(up_done[k])
-            out = self.run_device(dev_reads[k], ref, regions[k])
+            out = self.run_device(dev_reads[k], ref, regions[k], targets=None if targets is None else targets[k])
             ev = torch.cuda.Event(); ev.record(main); comp_done[k] = ev
             # results: device -> device staging (so the next region can reuse the work buffers) -> pinned host
             ho = host_outs[k % 2]
@@ -224,11 +229,11 @@ class RegionRunner:
         return total
 
     # ---- host-buffer mode with the VCF text assembled on the GPU ---------------------------------------------------------
-    def run_host_text(self, host_regions, regions, ref: torch.Tensor, textgen, write) -> int:
+    def run_host_text(self, host_regions, regions, ref: torch.Tensor, textgen, write, targets=None) -> int:
         """Pinned host read arrays of consecutive regions of ONE contig -> H2D -> kernels -> compact records -> VCF text on
         the GPU (vcf_text.GpuVcfText, which carries partial 1000-site batches across regions) -> D2H of the text.
         write(memoryview) receives the text chunks in order.  H2D of region k+1 and D2H of chunk k-1 overlap the kernels of
-        region k; the host does no per-record work.  Returns the site count."""
+        region k; the host does no per-record work.  targets: optional per-region intervals (run_device).  Returns the site count."""
         assert self.records, "run_host_text needs a RegionRunner(records=True)"
         dev = self.device
         main = torch.cuda.current_stream(dev)
@@ -256,7 +261,7 @@ class RegionRunner:
             if k + 1 < n_reg:
                 start_upload(k + 1)
             main.wait_event(up_done[k])
-            out = self.run_device(dev_reads[k], ref, regions[k])
+            out = self.run_device(dev_reads[k], ref, regions[k], targets=None if targets is None else targets[k])
             chunk = textgen.push(out.rec) if out.n else None        # copies the records: the work buffers are free again
             self.launches += 3 if chunk is not None else 0
             ev = torch.cuda.Event(); ev.record(main); comp_done[k] = ev
@@ -273,7 +278,7 @@ class RegionRunner:
         return total
 
     # ---- host-buffer mode, records kept on the device (multi-GPU: the text is made after the count / head exchange) ----------
-    def run_host_collect(self, host_regions, regions, refs, on_region=None) -> list:
+    def run_host_collect(self, host_regions, regions, refs, on_region=None, targets=None) -> list:
         """Pinned host reads of arbitrary regions (refs[k]: the device reference of region k's contig) -> H2D -> kernels ->
         compact records, returned as one device tensor per region -- or handed to on_region(k, RegionOutput) right after region
         k's kernels were enqueued (e.g. ShardedVcfWriter.add_region).  The H2D of region k+1 overlaps the kernels of region k."""
@@ -300,7 +305,7 @@ class RegionRunner:
             if k + 1 < n_reg:
                 start_upload(k + 1)
             main.wait_event(up_done[k])
-            o = self.run_device(dev_reads[k], refs[k], regions[k])
+            o = self.run_device(dev_reads[k], refs[k], regions[k], targets=None if targets is None else targets[k])
             if on_region is not None:
                 on_region(k, o)
                 out[k] = o.n

@@ -51,15 +51,71 @@ def plan_regions(contigs: Sequence[Tuple[str, int]], region_len: int) -> List[Re
     return out
 
 
-def assign_lpt(regions: Sequence[Region], world_size: int) -> List[List[int]]:
-    """Longest-processing-time-first assignment of regions to ranks (balances 25 unequal contigs).
+def plan_target_units(contigs: Sequence[Tuple[str, int]], targets: Dict[str, np.ndarray],
+                      region_len: int) -> Tuple[List[Region], List[np.ndarray]]:
+    """Work units of a targeted run.  targets: contig -> merged, sorted [k, 2] [start, end) intervals.  An interval longer
+    than region_len is cut like plan_regions cuts a contig; consecutive intervals (or pieces) share a unit while the unit's
+    emitted span [first start, last end) stays <= region_len.  Units have disjoint emit spans in contig order.  Returns the
+    units and, aligned with them, each unit's intervals as int64 [k, 2] (kept out of the hashed Region)."""
+    units: List[Region] = []
+    unit_iv: List[np.ndarray] = []
+    for ci, (name, L) in enumerate(contigs):
+        iv = targets.get(name)
+        if iv is None or len(iv) == 0:
+            continue
+        pieces = []
+        for s, e in np.asarray(iv, np.int64).reshape(-1, 2).tolist():
+            n = max(1, -(-(e - s) // region_len))
+            step = -(-(e - s) // n)
+            pieces += [(s + k * step, min(e, s + (k + 1) * step)) for k in range(n) if s + k * step < e]
+        cur: List[Tuple[int, int]] = []
+        for s, e in pieces + [(None, None)]:
+            if cur and (s is None or e - cur[0][0] > region_len):
+                units.append(Region(name, ci, L, cur[0][0], cur[-1][1]))
+                unit_iv.append(np.array(cur, np.int64))
+                cur = []
+            if s is not None:
+                cur.append((s, e))
+    return units, unit_iv
+
+
+def listed_tiles(region: Region, intervals: np.ndarray, tile: int = 1024) -> np.ndarray:
+    """The tiles (indices from region.start) the GPU computes for a unit: those holding any position of [start-16, end+16)
+    of an interval, clipped to the unit's computed span."""
+    iv = np.asarray(intervals, np.int64).reshape(-1, 2)
+    a = np.maximum(iv[:, 0] - FLANK, region.start) - region.start
+    b = np.minimum(iv[:, 1] + FLANK, region.end) - region.start
+    keep = a < b
+    n_tiles = -(-region.length // tile)
+    diff = np.zeros(n_tiles + 1, np.int64)
+    np.add.at(diff, a[keep] // tile, 1)
+    np.add.at(diff, (b[keep] - 1) // tile + 1, -1)
+    return np.nonzero(np.cumsum(diff[:n_tiles]) > 0)[0]
+
+
+def fetch_ranges(region: Region, intervals: np.ndarray) -> np.ndarray:
+    """[start-16, end+16) of every interval, clipped to the contig and merged: the reference ranges whose reads a unit needs."""
+    out: List[List[int]] = []
+    for s, e in np.asarray(intervals, np.int64).reshape(-1, 2).tolist():
+        s, e = max(0, s - FLANK), min(region.contig_len, e + FLANK)
+        if out and s <= out[-1][1]:
+            out[-1][1] = max(out[-1][1], e)
+        else:
+            out.append([s, e])
+    return np.array(out, np.int64).reshape(-1, 2)
+
+
+def assign_lpt(regions: Sequence[Region], world_size: int, weights: Sequence[int] = None) -> List[List[int]]:
+    """Longest-processing-time-first assignment of regions to ranks (balances 25 unequal contigs).  weights: optional cost of
+    each region (a targeted run passes its listed tiles); default: the computed span.
     Deterministic; returns per-rank lists of region indices, each in (contig, position) order."""
-    order = sorted(range(len(regions)), key=lambda i: (-regions[i].length, i))
+    w = [rg.length for rg in regions] if weights is None else [int(x) for x in weights]
+    order = sorted(range(len(regions)), key=lambda i: (-w[i], i))
     load = [0] * world_size
     mine: List[List[int]] = [[] for _ in range(world_size)]
     for i in order:
         r = min(range(world_size), key=lambda k: (load[k], k))
-        load[r] += regions[i].length
+        load[r] += w[i]
         mine[r].append(i)
     for m in mine:
         m.sort()
