@@ -24,7 +24,8 @@
 // CG = 2 pairs two CTAs (cta_group::2): M = 256, each CTA holds half of W (N/2 rows) -- that is what makes the
 // layer-1 weights (2 x 96 KB) fit; the leader CTA issues the MMAs, tcgen05.commit multicasts completion.
 //
-// Kernels: lstm0_pair2_kernel (layer 0, production), lstm_tc_kernel<1,2,4> (layer 1, production),
+// Kernels: lstm0_pair2_kernel (layer 0, production), lstm1_pair2x3_kernel (layer 1, production), lstm1_pair2_kernel
+// (layer 1, single-pass NSNP_PREC_F16X1), lstm_tc_kernel<1,2,4> (layer-1 alternative NSNP_L1_VARIANT=0 and the debug entry),
 // lstm_tc_kernel<0,...> (layer-0 alternative NSNP_L0_VARIANT=0 and the raw-accumulator debug entry), tail_tc_kernel.
 #include <cuda_fp16.h>
 #include <stdlib.h>
@@ -746,14 +747,255 @@ lstm1_pair2_kernel(const unsigned char* __restrict__ blob, const __half* __restr
     if (threadIdx.x < 32) tmem_dealloc<2>(*tmem_slot, 512);
 }
 
+// ------------------------------------------------------------------------------------------------------------------
+// Layer 1, three-pass (default NSNP_PREC_F16X3) variant with the same two-groups-per-CTA alternation.  Two groups' full
+// operands (2 x 96 KB) next to W hi + lo (96 KB) would not fit, but the input part of the operand (the layer-0 output,
+// 128 of the 192 columns) is only read during its own group's MMA burst and the bursts strictly alternate: the two groups
+// share ONE input buffer and keep only their h part (64 columns, hi + lo) to themselves.  The input buffer is refilled
+// per burst by a producer warp in two halves, each with a full and an empty mbarrier:
+//     hi half (passes 0 and 1 read it): empty once pass 1 of the input part has completed -- the copy of the other group's
+//             rows overlaps pass 2 and the 12 h-part MMAs;
+//     lo half (pass 2 reads it): empty once pass 2 of the input part has completed.
+// The full barriers exist per group (a group waits for its own rows only, one phase per step of that group); warp 0 of the
+// group waits for them before it reports the group ready, so barReady covers "both CTAs' input rows have landed".  Same MMA
+// order (input part: 3 passes over kb 0-7, then h part: 3 passes over kb 8-11) and cell arithmetic as lstm_tc_kernel<1>:
+// bit-identical output.
+constexpr int kP2x3Threads = kP2Threads + 32;                   // + the producer warp
+struct P2Smem1x3 {
+    static constexpr size_t b_bytes = (size_t)kTcK1 * 128 * 2;                  // this CTA's half of W, one of hi / lo
+    static constexpr size_t in_bytes = (size_t)kTcIn1 * kRows * 2;             // input part, one of hi / lo (shared by both groups)
+    static constexpr size_t h_bytes = (size_t)kH * kRows * 2;                  // one group's h part, one of hi / lo
+    static constexpr size_t off_bhi = 0, off_blo = b_bytes, off_in = 2 * b_bytes, off_h = off_in + 2 * in_bytes,
+                            off_bias = off_h + 4 * h_bytes, off_bar = off_bias + 256 * sizeof(float), total = off_bar + 128;
+};
+static_assert(P2Smem1x3::total <= 232448, "lstm1_pair2x3_kernel: shared memory above the per-block opt-in limit");
+
+__global__ void __launch_bounds__(kP2x3Threads, 1)
+lstm1_pair2x3_kernel(const unsigned char* __restrict__ blob, const __half* __restrict__ h0_in, float* __restrict__ h16, int64_t n)
+{
+    using S = P2Smem1x3;
+    constexpr int K = kTcK1, IN = kTcIn1, KB = K / 16, XB = IN / 16, RB = 128, UB = 4, kS = TcCfg<1>::STEPS;
+    constexpr uint32_t LBO_A = kRows * 16, LBO_B = RB * 16, SBO = 128;
+    constexpr uint32_t kPartBytes = 16u * kRows * 16u;              // 32 KB: the hi (or lo) half of one (tile, position) of the layer-0 output
+    extern __shared__ __align__(1024) unsigned char smem[];
+    const bool producer = threadIdx.x >= kP2Threads;               // warp-uniform
+    const int grp = producer ? 0 : (int)threadIdx.x / kP2GroupThreads;
+    const int tid = (int)threadIdx.x - grp * kP2GroupThreads, lane = tid & 31, warp = tid >> 5;
+    unsigned char* sBhi = smem + S::off_bhi; unsigned char* sBlo = smem + S::off_blo;
+    unsigned char* sInHi = smem + S::off_in; unsigned char* sInLo = sInHi + S::in_bytes;
+    unsigned char* sHhi = smem + S::off_h + grp * 2 * S::h_bytes; unsigned char* sHlo = sHhi + S::h_bytes;
+    float* sBias = reinterpret_cast<float*>(smem + S::off_bias);
+    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + S::off_bar);
+    uint64_t* barH = bars + grp;               // [0,1]   gates of this group complete (commit, multicast to both CTAs)
+    uint64_t* barReady = bars + 2 + grp;       // [2,3]   leader CTA: all 16 warps of this group (both CTAs) are ready, input rows landed
+    uint64_t* barTurn = bars + 4;              // [4,5]   leader CTA: token, barTurn[g] = "group g may issue"
+    uint64_t* barHiFull = bars + 6;            // [6,7]   this CTA: the hi input rows of group g's next step have landed
+    uint64_t* barLoFull = bars + 8;            // [8,9]   this CTA: the lo input rows of group g's next step have landed
+    uint64_t* barHiEmpty = bars + 10;          // [10]    passes 0 and 1 of the last burst's input part are complete (multicast)
+    uint64_t* barLoEmpty = bars + 11;          // [11]    pass 2 of the last burst's input part is complete (multicast)
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + S::off_bar + 96);
+
+    const int quad = warp & 3, sub = warp >> 2;
+    const int row = quad * 32 + lane;
+    const uint32_t cta_rank = cluster_ctarank();
+    const int cluster_id = (int)(blockIdx.x >> 1);
+    const int dir = cluster_id & 1;
+    const int quad_stride = (int)(gridDim.x >> 2);
+    const int n_quads = (int)((n + 4 * kRows - 1) / (4 * kRows));
+    const int64_t last_tile = (n + kRows - 1) / kRows - 1;
+    const int q0 = cluster_id >> 1;
+    const int my_quads = q0 < n_quads ? (n_quads - q0 + quad_stride - 1) / quad_stride : 0;
+    const int total_g = my_quads * kS;                          // each group's stream of (quad, step) pairs; bursts alternate g0, g1, g0, ...
+    auto tile_of = [&](int qi, int g) -> int64_t { return (int64_t)(q0 + qi * quad_stride) * 4 + (int64_t)cta_rank * 2 + g; };
+
+    if (threadIdx.x == 0) {
+        mbar_init(bars + 0, 1); mbar_init(bars + 1, 1); mbar_init(bars + 2, 16); mbar_init(bars + 3, 16);
+        for (int i = 4; i < 12; ++i) mbar_init(bars + i, 1);
+        fence_mbar_init();
+    }
+    if (threadIdx.x < 32) tmem_alloc<2>(tmem_slot, 512);
+    {
+        const uint4* ghi = reinterpret_cast<const uint4*>(blob + tc_off(1, dir, 0));
+        const uint4* glo = reinterpret_cast<const uint4*>(blob + tc_off(1, dir, 1));
+        uint4* dhi = reinterpret_cast<uint4*>(sBhi); uint4* dlo = reinterpret_cast<uint4*>(sBlo);
+        for (int i = (int)threadIdx.x; i < (K / 8) * RB; i += kP2x3Threads) {
+            const int ch = i / RB, r = i - ch * RB;
+            const int g = ch * 256 + (int)cta_rank * RB + r;
+            dhi[i] = __ldg(ghi + g); dlo[i] = __ldg(glo + g);
+        }
+        const float* gb = reinterpret_cast<const float*>(blob + kOffTcBias1) + dir * 256;
+        for (int i = (int)threadIdx.x; i < 256; i += kP2x3Threads) sBias[i] = __ldg(gb + i);
+    }
+    __syncthreads();
+
+    // input rows of burst b (group b & 1, its stream element b >> 1): h0[tile][t][hi|lo][16 chunks][128 rows][8];
+    // a padding tile re-reads the last real one
+    auto rows_of = [&](int b) -> const __half* {
+        const int gs = b >> 1, qi = gs / kS, st = gs - qi * kS;
+        const int t = dir == 0 ? st : (kT - 1 - st);
+        const int64_t tile = min(tile_of(qi, b & 1), last_tile);
+        return h0_in + ((size_t)tile * kT + t) * (size_t)kPartBytes;       // kPartBytes halfs = hi + lo per (tile, t)
+    };
+    const int total_b = 2 * total_g;
+    if (producer && lane == 0 && total_b > 0) {                 // the first burst's rows: the buffer is free
+        const __half* src = rows_of(0);
+        mbar_expect_tx(barHiFull, kPartBytes); bulk_g2s(sInHi, src, kPartBytes, barHiFull);
+        mbar_expect_tx(barLoFull, kPartBytes); bulk_g2s(sInLo, src + kPartBytes / 2, kPartBytes, barLoFull);
+        if (total_b > 1) bulk_prefetch_l2(rows_of(1), 2 * kPartBytes);
+    }
+    auto report_ready = [&]() {
+        fence_async_smem();
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive_remote_relaxed(barReady, 0);      // the leader maps to itself
+    };
+    uint32_t phaseIn = 0;                                           // parity of this group's full barriers
+    auto wait_input = [&]() {                                       // warp 0 of a group: both halves of its next rows have landed
+        mbar_wait(barHiFull + grp, phaseIn);
+        mbar_wait(barLoFull + grp, phaseIn);
+        phaseIn ^= 1;
+    };
+    tc_fence_before();
+    cluster_sync_all();                                            // barriers initialised, TMEM allocated (both CTAs)
+    tc_fence_after();
+
+    if (producer) {
+        // producer warp: burst b's rows go into the buffer as soon as burst b - 1 has finished reading each half; it never
+        // touches TMEM and skips the epilogue
+        if (lane == 0) {
+            for (int b = 1; b < total_b; ++b) {
+                const __half* src = rows_of(b);
+                uint64_t* full_hi = barHiFull + (b & 1); uint64_t* full_lo = barLoFull + (b & 1);
+                mbar_wait(barHiEmpty, (uint32_t)((b - 1) & 1));
+                mbar_expect_tx(full_hi, kPartBytes); bulk_g2s(sInHi, src, kPartBytes, full_hi);
+                // the next burst's rows: pull them into L2 now, so that their copy (one burst from now) pays L2 latency instead of DRAM latency
+                if (b + 1 < total_b) bulk_prefetch_l2(rows_of(b + 1), 2 * kPartBytes);
+                mbar_wait(barLoEmpty, (uint32_t)((b - 1) & 1));
+                mbar_expect_tx(full_lo, kPartBytes); bulk_g2s(sInLo, src + kPartBytes / 2, kPartBytes, full_lo);
+            }
+        }
+        __syncwarp();
+    } else {
+        float c[UB][8];
+#pragma unroll
+        for (int j = 0; j < UB; ++j)
+#pragma unroll
+            for (int u = 0; u < 8; ++u) c[j][u] = 0.f;
+
+        if (total_g > 0) {
+            if (warp == 0) wait_input();
+            report_ready();
+        }
+
+        const uint32_t tmem_base = *tmem_slot + (uint32_t)grp * 256u;
+        const uint32_t in_hi = smem_u32(sInHi), in_lo = smem_u32(sInLo), h_hi = smem_u32(sHhi), h_lo = smem_u32(sHlo);
+        const uint32_t b_hi = smem_u32(sBhi), b_lo = smem_u32(sBlo);
+        constexpr uint32_t idesc = make_idesc(256, 256);
+        const bool issuer = cta_rank == 0 && tid == 0;
+        uint32_t phaseH = 0, phaseR = 0, phaseT = 0;
+        if (cta_rank == 0 && threadIdx.x == 0) mbar_arrive(barTurn + 0);          // group 0 issues first
+
+        int step = 0, qi = 0;
+        for (int g = 0; g < total_g; ++g) {
+            const bool more = g + 1 < total_g;
+            const int64_t site = tile_of(qi, grp) * kRows + row;
+            const bool live = site < n;
+            float* const out = h16 + site * 128 + dir * kH + sub * UB * 8;      // this thread's hidden units of the t = 16 state
+            if (step == 0) {                                        // a new tile: the recurrence starts from c = 0, h = 0
+#pragma unroll
+                for (int j = 0; j < UB; ++j)
+#pragma unroll
+                    for (int u = 0; u < 8; ++u) c[j][u] = 0.f;
+            }
+            if (issuer) {
+                const bool refill = more || grp == 0;              // another burst follows this one
+                mbar_wait_cluster(barReady, phaseR);               // every warp of this group, in both CTAs, has reported
+                mbar_wait(barTurn + grp, phaseT);                  // and it is this group's turn on the tensor pipe
+                tc_fence_after();
+                // pass 0: a_hi.w_hi   pass 1: a_hi.w_lo   pass 2: a_lo.w_hi; input part first, then the h part
+#pragma unroll 1
+                for (int pass = 0; pass < 3; ++pass) {
+#pragma unroll 1
+                    for (int kb = 0; kb < XB; ++kb)
+                        umma_f16<2>(tmem_base, make_desc((pass == 2 ? in_lo : in_hi) + kb * 2 * LBO_A, LBO_A, SBO),
+                                    make_desc((pass == 1 ? b_lo : b_hi) + kb * 2 * LBO_B, LBO_B, SBO), idesc, (pass | kb) ? 1u : 0u);
+                    if (pass == 1 && refill) umma_commit<2>(barHiEmpty);     // the hi input rows are read: the producer may refill them
+                }
+                if (refill) umma_commit<2>(barLoEmpty);
+                if (step > 0) {                                    // h = 0 at the first step of a tile: input k-blocks only
+#pragma unroll 1
+                    for (int pass = 0; pass < 3; ++pass) {
+#pragma unroll 1
+                        for (int kb = XB; kb < KB; ++kb)
+                            umma_f16<2>(tmem_base, make_desc((pass == 2 ? h_lo : h_hi) + (kb - XB) * 2 * LBO_A, LBO_A, SBO),
+                                        make_desc((pass == 1 ? b_lo : b_hi) + kb * 2 * LBO_B, LBO_B, SBO), idesc, 1u);
+                    }
+                }
+                umma_commit<2>(barH);
+                mbar_arrive(barTurn + (grp ^ 1));                  // hand the token to the other group
+            }
+            phaseR ^= 1; phaseT ^= 1;
+            mbar_wait(barH, phaseH);
+            phaseH ^= 1;
+            tc_fence_after();
+
+            uint32_t vb[2][16];
+            const uint32_t tacc = tmem_base + ((uint32_t)(quad * 32) << 16) + (uint32_t)(sub * UB) * 32u;
+            tmem_ld16_nowait(tacc, vb[0]);
+            tmem_wait_ld();
+            float hv[8];
+#pragma unroll
+            for (int hb = 0; hb < 2 * UB; ++hb) {
+                const int jl = hb >> 1, uh = hb & 1, jb = sub * UB + jl;
+                if (hb + 1 < 2 * UB) tmem_ld16_nowait(tacc + (hb + 1) * 16, vb[(hb + 1) & 1]);
+#pragma unroll
+                for (int u = 0; u < 4; ++u) {
+                    const uint32_t* v = vb[hb & 1];
+                    // same cell update as lstm_tc_kernel<1> (scales folded into the weights, scaled cell state, bias in the epilogue)
+                    const float* bq = sBias + jb * 32 + uh * 16 + u;
+                    const float xi_ = fminf(__uint_as_float(v[u]) + bq[0], 36.f), xf_ = fminf(__uint_as_float(v[4 + u]) + bq[4], 36.f);
+                    const float xg_ = fminf(__uint_as_float(v[8 + u]) + bq[8], 36.f), xo_ = __uint_as_float(v[12 + u]) + bq[12];
+                    const float ei = ex2_approx(xi_), ef = ex2_approx(xf_), eg = ex2_approx(xg_), eo = ex2_approx(xo_);
+                    const float pi = 1.f + ei, pf = 1.f + ef, pg = 1.f + eg;
+                    const float pig = pi * pg;
+                    const float num = fmaf(c[jl][uh * 4 + u], pig, fmaf(eg, 2.f * kLog2e, -2.f * kLog2e) * pf);
+                    const float cn = num * rcp_approx(pf * pig);
+                    c[jl][uh * 4 + u] = cn;
+                    const float ec = ex2_approx(cn);
+                    hv[uh * 4 + u] = (1.f - ec) * rcp_approx((1.f + eo) * (1.f + ec));
+                }
+                if (hb + 1 < 2 * UB) tmem_wait_ld();
+                if (uh == 1) {
+                    const HiLo8 sp = split8(hv);
+                    reinterpret_cast<uint4*>(sHhi + jb * LBO_A)[row] = sp.hi;
+                    reinterpret_cast<uint4*>(sHlo + jb * LBO_A)[row] = sp.lo;
+                    if (live && step == kS - 1) {
+                        float4* o = reinterpret_cast<float4*>(out + jl * 8);
+                        o[0] = make_float4(hv[0], hv[1], hv[2], hv[3]); o[1] = make_float4(hv[4], hv[5], hv[6], hv[7]);
+                    }
+                }
+            }
+            if (more) {
+                if (warp == 0) wait_input();
+                report_ready();
+            }
+            if (++step == kS) { step = 0; ++qi; }
+        }
+    }
+
+    tc_fence_before();
+    cluster_sync_all();
+    if (threadIdx.x < 32) tmem_dealloc<2>(*tmem_slot, 512);
+}
+
 template <class Kern, class... Args>
-int launch_pair2(Kern kern, const char* name, size_t smem_bytes, int64_t m, cudaStream_t stream, Args... args) {
+int launch_pair2(Kern kern, const char* name, size_t smem_bytes, int threads, int64_t m, cudaStream_t stream, Args... args) {
     // persistent: at most one CTA per SM; clusters alternate between the two directions, so an even number of clusters
     const unsigned quads = (unsigned)((m + 4 * kRows - 1) / (4 * kRows));
     unsigned clusters = 2 * quads; if (clusters > (unsigned)kNumSMs / 2) clusters = ((unsigned)kNumSMs / 2) & ~1u;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(2 * clusters, 1, 1);
-    cfg.blockDim = dim3(kP2Threads, 1, 1);
+    cfg.blockDim = dim3((unsigned)threads, 1, 1);
     cfg.dynamicSmemBytes = smem_bytes;
     cfg.stream = stream;
     cudaLaunchAttribute attr[1];
@@ -772,7 +1014,7 @@ int launch_l0_pair2(const void* blob, const int32_t* xi, const float* xf, void* 
             return cuda_status("cudaFuncSetAttribute(lstm0_pair2_kernel)");
         attr_done = true;
     }
-    return launch_pair2(lstm0_pair2_kernel, "lstm0_pair2_kernel", P2Smem::total, m, stream, (const unsigned char*)blob, xi, xf, (__half*)h0_out, m, pos, pos_bias, npass);
+    return launch_pair2(lstm0_pair2_kernel, "lstm0_pair2_kernel", P2Smem::total, kP2Threads, m, stream, (const unsigned char*)blob, xi, xf, (__half*)h0_out, m, pos, pos_bias, npass);
 }
 
 int launch_l1_pair2(const void* blob, const void* h0_in, float* h16, int64_t m, cudaStream_t stream) {
@@ -782,7 +1024,17 @@ int launch_l1_pair2(const void* blob, const void* h0_in, float* h16, int64_t m, 
             return cuda_status("cudaFuncSetAttribute(lstm1_pair2_kernel)");
         attr_done = true;
     }
-    return launch_pair2(lstm1_pair2_kernel, "lstm1_pair2_kernel", P2Smem1::total, m, stream, (const unsigned char*)blob, (const __half*)h0_in, h16, m);
+    return launch_pair2(lstm1_pair2_kernel, "lstm1_pair2_kernel", P2Smem1::total, kP2Threads, m, stream, (const unsigned char*)blob, (const __half*)h0_in, h16, m);
+}
+
+int launch_l1_pair2x3(const void* blob, const void* h0_in, float* h16, int64_t m, cudaStream_t stream) {
+    static bool attr_done = false;
+    if (!attr_done) {
+        if (cudaFuncSetAttribute(lstm1_pair2x3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P2Smem1x3::total) != cudaSuccess)
+            return cuda_status("cudaFuncSetAttribute(lstm1_pair2x3_kernel)");
+        attr_done = true;
+    }
+    return launch_pair2(lstm1_pair2x3_kernel, "lstm1_pair2x3_kernel", P2Smem1x3::total, kP2x3Threads, m, stream, (const unsigned char*)blob, (const __half*)h0_in, h16, m);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -1039,12 +1291,14 @@ int launch_lstm_tc(const void* blob, const int32_t* xi, const float* xf, void* h
         if (int e = variant == 1 ? launch_l0_pair2(blob, xi, xf, h0, m, pos, pos_bias, npass, stream)
                                  : launch_one<0, 2, 2, false>(blob, xi, xf, nullptr, h0, nullptr, nullptr, m, npass << 16, stream)) return e;
     }
-    // layer 1: W only fits split across a CTA pair (2 x 104 KB); one CTA per SM, 16 warps for the epilogue
+    // layer 1: W only fits split across a CTA pair (2 x 96 KB hi + lo); one CTA per SM
     ProfScope prof(NSNP_PROF_LSTM1, stream);
     static const int pf = [] { const char* v = getenv("NSNP_L1_PREFETCH"); return v ? atoi(v) : 1; }();
-    // single pass: two alternating groups per CTA (lstm1_pair2_kernel); NSNP_L1_VARIANT=0 keeps the one-group kernel (A/B, tests)
+    // default: two alternating groups per CTA (lstm1_pair2x3_kernel, single pass: lstm1_pair2_kernel);
+    // NSNP_L1_VARIANT=0 keeps the one-group kernel lstm_tc_kernel<1,2,4> (A/B, tests)
     static const int l1_variant = [] { const char* v = getenv("NSNP_L1_VARIANT"); return v ? atoi(v) : 1; }();
     if (npass == 1 && l1_variant == 1) return launch_l1_pair2(blob, h0, h16, m, stream);
+    if (npass == 3 && l1_variant == 1) return launch_l1_pair2x3(blob, h0, h16, m, stream);
     return launch_one<1, 2, 4, false>(blob, nullptr, nullptr, h0, nullptr, h16, nullptr, m, (pf << 8) | (npass << 16), stream);
 }
 
