@@ -148,6 +148,21 @@ int nsnp_select_candidates_targets(const int32_t* counts_dev, uint8_t* flags_dev
                                    int32_t* n_dev, void* workspace_dev, size_t workspace_bytes, int32_t* status_dev,
                                    void* stream);
 
+/* ---- s1, step B for a list of given sites ------------------------------------------------------------
+ * An extension of this library with no reference counterpart (NanoSNP calls only gate-passing positions).
+ * sites: n_sites intervals of listed positions, with the same format and checks as the targets above (runs of
+ * consecutive sites are one interval).  A position is a candidate iff it lies in an interval, its centre
+ * reference base is one of ACGTacgt, and every position of [c - 16, c + 16] is covered -- the GATE bit (AF
+ * thresholds, min_coverage) is ignored, so hom-ref and low-depth sites are selected too.  Flags come from
+ * nsnp_pileup_counts_targets with the same intervals.  n_sites == 0 selects no site.
+ */
+size_t nsnp_select_sites_workspace_bytes(int64_t region_len, int64_t n_sites);
+int nsnp_select_candidates_sites(const uint8_t* flags_dev, const uint8_t* ref_dev, int64_t contig_len,
+                                 int64_t region_start, int64_t region_len, int64_t emit_start, int64_t emit_end,
+                                 const int32_t* sites, int64_t n_sites, int32_t* pos_dev, int64_t capacity,
+                                 int32_t* n_dev, void* workspace_dev, size_t workspace_bytes, int32_t* status_dev,
+                                 void* stream);
+
 /* ---- s1, step C: window gather ------------------------------------------------------------------
  * Replaces the ring-buffer window emit (main.cpp:220-251), DNA_CreatePredictData
  * (make_predict_data/main.cpp:76-127) and make_bin_predict_data.py:35-55: writes position_matrix

@@ -92,6 +92,8 @@ SYMBOLS = {
     "nsnp_select_targets_workspace_bytes": (_SZ, [_I64, _I64]),
     "nsnp_select_candidates_targets": (C.c_int, [_P, _P, _P, _I64, _I64, _I64, _I64, _I64, _P, _I64, C.POINTER(Params), C.c_int, _P, _I64, _P,
                                                  _P, _SZ, _P, _P]),
+    "nsnp_select_sites_workspace_bytes": (_SZ, [_I64, _I64]),
+    "nsnp_select_candidates_sites": (C.c_int, [_P, _P, _I64, _I64, _I64, _I64, _I64, _P, _I64, _P, _I64, _P, _P, _SZ, _P, _P]),
     "nsnp_gather_windows": (C.c_int, [_P, _P, _I64, _I64, _P, _P, _I64, _P, _P, _P, _P]),
     "nsnp_model_blob_bytes": (_SZ, []),
     "nsnp_model_pack_weights": (C.c_int, [C.POINTER(ModelWeights), _P, _SZ]),

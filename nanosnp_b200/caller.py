@@ -56,10 +56,11 @@ def call_contig(runner: RegionRunner, reads: PackedReads, ref: np.ndarray, conti
 
 
 def call_contig_text(runner: RegionRunner, reads: PackedReads, ref: np.ndarray, contig: str, sink, batch_size: int = 1000,
-                     region_len: int = 12_500_000, regions=None, region_reads=None, targets=None) -> dict:
+                     region_len: int = 12_500_000, regions=None, region_reads=None, targets=None, sites: bool = False) -> dict:
     """call_contig with the VCF text assembled on the GPU (csrc/vcf_dev.cu): the host only writes the bytes.
     region_reads: optional ready-made per-region PackedReads (e.g. BamReader.fetch); else `reads` is sliced.
-    targets: optional per-region intervals, aligned with `regions` (shard.plan_target_units)."""
+    targets: optional per-region intervals, aligned with `regions` (shard.plan_target_units).  sites: the targets are
+    given sites, called whether they pass the gate or not (RegionRunner.run_device)."""
     from .vcf_text import GpuVcfText
     L = int(len(ref))
     ref_dev = torch.from_numpy(np.ascontiguousarray(ref)).to(runner.device)
@@ -75,7 +76,7 @@ def call_contig_text(runner: RegionRunner, reads: PackedReads, ref: np.ndarray, 
         nbytes[0] += len(mv)
         if sink is not None:
             sink.write(mv)
-    n = runner.run_host_text(host_regions, regions, ref_dev, gen, write, targets)
+    n = runner.run_host_text(host_regions, regions, ref_dev, gen, write, targets, sites)
     return {"sites": n, "vcf_bytes": nbytes[0], "regions": len(regions)}
 
 

@@ -21,6 +21,7 @@ struct SelArgs {
     int64_t emit_start, emit_end;      // contig coordinates
     const int32_t* targets;            // nullptr, or n_targets sorted disjoint [start, end) pairs (contig coordinates)
     int n_targets;
+    const uint8_t* ref;                // sites mode: the contig, for the centre-base rule
 };
 
 // target bits of the 8 positions [c0, c0 + 8): binary search for the first interval ending after c0, then at most 8 more
@@ -39,6 +40,7 @@ __device__ __forceinline__ uint32_t target_mask8(const SelArgs& a, int64_t c0) {
 }
 
 // 8-bit candidate mask of positions [seg0 + 8*tid, +8): bit j set <=> site
+template <bool kSites>
 __device__ __forceinline__ uint32_t cand_mask8(const SelArgs& a, int64_t seg0, uint32_t* covw /* smem, (kSeg+64)/32 + 2 words */) {
     const int tid = threadIdx.x;
     uint8_t* cov8 = reinterpret_cast<uint8_t*>(covw);
@@ -65,7 +67,17 @@ __device__ __forceinline__ uint32_t cand_mask8(const SelArgs& a, int64_t seg0, u
     };
     uint32_t gate = 0, gdummy;
     const int64_t i0 = seg0 + (int64_t)tid * 8;
-    cov8[tid + 2] = (uint8_t)pack8(i0, gate);
+    const uint32_t own = pack8(i0, gate);
+    cov8[tid + 2] = (uint8_t)own;
+    if constexpr (kSites) {
+        // the pileup epilogue folds the ACGT centre-base rule (make_predict_data/main.cpp:92, SURVEY 8a P10) into the GATE
+        // bit; the listed covered positions replace that bit here, so the rule is applied again
+        gate = own ? own & target_mask8(a, a.region_start + i0) : 0u;
+        for (uint32_t g = gate; g; g &= g - 1) {
+            const int j = __ffs(g) - 1;
+            if (nt4(__ldg(a.ref + a.region_start + i0 + j)) >= 4) gate &= ~(1u << j);
+        }
+    }
     if (tid < 2) cov8[tid] = (uint8_t)pack8(seg0 - 16 + 8 * tid, gdummy);
     else if (tid < 4) cov8[kSelThreads + tid] = (uint8_t)pack8(seg0 + kSeg + 8 * (tid - 2), gdummy);
     else if (tid < 12) cov8[kSelThreads + tid] = 0;              // padding read by the unaligned extraction
@@ -80,15 +92,16 @@ __device__ __forceinline__ uint32_t cand_mask8(const SelArgs& a, int64_t seg0, u
         const uint32_t hi = (covw[(b >> 5) + 1] >> (b & 31)) & 1u;
         if (lo == 0xFFFFFFFFu && hi) m |= 1u << j;
     }
-    if (a.targets && m) m &= target_mask8(a, a.region_start + i0);
+    if (!kSites && a.targets && m) m &= target_mask8(a, a.region_start + i0);
     return m;
 }
 
+template <bool kSites>
 __global__ void __launch_bounds__(kSelThreads) select_count_kernel(SelArgs a, int32_t* seg_counts) {
     __shared__ uint32_t covw[(kSeg + 64) / 32 + 4];
     __shared__ int wsum[kSelThreads / 32];
     const int64_t seg0 = (int64_t)blockIdx.x * kSeg;
-    const int cnt = __popc(cand_mask8(a, seg0, covw));
+    const int cnt = __popc(cand_mask8<kSites>(a, seg0, covw));
     const int ws = __reduce_add_sync(0xffffffffu, cnt);
     if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5] = ws;
     __syncthreads();
@@ -131,12 +144,13 @@ __global__ void __launch_bounds__(1024) select_scan_kernel(int32_t* seg_counts, 
     }
 }
 
+template <bool kSites>
 __global__ void __launch_bounds__(kSelThreads) select_write_kernel(SelArgs a, const int32_t* seg_offsets, int32_t* pos_out, int64_t capacity) {
     __shared__ uint32_t covw[(kSeg + 64) / 32 + 4];
     __shared__ int wsum[kSelThreads / 32];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int64_t seg0 = (int64_t)blockIdx.x * kSeg;
-    uint32_t m = cand_mask8(a, seg0, covw);
+    uint32_t m = cand_mask8<kSites>(a, seg0, covw);
     const int cnt = __popc(m);
     int inc = cnt;
 #pragma unroll
@@ -240,20 +254,22 @@ size_t nsnp_select_workspace_bytes(int64_t region_len) {
 }  // extern "C"
 
 // targets == nullptr && n_targets < 0: every position of the emit range (nsnp_select_candidates)
+// sites: listed positions replace the gate (nsnp_select_candidates_sites; params and recompute_gate are unused)
 static int select_candidates(const int32_t* counts_dev, uint8_t* flags_dev, const uint8_t* ref_dev, int64_t contig_len,
                              int64_t region_start, int64_t region_len, int64_t emit_start, int64_t emit_end,
                              const int32_t* targets, int64_t n_targets, const nsnp_params_t* params, int recompute_gate,
                              int32_t* pos_dev, int64_t capacity, int32_t* n_dev, void* workspace_dev, size_t workspace_bytes,
-                             int32_t* status_dev, void* stream_)
+                             int32_t* status_dev, void* stream_, bool sites = false)
 {
     cudaStream_t stream = (cudaStream_t)stream_;
-    if (!flags_dev || !pos_dev || !n_dev || !workspace_dev || !status_dev || !params)
+    if (!flags_dev || !pos_dev || !n_dev || !workspace_dev || !status_dev || (!params && !sites) || (sites && !ref_dev))
         return set_error(NSNP_E_INVALID, "nsnp_select_candidates: null argument");
     if (recompute_gate && (!counts_dev || !ref_dev)) return set_error(NSNP_E_INVALID, "nsnp_select_candidates: recompute_gate needs counts and ref");
     if (region_start < 0 || region_len < 0 || region_start + region_len > contig_len || capacity < 0)
         return set_error(NSNP_E_INVALID, "nsnp_select_candidates: bad region");
     if (n_targets >= 0) {
-        if (int e = check_targets("nsnp_select_candidates_targets", targets, n_targets, region_start, region_start + region_len)) return e;
+        if (int e = check_targets(sites ? "nsnp_select_candidates_sites" : "nsnp_select_candidates_targets", targets, n_targets,
+                                  region_start, region_start + region_len)) return e;
     }
     const size_t ws_need = n_targets >= 0 ? nsnp_select_targets_workspace_bytes(region_len, n_targets) : nsnp_select_workspace_bytes(region_len);
     if (workspace_bytes < ws_need) return set_error(NSNP_E_WORKSPACE, "select workspace too small");
@@ -265,7 +281,7 @@ static int select_candidates(const int32_t* counts_dev, uint8_t* flags_dev, cons
         if (int e = cuda_status("regate_kernel")) return e;
     }
     ProfScope prof(NSNP_PROF_SELECT, stream);
-    SelArgs a{flags_dev, region_start, region_len, emit_start, emit_end, nullptr, 0};
+    SelArgs a{flags_dev, region_start, region_len, emit_start, emit_end, nullptr, 0, ref_dev};
     const int n_seg = (int)((region_len + kSeg - 1) / kSeg);
     int32_t* seg = (int32_t*)workspace_dev;
     if (n_targets > 0) {                        // the interval copy sits behind the segment counts
@@ -273,9 +289,11 @@ static int select_candidates(const int32_t* counts_dev, uint8_t* flags_dev, cons
         cudaMemcpyAsync(iv, targets, (size_t)n_targets * 8, cudaMemcpyHostToDevice, stream);
         a.targets = iv; a.n_targets = (int)n_targets;
     }
-    select_count_kernel<<<n_seg, kSelThreads, 0, stream>>>(a, seg);
+    if (sites) select_count_kernel<true><<<n_seg, kSelThreads, 0, stream>>>(a, seg);
+    else select_count_kernel<false><<<n_seg, kSelThreads, 0, stream>>>(a, seg);
     select_scan_kernel<<<1, 1024, 0, stream>>>(seg, n_seg, n_dev, capacity, status_dev);
-    select_write_kernel<<<n_seg, kSelThreads, 0, stream>>>(a, seg, pos_dev, capacity);
+    if (sites) select_write_kernel<true><<<n_seg, kSelThreads, 0, stream>>>(a, seg, pos_dev, capacity);
+    else select_write_kernel<false><<<n_seg, kSelThreads, 0, stream>>>(a, seg, pos_dev, capacity);
     return cuda_status("select kernels");
 }
 
@@ -303,6 +321,21 @@ int nsnp_select_candidates_targets(const int32_t* counts_dev, uint8_t* flags_dev
     if (n_targets < 0) return set_error(NSNP_E_INVALID, "nsnp_select_candidates_targets: negative interval count");
     return select_candidates(counts_dev, flags_dev, ref_dev, contig_len, region_start, region_len, emit_start, emit_end, targets,
                              n_targets, params, recompute_gate, pos_dev, capacity, n_dev, workspace_dev, workspace_bytes, status_dev, stream);
+}
+
+size_t nsnp_select_sites_workspace_bytes(int64_t region_len, int64_t n_sites) {
+    return nsnp_select_targets_workspace_bytes(region_len, n_sites);
+}
+
+int nsnp_select_candidates_sites(const uint8_t* flags_dev, const uint8_t* ref_dev, int64_t contig_len, int64_t region_start,
+                                 int64_t region_len, int64_t emit_start, int64_t emit_end, const int32_t* sites, int64_t n_sites,
+                                 int32_t* pos_dev, int64_t capacity, int32_t* n_dev, void* workspace_dev, size_t workspace_bytes,
+                                 int32_t* status_dev, void* stream)
+{
+    if (n_sites < 0) return set_error(NSNP_E_INVALID, "nsnp_select_candidates_sites: negative interval count");
+    return select_candidates(nullptr, const_cast<uint8_t*>(flags_dev), ref_dev, contig_len, region_start, region_len, emit_start,
+                             emit_end, sites, n_sites, nullptr, 0, pos_dev, capacity, n_dev, workspace_dev, workspace_bytes,
+                             status_dev, stream, true);
 }
 
 int nsnp_gather_windows(const int32_t* counts_dev, const uint8_t* ref_dev, int64_t region_start, int64_t region_len,

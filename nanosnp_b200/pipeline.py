@@ -104,13 +104,27 @@ class PileupEngine:
     # -- s1 step B ---------------------------------------------------------------------------------
     def select(self, flags: torch.Tensor, ref: torch.Tensor, region_start: int, emit_start: int, emit_end: int,
                capacity: int, counts: Optional[torch.Tensor] = None, recompute_gate: bool = False,
-               pos: Optional[torch.Tensor] = None, n_dev: Optional[torch.Tensor] = None, targets: Optional[np.ndarray] = None):
-        """targets: optional [k, 2] sorted disjoint [start, end) contig intervals: only sites inside them are selected."""
+               pos: Optional[torch.Tensor] = None, n_dev: Optional[torch.Tensor] = None, targets: Optional[np.ndarray] = None,
+               sites: bool = False):
+        """targets: optional [k, 2] sorted disjoint [start, end) contig intervals: only sites inside them are selected.
+        sites: every covered position of the targets with an ACGT centre base and a full 33-row window is selected, whether it
+        passes the allele-frequency / depth gate or not (`--sites`); needs targets."""
         region_len = int(flags.shape[0])
         if pos is None:
             pos = torch.empty(max(capacity, 1), dtype=torch.int32, device=self.device)
         if n_dev is None:
             n_dev = torch.zeros(1, dtype=torch.int32, device=self.device)
+        if sites:
+            if targets is None:
+                raise ValueError("select(sites=True) needs the site intervals as targets")
+            iv = _intervals(targets)
+            ws = self._workspace("select", self.lib.nsnp_select_sites_workspace_bytes(region_len, len(iv)))
+            with torch.cuda.device(self.device):
+                _lib.check(self.lib.nsnp_select_candidates_sites(
+                    flags.data_ptr(), ref.data_ptr(), int(ref.shape[0]), region_start, region_len, emit_start, emit_end, iv.ctypes.data,
+                    len(iv), pos.data_ptr(), capacity, n_dev.data_ptr(), ws.data_ptr(), ws.numel(), self.status.data_ptr(),
+                    _stream(self.device)))
+            return pos, n_dev
         if targets is not None:
             iv = _intervals(targets)
             ws = self._workspace("select", self.lib.nsnp_select_targets_workspace_bytes(region_len, len(iv)))

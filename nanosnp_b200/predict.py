@@ -76,14 +76,16 @@ def _region_reads(reads, reader, rid, regions, targets=None):
 
 
 def predict(model: LSTMNetwork, testing_paths, reference_index_file, batch_size, output_file, device, reference=None, region_len=12_500_000,
-            targets=None):
+            targets=None, sites=False):
     """predict.py:37-195.  `.pd` text files: windows -> model -> records.  Read inputs (`.bam`, `.reads.npz`): the whole
     s1 + s2 path incl. the VCF text runs on the GPU region by region (caller.call_contig_text); under torchrun every rank
     computes and formats its LPT share of the regions and writes its own segments of the one output file
     (caller.write_sharded_vcf).
     targets: None (every position), or contig -> merged [k, 2] 0-based [start, end) intervals (targets.build_targets): only
     sites inside them are called, and the GPU computes only the pileup tiles near them.  The VCF is the one the reference
-    writes from `.pd` files holding only those sites (batches are consecutive kept sites)."""
+    writes from `.pd` files holding only those sites (batches are consecutive kept sites).
+    sites: the targets are a list of given sites (targets.load_sites_vcf): every listed position with a full 33-row window
+    and an ACGT centre base is called, whether it passes the allele-frequency / depth gate or not.  Read inputs only."""
     import io
     from .caller import call_contig_text, write_sharded_vcf, _pinned
     from .dataset import load_fasta
@@ -93,6 +95,9 @@ def predict(model: LSTMNetwork, testing_paths, reference_index_file, batch_size,
     from .targets import in_targets
     runner = None
     fasta = None
+    if sites and any(f.endswith(".pd") for f in testing_paths):
+        raise ValueError("--sites needs read inputs (.bam / .reads.npz): a .pd file holds only the windows of gate-passing "
+                         "positions, so the hom-ref sites of the list would be missing")
 
     def get_runner():
         nonlocal runner
@@ -138,7 +143,7 @@ def predict(model: LSTMNetwork, testing_paths, reference_index_file, batch_size,
             ref_dev = torch.from_numpy(np.ascontiguousarray(fasta[contig])).to(device)
             r = get_runner()
             for k, (i, rg, hr) in enumerate(zip(idx, rgs, host)):
-                out = r.run_device(r.upload(hr), ref_dev, rg, targets=None if ivs is None else ivs[k])
+                out = r.run_device(r.upload(hr), ref_dev, rg, targets=None if ivs is None else ivs[k], sites=sites)
                 recs[i] = out.rec.clone()                    # records stay on this GPU until the text is made
         for i in mine:
             recs.setdefault(i, torch.zeros((0, 32), dtype=torch.uint8, device=device))
@@ -183,7 +188,7 @@ def predict(model: LSTMNetwork, testing_paths, reference_index_file, batch_size,
                 else:
                     regions, unit_iv = plan_target_units([(contig, len(fasta[contig]))], targets, region_len)
                 call_contig_text(get_runner(), reads, fasta[contig], contig, fwriter, batch_size, region_len, regions,
-                                 _region_reads(reads, reader, rid, regions, unit_iv), unit_iv)
+                                 _region_reads(reads, reader, rid, regions, unit_iv), unit_iv, sites)
         model._forward().reevaluated()                          # f16x1: raises if a region had more low-margin sites than are re-run
 
 
@@ -202,6 +207,9 @@ def main(argv=None):
     parser.add_argument("--bed", default=None, help="call only inside these intervals (BED: 0-based, half-open; first three fields)")
     parser.add_argument("--region", action="append", default=[],
                         help="call only inside CTG or CTG:START-END (1-based, inclusive); repeatable, combines with --bed")
+    parser.add_argument("--sites", default=None,
+                        help="genotype the sites of this VCF (CHROM, POS; plain or gzip): every listed position with a full window "
+                             "is called, whatever its allele frequency; with --bed / --region only the sites inside them")
     opt = parser.parse_args(argv)
     if opt.no_cuda:
         raise SystemExit("nanosnp_b200.predict: --no_cuda is not supported (no CPU fallback); use the reference's predict.py on CPU")
@@ -236,14 +244,19 @@ def main(argv=None):
         testing_paths = sorted(opt.data + "/" + f for f in os.listdir(opt.data) if f.endswith((".pd", ".reads.npz", ".bam")))
     assert os.path.exists(opt.reference + ".fai"), "reference index file does not exist."
     targets = None
-    if opt.bed is not None or opt.region:
-        from .targets import build_targets
+    if opt.bed is not None or opt.region or opt.sites is not None:
+        from .targets import build_targets, intersect_targets, load_sites_vcf
         with open(opt.reference + ".fai") as f:
             contigs = [(l.split()[0], int(l.split()[1])) for l in f if l.strip()]
         quiet = int(os.environ.get("RANK", "0")) != 0                   # report skipped intervals once, not once per rank
-        targets = build_targets(contigs, opt.bed, opt.region, report=None if quiet else sys.stderr)
+        report = None if quiet else sys.stderr
+        if opt.bed is not None or opt.region:
+            targets = build_targets(contigs, opt.bed, opt.region, report=report)
+        if opt.sites is not None:
+            listed = load_sites_vcf(opt.sites, contigs, report=report)
+            targets = listed if targets is None else intersect_targets(listed, targets)
     predict(pred_model, testing_paths, opt.reference + ".fai", opt.batch_size, opt.output, device, reference=opt.reference,
-            region_len=opt.region_len, targets=targets)
+            region_len=opt.region_len, targets=targets, sites=opt.sites is not None)
     if int(os.environ.get("WORLD_SIZE", "1")) > 1:
         import torch.distributed as dist
         dist.barrier()

@@ -88,10 +88,11 @@ class RegionRunner:
         return t[:n].view(*shape)
 
     def run_device(self, reads: PackedReads, ref: torch.Tensor, region: Region, timer: Optional[StageTimer] = None,
-                   targets: Optional[np.ndarray] = None) -> RegionOutput:
+                   targets: Optional[np.ndarray] = None, sites: bool = False) -> RegionOutput:
         """targets: the unit's [k, 2] sorted disjoint [start, end) intervals (contig coordinates, inside the emit span), or None
         for every position of the region.  With targets only the tiles near them are computed and only sites inside them
-        are kept; the launch count does not depend on k."""
+        are kept; the launch count does not depend on k.  sites: the targets are a list of given sites (`--sites`): each
+        listed position with a full window and an ACGT centre base is called, whether it passes the gate or not."""
         eng = self.eng
         rlen = region.length
         timer = timer or StageTimer(False)
@@ -101,11 +102,14 @@ class RegionRunner:
         eng.pileup_counts(reads, ref, region.start, rlen, counts=counts, flags=flags, targets=targets)
         timer.stop()
         self.launches += (2 if reads.n_reads else 1) + (targets is not None)
-        cap = max(1024, region.emit_end - region.emit_start)
+        if sites:                                 # at most one candidate per listed position
+            cap = max(1024, int(np.subtract(targets[:, 1], targets[:, 0], dtype=np.int64).sum()))
+        else:
+            cap = max(1024, region.emit_end - region.emit_start)
         pos = self._buf("pos", (cap,), torch.int32)
         n_dev = self._buf("n", (1,), torch.int32)
         timer.start("select")
-        eng.select(flags, ref, region.start, region.emit_start, region.emit_end, cap, pos=pos, n_dev=n_dev, targets=targets)
+        eng.select(flags, ref, region.start, region.emit_start, region.emit_end, cap, pos=pos, n_dev=n_dev, targets=targets, sites=sites)
         timer.stop()
         self.launches += 3
         if self.blocking_sync:
@@ -229,11 +233,12 @@ class RegionRunner:
         return total
 
     # ---- host-buffer mode with the VCF text assembled on the GPU ---------------------------------------------------------
-    def run_host_text(self, host_regions, regions, ref: torch.Tensor, textgen, write, targets=None) -> int:
+    def run_host_text(self, host_regions, regions, ref: torch.Tensor, textgen, write, targets=None, sites: bool = False) -> int:
         """Pinned host read arrays of consecutive regions of ONE contig -> H2D -> kernels -> compact records -> VCF text on
         the GPU (vcf_text.GpuVcfText, which carries partial 1000-site batches across regions) -> D2H of the text.
         write(memoryview) receives the text chunks in order.  H2D of region k+1 and D2H of chunk k-1 overlap the kernels of
-        region k; the host does no per-record work.  targets: optional per-region intervals (run_device).  Returns the site count."""
+        region k; the host does no per-record work.  targets, sites: optional per-region intervals and their mode (run_device).
+        Returns the site count."""
         assert self.records, "run_host_text needs a RegionRunner(records=True)"
         dev = self.device
         main = torch.cuda.current_stream(dev)
@@ -261,7 +266,7 @@ class RegionRunner:
             if k + 1 < n_reg:
                 start_upload(k + 1)
             main.wait_event(up_done[k])
-            out = self.run_device(dev_reads[k], ref, regions[k], targets=None if targets is None else targets[k])
+            out = self.run_device(dev_reads[k], ref, regions[k], targets=None if targets is None else targets[k], sites=sites)
             chunk = textgen.push(out.rec) if out.n else None        # copies the records: the work buffers are free again
             self.launches += 3 if chunk is not None else 0
             ev = torch.cuda.Event(); ev.record(main); comp_done[k] = ev
