@@ -199,15 +199,19 @@ def from_records(records, with_nmask: bool = True) -> PackedReads:
         soff.append(nb)
         bases.append(seq)
         nb += (len(seq) + 15) // 16 * 16
-    seq2 = np.zeros((nb + 3) // 4 + 8, np.uint8)
-    nmask = np.zeros((nb + 7) // 8 + 8, np.uint8)
+    # one code per base slot (reads start on 16-base boundaries; padding slots stay 0), 4 = not ACGT -> an nmask bit
+    lut = np.full(256, 4, np.uint8)
+    for ch, c in code.items():
+        lut[ord(ch)] = lut[ord(ch.lower())] = c
+    codes = np.zeros(nb + 16, np.uint8)
     for so, seq in zip(soff, bases):
-        for j, ch in enumerate(seq.upper()):
-            k = so + j
-            if ch in code:
-                seq2[k >> 2] |= code[ch] << (2 * (k & 3))
-            else:
-                nmask[k >> 3] |= 1 << (k & 7)
+        codes[so:so + len(seq)] = lut[np.frombuffer(seq.encode("latin-1"), np.uint8)]
+    isn = codes == 4
+    c2 = np.where(isn, 0, codes).astype(np.uint8)[: (nb + 3) // 4 * 4].reshape(-1, 4)
+    seq2 = np.zeros((nb + 3) // 4 + 8, np.uint8)
+    seq2[: c2.shape[0]] = c2[:, 0] | (c2[:, 1] << 2) | (c2[:, 2] << 4) | (c2[:, 3] << 6)
+    nmask = np.zeros((nb + 7) // 8 + 8, np.uint8)
+    nmask[: (nb + 7) // 8] = np.packbits(isn[: (nb + 7) // 8 * 8], bitorder="little")
     return PackedReads(np.asarray(pos, np.int32), np.asarray(flag, np.uint16), np.asarray(mapq, np.uint8),
                        np.asarray(coff, np.int64), np.asarray(cig, np.uint32), np.asarray(soff, np.int64), seq2,
                        nmask if with_nmask else None)
