@@ -31,11 +31,18 @@ constexpr size_t kBlobFloats = kOffHeadB + 24 + 8;
 // ---- tensor-core section of the blob (fp16 hi/lo split weights in the UMMA K-major no-swizzle layout) ----
 //   B[k/8][n][k%8] halfs, n = unit_block*32 + unit_half*16 + gate*4 + unit_in_half  (TMEM column order: every
 //   16 columns hold i,f,g,o of 4 hidden units, so the epilogue can pipeline 16-column TMEM loads)
-//   layer 0: K = 96  = [x 0..17 | bias column 18 | pad ..31 | h 32..95]; lo part of k < 32 is pre-scaled by 2^10
+//   layer 0: K = 96  = [x 0..17 | bias column 18 | pad ..31 | h 32..95]; lo part of k < 32 is pre-scaled by 2^10, hi part
+//            of k < 32 by 2^8 (the inputs are staged as x 2^-8, see kTcInScale)
 //   layer 1: K = 192 = [l0 out 0..127 | h 128..191]; its bias is added in the epilogue (a bias column would cost a whole
 //            k-block = 2 of 38 MMAs per step on a tensor-bound kernel): float [2 dirs][256] in column order n, at kOffTcBias1
 constexpr int kTcK0 = 96, kTcIn0 = 32, kTcK1 = 192, kTcIn1 = 128;
 constexpr float kTcLoScale = 1024.0f;
+// Layer-0 inputs (counts) are staged as x 2^-8 with a saturating fp16 conversion, so that counts up to 65504 x 2^8 =
+// 16 769 024 keep their fp16 hi/lo split (fp16 itself ends at 65504: a raw count of 65 520 would round to inf and turn the
+// gates into inf - inf = NaN); larger ones saturate at twice that.  The hi weight halves of those columns carry 2^8 back: every
+// product, hence every accumulator, is the unscaled one for integer counts below 65 520.  It limits those weights to
+// |w| < 65504 / 2^8 / (2 log2 e).
+constexpr float kTcInScale = 256.0f;
 constexpr size_t kTcBytes0 = (size_t)kTcK0 * 256 * 2;       // one (hi or lo) array of one direction
 constexpr size_t kTcBytes1 = (size_t)kTcK1 * 256 * 2;
 constexpr size_t kOffTcBytes = ((kBlobFloats * 4 + 255) / 256) * 256;

@@ -9,7 +9,8 @@
 //     a.w  ~=  a_hi.w_hi + a_hi.w_lo + a_lo.w_hi        (dropped term a_lo.w_lo ~ 2^-22 relative)
 // implemented as three K-passes into the same accumulator.  Counts (layer-0 inputs, integers that reach
 // hundreds) use a pre-scaled low part -- (x_hi 2^-10).(w_lo 2^10) -- so the low weight halves stay in the
-// normal fp16 range.  Layer 0's bias rides in the GEMM as a constant-1 input column (its input k-blocks have spare
+// normal fp16 range; they are staged as x 2^-8 against hi weights x 2^8 (kTcInScale), so that counts past fp16's
+// 65504 stay finite.  Layer 0's bias rides in the GEMM as a constant-1 input column (its input k-blocks have spare
 // columns); layer 1 is tensor-bound, so its bias is added in the epilogue instead of costing a k-block.  The activation
 // scales (-log2 e, -2 log2 e) are folded into the packed weights: every exponential is a bare ex2 of an accumulator.
 //
@@ -29,6 +30,8 @@
 // lstm_tc_kernel<0,...> (layer-0 alternative NSNP_L0_VARIANT=0 and the raw-accumulator debug entry), tail_tc_kernel.
 #include <cuda_fp16.h>
 #include <stdlib.h>
+#include <cmath>
+#include <cstdio>
 #include "model_common.cuh"
 #include "tc_ptx.cuh"
 
@@ -38,9 +41,28 @@ namespace {
 constexpr int kRows = 128;             // sites per CTA = TMEM lanes
 constexpr float kLog2e = 1.4426950408889634f;
 
-// hi copy of integer counts scaled by 2^-10 (exact: counts are integers, results stay normal or zero)
+// split8 for the staged layer-0 inputs (x 2^-8): both halves saturate at +-65504 instead of rounding to inf (NaN stays NaN),
+// in the same one conversion per pair.  Exact split for |x| <= 65504 x 2^8; up to twice that the lo half carries the excess
+// over 65504 at fp16 precision, and larger counts saturate at 2 x 65504 x 2^8.
+__device__ __forceinline__ HiLo8 split8_staged(const float (&v)[8]) {
+    uint32_t h[4], l[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const float a = v[2 * i] * (1.0f / kTcInScale), b = v[2 * i + 1] * (1.0f / kTcInScale);
+        asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(h[i]) : "f"(b), "f"(a));
+        const float2 f = __half22float2(*reinterpret_cast<const __half2*>(&h[i]));
+        asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(l[i]) : "f"(b - f.y), "f"(a - f.x));
+    }
+    HiLo8 o;
+    o.hi = make_uint4(h[0], h[1], h[2], h[3]);
+    o.lo = make_uint4(l[0], l[1], l[2], l[3]);
+    return o;
+}
+
+// hi copy of the staged counts (x 2^-8) scaled by 2^-2, i.e. x_hi 2^-10: the operand of the pre-scaled lo weights
+// (exact: counts are integers, the results stay normal or zero)
 __device__ __forceinline__ uint4 scale_hi(const uint4& hi) {
-    const __half2 k = __float2half2_rn(1.0f / kTcLoScale);
+    const __half2 k = __float2half2_rn(kTcInScale / kTcLoScale);
     auto m = [&](uint32_t x) { __half2 t = *reinterpret_cast<__half2*>(&x); return h2_bits(__hmul2(t, k)); };
     return make_uint4(m(hi.x), m(hi.y), m(hi.z), m(hi.w));
 }
@@ -152,14 +174,14 @@ lstm_tc_kernel(const unsigned char* __restrict__ blob, const int32_t* __restrict
                 float v[8];
 #pragma unroll
                 for (int j = 0; j < 8; ++j) v[j] = xval(ch * 8 + j);
-                const HiLo8 s = split8(v);
+                const HiLo8 s = split8_staged(v);
                 reinterpret_cast<uint4*>(sAhi + ch * LBO_A)[row] = s.hi;
                 reinterpret_cast<uint4*>(sAlo + ch * LBO_A)[row] = s.lo;
                 reinterpret_cast<uint4*>(sAsc + ch * LBO_A)[row] = scale_hi(s.hi);
             }
         } else if (sub == NWQ - 1) {
             const float v[8] = {xval(0), xval(1), 1.0f, 0.f, 0.f, 0.f, 0.f, 0.f};  // x16, x17, bias column
-            const HiLo8 s = split8(v);
+            const HiLo8 s = split8_staged(v);
             reinterpret_cast<uint4*>(sAhi + 2 * LBO_A)[row] = s.hi;
             reinterpret_cast<uint4*>(sAlo + 2 * LBO_A)[row] = s.lo;
             reinterpret_cast<uint4*>(sAsc + 2 * LBO_A)[row] = scale_hi(s.hi);
@@ -456,14 +478,14 @@ lstm0_pair2_kernel(const unsigned char* __restrict__ blob, const int32_t* __rest
                 float v[8];
 #pragma unroll
                 for (int j = 0; j < 8; ++j) v[j] = xval(ch * 8 + j);
-                const HiLo8 sp = split8(v);
+                const HiLo8 sp = split8_staged(v);
                 reinterpret_cast<uint4*>(sAhi + ch * LBO_A)[row] = sp.hi;
                 reinterpret_cast<uint4*>(sAlo + ch * LBO_A)[row] = sp.lo;
                 reinterpret_cast<uint4*>(sAsc + ch * LBO_A)[row] = scale_hi(sp.hi);
             }
         } else {
             const float v[8] = {xval(0), xval(1), 1.0f, 0.f, 0.f, 0.f, 0.f, 0.f};  // x16, x17, bias column
-            const HiLo8 sp = split8(v);
+            const HiLo8 sp = split8_staged(v);
             reinterpret_cast<uint4*>(sAhi + 2 * LBO_A)[row] = sp.hi;
             reinterpret_cast<uint4*>(sAlo + 2 * LBO_A)[row] = sp.lo;
             reinterpret_cast<uint4*>(sAsc + 2 * LBO_A)[row] = scale_hi(sp.hi);
@@ -1309,8 +1331,17 @@ int debug_tc_gates(const void* blob, const int32_t* xi, int layer, int dir, int 
     return set_error(NSNP_E_UNSUPPORTED, "debug_tc_gates: layer %d with cta_group %d is not built", layer, cg);
 }
 
-// host: fp16 hi/lo split weights in the [k/8][n][k%8] operand layout
+// host: fp16 hi/lo split weights in the [k/8][n][k%8] operand layout.  A weight whose hi or lo half would not be a finite fp16
+// (with the folded activation scale and, for layer-0 input columns, 2^8) is refused: the kernels would turn it into NaN.
 int pack_tc_weights(const nsnp_model_weights_t* w, unsigned char* blob) {
+    auto refuse = [](const char* what, int layer, int d, int row, int col, float v) {
+        const char* sfx = d ? "_reverse" : "";
+        char name[96];
+        if (col < 0) snprintf(name, sizeof name, "lstm.bias_ih_l%d%s + lstm.bias_hh_l%d%s[%d]", layer, sfx, layer, sfx, row);
+        else snprintf(name, sizeof name, "%s_l%d%s[%d][%d]", what, layer, sfx, row, col);
+        return set_error(NSNP_E_INVALID, "%s = %g is outside the tensor-core weight range (the fp16 halves of w times its activation "
+                         "scale, and times 2^8 for layer-0 inputs and bias, must be finite)", name, v);
+    };
     for (int layer = 0; layer < 2; ++layer) {
         const int K = layer == 0 ? kTcK0 : kTcK1, IN = layer == 0 ? kTcIn0 : kTcIn1, nin = layer == 0 ? kF : 128;
         for (int d = 0; d < 2; ++d) {
@@ -1325,12 +1356,19 @@ int pack_tc_weights(const nsnp_model_weights_t* w, unsigned char* blob) {
                     if (k < nin) v = wih[rowi * nin + k];
                     else if (layer == 0 && k == nin) v = bi[rowi] + bh[rowi];          // layer 0: bias rides as a constant-1 input column
                     else if (k >= IN) v = whh[rowi * kH + (k - IN)];
-                    v *= gate == 2 ? -2.0f * kLog2e : -kLog2e;         // activation scale folded into the weights (see the epilogue)
-                    const float scale = (layer == 0 && k < IN) ? kTcLoScale : 1.0f;
+                    const float raw = v;
+                    v *= gate == 2 ? -2.0f * kLog2e : -kLog2e;         // activation scale folded into the packed weights (see the epilogue)
+                    const bool input = layer == 0 && k < IN;           // layer-0 input column: x is staged as x 2^-8 (kTcInScale)
                     const __half h = __float2half_rn(v);
-                    const __half l = __float2half_rn((v - __half2float(h)) * scale);
+                    const __half hs = input ? __float2half_rn(__half2float(h) * kTcInScale) : h;   // exact unless it overflows
+                    const __half l = __float2half_rn((v - __half2float(h)) * (input ? kTcLoScale : 1.0f));
+                    if (!std::isfinite(__half2float(hs)) || !std::isfinite(__half2float(l))) {
+                        if (k < nin) return refuse("lstm.weight_ih", layer, d, rowi, k, raw);
+                        if (k < IN) return refuse(nullptr, layer, d, rowi, -1, raw);
+                        return refuse("lstm.weight_hh", layer, d, rowi, k - IN, raw);
+                    }
                     const size_t idx = ((size_t)(k >> 3) * 256 + n) * 8 + (k & 7);
-                    hi[idx] = h; lo[idx] = l;
+                    hi[idx] = hs; lo[idx] = l;
                 }
                 if (layer == 1) reinterpret_cast<float*>(blob + kOffTcBias1)[d * 256 + n] = (bi[rowi] + bh[rowi]) * (gate == 2 ? -2.0f * kLog2e : -kLog2e);
             }
@@ -1345,8 +1383,12 @@ int pack_tc_weights(const nsnp_model_weights_t* w, unsigned char* blob) {
             for (int k = 0; k < 128; ++k) {
                 const float v = Wd[(size_t)k * 256 + n];
                 const __half h = __float2half_rn(v);
+                const __half l = __float2half_rn(v - __half2float(h));
+                if (!std::isfinite(__half2float(h)) || !std::isfinite(__half2float(l)))
+                    return set_error(NSNP_E_INVALID, "dense.weight . output_proj.weight (folded)[%d][%d] = %g is outside the tensor-core weight "
+                                     "range (its fp16 halves must be finite)", n, k, v);
                 const size_t idx = ((size_t)(k >> 3) * 256 + n) * 8 + (k & 7);
-                hi[idx] = h; lo[idx] = __float2half_rn(v - __half2float(h));
+                hi[idx] = h; lo[idx] = l;
             }
     }
     return NSNP_OK;
