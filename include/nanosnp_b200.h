@@ -219,7 +219,9 @@ int nsnp_model_f16x1_reset(void* workspace_dev, void* stream);
 int nsnp_model_f16x1_reevaluated(const void* workspace_dev, int64_t* count_out, void* stream);
 
 /* debug aid for the tensor-core path: raw gate pre-activations [m][256] (TMEM column order) of the FIRST step of one
- * (layer, direction); cg = 1 or 2 CTAs per MMA.  Used by the GPU tests to validate operand layouts. */
+ * (layer, direction), computed by the production LSTM kernels (lstm0_pair2_kernel, lstm1_pair2x3_kernel); cg must be 2
+ * (CTA pairs, the only configuration built), anything else returns NSNP_E_UNSUPPORTED.  Used by the GPU tests to validate
+ * operand layouts. */
 int nsnp_debug_lstm_tc_gates(const void* blob_dev, const int32_t* x_i32_dev, int layer, int dir, int cg, const void* h0_dev,
                              float* gates_out_dev, int64_t m, void* stream);
 

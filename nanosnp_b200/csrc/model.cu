@@ -12,7 +12,6 @@
 //                        lanes own hidden-unit pairs, warps own site groups, cell state in registers.
 //   lstm_dir_kernel<L1>  one CTA = 32 sites x one direction, 197 KB of weights resident.
 //   tail_kernel          proj + dense/tanh + heads + softmax on the t=16 state.
-#include <stdlib.h>
 #include "model_common.cuh"
 
 namespace nsnp {
@@ -237,9 +236,9 @@ __global__ void __launch_bounds__(256, 4) tail_kernel(const float* __restrict__ 
 }
 constexpr size_t kTailSmem = (size_t)kTailS * (128 + 256) * sizeof(float);
 
-// sites per LSTM launch: whole waves of 128-site tiles on 148 SMs for both LSTM kernels; bounds the layer-0 output buffer
-// (16.9 KB per site).  NSNP_CHUNK_WAVES (experiments) scales it.
-static const int64_t kChunkSites = [] { const char* v = getenv("NSNP_CHUNK_WAVES"); const int w = v ? atoi(v) : 4; return (int64_t)148 * 128 * (w < 1 ? 1 : w); }();
+// sites per LSTM launch: four whole waves of 128-site tiles on 148 SMs for both LSTM kernels; bounds the layer-0 output
+// buffer (16.9 KB per site)
+constexpr int64_t kChunkSites = (int64_t)148 * 128 * 4;
 
 
 // ---- NSNP_PREC_F16X1: single-pass tensor-core LSTM + re-evaluation of the low-margin sites in NSNP_PREC_F16X3 -------------
@@ -444,11 +443,9 @@ static int model_forward(const void* blob_dev, const int32_t* x_i32_dev, const f
     }
     float* h0 = (float*)((char*)workspace_dev + 256);          // after the header
     const int64_t ch = n < kChunkSites ? n : kChunkSites;
-    static const bool tail_tc_env = [] { const char* v = getenv("NSNP_TAIL_TC"); return !(v && v[0] == '0'); }();
     const bool tc = precision == NSNP_PREC_F16X3 || precision == NSNP_PREC_F16X1;
     // single pass only pays for batches well above the re-evaluation batch; smaller ones run the three-pass path directly
     const bool x1 = precision == NSNP_PREC_F16X1 && n > 4 * (int64_t)kX1Cap;
-    const bool tail_tc = tail_tc_env && tc;
     float* h16 = h0 + ((ch + 127) / 128 * 128) * kT * 128;
     // n_dev (device-side site count) only makes sense for a single chunk; larger batches are chunked by the host count
     for (int64_t off = 0; off < n; off += ch) {
@@ -459,17 +456,15 @@ static int model_forward(const void* blob_dev, const int32_t* x_i32_dev, const f
         dim3 g0((unsigned)((m + Cfg<0>::S - 1) / Cfg<0>::S), 2), g1((unsigned)((m + Cfg<1>::S - 1) / Cfg<1>::S), 2);
         if (tc) {
             if (int e = launch_lstm_tc(blob_dev, xi, xf, h0, h16 + off * 128, m, pos_dev ? pos_dev + off : nullptr, pos_bias, x1 ? 1 : 3, stream)) return e;
-            if (tail_tc) continue;                   // one tensor-core tail launch over all chunks below
-        } else {
-            { ProfScope prof(NSNP_PROF_LSTM0, stream); lstm_dir_kernel<0><<<g0, 256, smem0, stream>>>(blob, xi, xf, nullptr, h0, m, nd); }
-            { ProfScope prof(NSNP_PROF_LSTM1, stream); lstm_dir_kernel<1><<<g1, 256, smem1, stream>>>(blob, nullptr, nullptr, h0, h16, m, nd); }
+            continue;                                // one tensor-core tail launch over all chunks below
         }
+        { ProfScope prof(NSNP_PROF_LSTM0, stream); lstm_dir_kernel<0><<<g0, 256, smem0, stream>>>(blob, xi, xf, nullptr, h0, m, nd); }
+        { ProfScope prof(NSNP_PROF_LSTM1, stream); lstm_dir_kernel<1><<<g1, 256, smem1, stream>>>(blob, nullptr, nullptr, h0, h16, m, nd); }
         ProfScope prof(NSNP_PROF_TAIL, stream);
-        tail_kernel<<<(unsigned)((m + kTailS - 1) / kTailS), 256, kTailSmem, stream>>>(blob, h16 + (tc ? off * 128 : 0), m, nd,
-                                                                                         gt_prob_dev + off * 21, zy_prob_dev + off * 3);
+        tail_kernel<<<(unsigned)((m + kTailS - 1) / kTailS), 256, kTailSmem, stream>>>(blob, h16, m, nd, gt_prob_dev + off * 21, zy_prob_dev + off * 3);
         if (int e = cuda_status("pileup model kernels")) return e;
     }
-    if (tc && tail_tc) {
+    if (tc) {
         ProfScope prof(NSNP_PROF_TAIL, stream);
         if (int e = launch_tail_tc(blob_dev, h16, n, n <= ch ? n_dev : nullptr, gt_prob_dev, zy_prob_dev, stream)) return e;
     }
@@ -484,8 +479,7 @@ static int model_forward(const void* blob_dev, const int32_t* x_i32_dev, const f
         const int32_t* xi_low = pos_dev ? x_i32_dev : (x_i32_dev ? w.x_low : nullptr);
         const float* xf_low = (!pos_dev && x_f32_dev) ? reinterpret_cast<const float*>(w.x_low) : nullptr;
         if (int e = launch_lstm_tc(blob_dev, xi_low, xf_low, h0, h16, kX1Cap, pos_dev ? w.pos_low : nullptr, pos_bias, 3, stream)) return e;
-        if (tail_tc) { if (int e = launch_tail_tc(blob_dev, h16, kX1Cap, nullptr, w.gt_low, w.zy_low, stream)) return e; }
-        else tail_kernel<<<(unsigned)((kX1Cap + kTailS - 1) / kTailS), 256, kTailSmem, stream>>>(blob, h16, kX1Cap, nullptr, w.gt_low, w.zy_low);
+        if (int e = launch_tail_tc(blob_dev, h16, kX1Cap, nullptr, w.gt_low, w.zy_low, stream)) return e;
         x1_scatter_kernel<<<kX1Cap / 8, 256, 0, stream>>>(w.cnt, w.idx, w.gt_low, w.zy_low, gt_prob_dev, zy_prob_dev);
         if (int e = cuda_status("x1 re-evaluation")) return e;
     }

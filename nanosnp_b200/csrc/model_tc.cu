@@ -1,9 +1,9 @@
 // s2 on the 5th-generation tensor cores: the LSTM gate contractions of PileupModel (model.py:18-25,34-35)
 // as tcgen05.mma with TMEM accumulators, hand-written for sm_100a.
 //
-// One CTA = 128 candidate sites x one direction of one layer; per time step
+// One group = 128 candidate sites x one direction of one layer; per time step
 //     gates[128 x 256] = [in_t | h_{t-1}] [128 x K]  .  W^T [K x 256]            (K = 96 layer 0, 192 layer 1)
-// runs as K/16 x 3 tcgen05.mma (M=128 or 256, N=256, K=16, kind::f16, fp32 accumulate in 256 TMEM columns).
+// runs as K/16 x 3 tcgen05.mma (M=256 over a CTA pair, N=256, K=16, kind::f16, fp32 accumulate in 256 TMEM columns).
 //
 // Precision: fp32-grade results from fp16 tensor-core inputs by hi/lo operand splitting,
 //     a.w  ~=  a_hi.w_hi + a_hi.w_lo + a_lo.w_hi        (dropped term a_lo.w_lo ~ 2^-22 relative)
@@ -18,18 +18,16 @@
 // matrices, [k/8][row][k%8]; a thread owns one site row, so it writes whole 16-byte core-matrix rows
 // (conflict free) and the next step's A operand is produced directly by the epilogue.
 //
-// Epilogue (8 warps = 2 per TMEM lane quadrant): tcgen05.ld 32 columns = (i,f,g,o) of 8 hidden units,
-// cell update with one reciprocal per (c', h) pair (5 ex2 + 2 rcp on the MUFU pipe), h -> fp16 hi/lo ->
-// st.shared (next step's operand) and -> global for layer 1.
+// Epilogue (8 warps per group = 2 per TMEM lane quadrant): tcgen05.ld 32 columns = (i,f,g,o) of 8 hidden units,
+// cell update with one reciprocal per (c', h) pair (5 ex2 + 2 rcp on the MUFU pipe, cell_update4), h -> fp16 hi/lo ->
+// st.shared (next step's operand) and -> global.
 //
-// CG = 2 pairs two CTAs (cta_group::2): M = 256, each CTA holds half of W (N/2 rows) -- that is what makes the
+// cta_group::2 pairs two CTAs: M = 256, each CTA holds half of W (N/2 rows) -- that is what makes the
 // layer-1 weights (2 x 96 KB) fit; the leader CTA issues the MMAs, tcgen05.commit multicasts completion.
 //
-// Kernels: lstm0_pair2_kernel (layer 0, production), lstm1_pair2x3_kernel (layer 1, production), lstm1_pair2_kernel
-// (layer 1, single-pass NSNP_PREC_F16X1), lstm_tc_kernel<1,2,4> (layer-1 alternative NSNP_L1_VARIANT=0 and the debug entry),
-// lstm_tc_kernel<0,...> (layer-0 alternative NSNP_L0_VARIANT=0 and the raw-accumulator debug entry), tail_tc_kernel.
+// Kernels: lstm0_pair2_kernel (layer 0), lstm1_pair2x3_kernel (layer 1), lstm1_pair2_kernel (layer 1, single-pass
+// NSNP_PREC_F16X1), tail_tc_kernel.  The first two also serve the raw-accumulator debug entry (kGates instantiations).
 #include <cuda_fp16.h>
-#include <stdlib.h>
 #include <cmath>
 #include <cstdio>
 #include "model_common.cuh"
@@ -67,319 +65,52 @@ __device__ __forceinline__ uint4 scale_hi(const uint4& hi) {
     return make_uint4(m(hi.x), m(hi.y), m(hi.z), m(hi.w));
 }
 
-template <int LAYER> struct TcCfg;
-template <> struct TcCfg<0> { static constexpr int K = kTcK0, IN = kTcIn0, STEPS = 33; };
-template <> struct TcCfg<1> { static constexpr int K = kTcK1, IN = kTcIn1, STEPS = 17; };
+constexpr int kSteps1 = 17;            // layer 1 needs the t = 16 state only: t = 0..16 forward, 32..16 backward
 
-template <int LAYER, int CG> struct TcSmem {
-    static constexpr int K = TcCfg<LAYER>::K;
-    static constexpr int RB = 256 / CG;                        // weight rows held by this CTA
-    static constexpr size_t b_bytes = (size_t)K * RB * 2;      // one of hi / lo
-    static constexpr size_t a_bytes = (size_t)K * kRows * 2;
-    static constexpr size_t sc_bytes = LAYER == 0 ? (size_t)kTcIn0 * kRows * 2 : 0;
-    static constexpr size_t off_bhi = 0, off_blo = b_bytes, off_ahi = 2 * b_bytes, off_alo = off_ahi + a_bytes,
-                            off_asc = off_alo + a_bytes, off_bar = off_asc + sc_bytes, off_bias = off_bar + 64,
-                            total = off_bias + (LAYER == 1 ? 256 * sizeof(float) : 0);
-};
-
-// NWQ warps share each TMEM lane quadrant (each thread = one site row x 64/NWQ hidden units).
-// DEBUG: dump the raw accumulators of the first step and return.
-template <int LAYER, int CG, int NWQ, bool DEBUG>
-__global__ void __launch_bounds__(128 * NWQ + (LAYER == 1 ? 32 : 0), (LAYER == 0 && CG == 2 && NWQ == 2) ? 2 : 1)
-lstm_tc_kernel(const unsigned char* __restrict__ blob, const int32_t* __restrict__ xi, const float* __restrict__ xf,
-               const __half* __restrict__ h0_in, __half* __restrict__ h0_out, float* __restrict__ h16, float* __restrict__ dbg,
-               int64_t n, int dir_override)
-{
-    using C = TcCfg<LAYER>;
-    using S = TcSmem<LAYER, CG>;
-    constexpr int K = C::K, IN = C::IN, RB = S::RB;
-    constexpr int KB = K / 16;                                   // MMA k-blocks per pass
-    constexpr int kThreads = 128 * NWQ + (LAYER == 1 ? 32 : 0);     // layer 1: + one producer warp (bulk copies of the next input)
-    constexpr int kEpiWarps = 4 * NWQ;
-    constexpr int UB = 8 / NWQ;                                  // blocks of 8 hidden units per thread
-    constexpr uint32_t LBO_A = kRows * 16, LBO_B = RB * 16, SBO = 128;
-    extern __shared__ __align__(1024) unsigned char smem[];
-    unsigned char* sBhi = smem + S::off_bhi; unsigned char* sBlo = smem + S::off_blo;
-    unsigned char* sAhi = smem + S::off_ahi; unsigned char* sAlo = smem + S::off_alo; unsigned char* sAsc = smem + S::off_asc;
-    uint64_t* bar = reinterpret_cast<uint64_t*>(smem + S::off_bar);
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + S::off_bar + 32);
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const bool producer = LAYER == 1 && warp == kEpiWarps;       // warp-uniform
-    const int quad = warp & 3, sub = producer ? 0 : (warp >> 2);
-    const int row = quad * 32 + lane;                            // site row = TMEM lane
-    const int dir = DEBUG ? dir_override : (int)blockIdx.y;
-    const uint32_t cta_rank = CG == 2 ? cluster_ctarank() : 0u;
-    const int64_t site0 = (int64_t)blockIdx.x * kRows;
-    int64_t site = site0 + row;
-    const bool live = site < n;
-    if (!live) site = n - 1;                                     // clamp loads, skip stores
-
-    // ---- one-time setup ----
-    if (tid == 0) { mbar_init(bar, 1); mbar_init(bar + 1, 1); mbar_init(bar + 2, 1); fence_mbar_init(); }
-    if (warp == 0) tmem_alloc<CG>(tmem_slot, LAYER == 1 ? 512 : 256);
-    {   // this CTA's weight rows: global [K/8][256][8] halfs -> shared [K/8][RB][8]
-        const uint4* ghi = reinterpret_cast<const uint4*>(blob + tc_off(LAYER, dir, 0));
-        const uint4* glo = reinterpret_cast<const uint4*>(blob + tc_off(LAYER, dir, 1));
-        uint4* dhi = reinterpret_cast<uint4*>(sBhi); uint4* dlo = reinterpret_cast<uint4*>(sBlo);
-        for (int i = tid; i < (K / 8) * RB; i += kThreads) {
-            const int ch = i / RB, r = i - ch * RB;
-            const int g = ch * 256 + (int)cta_rank * RB + r;
-            dhi[i] = __ldg(ghi + g); dlo[i] = __ldg(glo + g);
-        }
-        uint4* a = reinterpret_cast<uint4*>(sAhi);
-        const int n16 = (int)((2 * S::a_bytes + S::sc_bytes) / 16);
-        for (int i = tid; i < n16; i += kThreads) a[i] = make_uint4(0, 0, 0, 0);
+// LSTM cell update of one half block: v holds the accumulator columns i, f, g, o (4 each) of 4 hidden units, c their cell
+// states, h receives sigmoid(o) tanh(c').  kBias: add the gate bias (layer 1; layer 0 carries it in the GEMM).
+// The packed weights carry the activation scales (pack_tc_weights): the accumulators are
+//     xi = -log2e i,  xf = -log2e f,  xg = -2 log2e g,  xo = -log2e o
+// so every exponential is a bare ex2 (5 ex2 + 2 rcp per unit), and the cell state is kept as cs = -2 log2e c, which makes
+// the argument of tanh(c')'s exponential the state itself.
+// Only the upper clamps are needed: a huge argument would give ex2 = +inf and inf * 0 below, a very negative one gives
+// ex2 = 0, which is exact.  With the clamps every (1 + e) factor is <= 2^36 + 1, so the triple product stays below 2^108
+// and its reciprocal stays a normal float.  |c'| <= 33 after 33 steps, so ex2(cs') <= 2^96 needs no clamp; an overflowing
+// (1 + eo) makes rcp return 0 = the exact limit.
+template <bool kBias>
+__device__ __forceinline__ void cell_update4(const uint32_t* v, const float* bias, float* c, float* h) {
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+        float xi_ = __uint_as_float(v[u]), xf_ = __uint_as_float(v[4 + u]), xg_ = __uint_as_float(v[8 + u]), xo_ = __uint_as_float(v[12 + u]);
+        if (kBias) { xi_ += bias[u]; xf_ += bias[4 + u]; xg_ += bias[8 + u]; xo_ += bias[12 + u]; }
+        const float ei = ex2_approx(fminf(xi_, 36.f)), ef = ex2_approx(fminf(xf_, 36.f)), eg = ex2_approx(fminf(xg_, 36.f)), eo = ex2_approx(xo_);
+        const float pi = 1.f + ei, pf = 1.f + ef, pg = 1.f + eg;
+        // cs' = sigmoid(f) cs + K sigmoid(i) tanh(g), K = -2 log2e, over one common denominator
+        const float pig = pi * pg;
+        const float num = fmaf(c[u], pig, fmaf(eg, 2.f * kLog2e, -2.f * kLog2e) * pf);
+        const float cn = num * rcp_approx(pf * pig);
+        c[u] = cn;
+        const float ec = ex2_approx(cn);
+        h[u] = (1.f - ec) * rcp_approx((1.f + eo) * (1.f + ec));
     }
-    __syncthreads();
-    // constant chunk holding the bias column (1.0) -- layer 0: chunk 2 is rewritten every step with x16, x17
-    // layer 1: the (scaled) bias of this direction, added to the accumulators in the epilogue
-    const float* sBias = reinterpret_cast<const float*>(smem + S::off_bias);
-    if (LAYER == 1) {
-        const float* gb = reinterpret_cast<const float*>(blob + kOffTcBias1) + dir * 256;
-        for (int i = tid; i < 256; i += kThreads) reinterpret_cast<float*>(smem + S::off_bias)[i] = __ldg(gb + i);
-        __syncthreads();
-    }
-
-    float c[UB][8];
-#pragma unroll
-    for (int j = 0; j < UB; ++j)
-#pragma unroll
-        for (int u = 0; u < 8; ++u) c[j][u] = 0.f;
-
-    // ---- input staging.  Layer 0: counts row -> registers (prefetch) -> fp16 hi / lo / scaled-hi chunks.
-    //      Layer 1: layer-0 output is already fp16 hi|lo in global memory -> cp.async straight into the operand. ----
-    // layer 0 work split: sub 0 converts x[0..15] (chunks 0,1); the last sub converts x16, x17 + the bias column (chunk 2)
-    int2 xraw[8];                                                    // raw bits: converted only when stored (no stall at the load)
-    auto load_x = [&](int t) {
-        if (LAYER != 0) return;
-        const int2* g = reinterpret_cast<const int2*>(xi ? (const void*)(xi + (site * kT + t) * kF) : (const void*)(xf + (site * kT + t) * kF));
-        if (sub == 0) {
-#pragma unroll
-            for (int j = 0; j < 8; ++j) xraw[j] = ldg_nc_volatile(g + j);
-        } else if (sub == NWQ - 1) {
-            xraw[0] = ldg_nc_volatile(g + 8);
-        }
-    };
-    auto xval = [&](int j) -> float {
-        const int2 p = xraw[j >> 1];
-        const int b = (j & 1) ? p.y : p.x;
-        return xi ? (float)b : __int_as_float(b);
-    };
-    auto store_x = [&]() {
-        if (LAYER != 0) return;
-        if (sub == 0) {
-#pragma unroll
-            for (int ch = 0; ch < 2; ++ch) {
-                float v[8];
-#pragma unroll
-                for (int j = 0; j < 8; ++j) v[j] = xval(ch * 8 + j);
-                const HiLo8 s = split8_staged(v);
-                reinterpret_cast<uint4*>(sAhi + ch * LBO_A)[row] = s.hi;
-                reinterpret_cast<uint4*>(sAlo + ch * LBO_A)[row] = s.lo;
-                reinterpret_cast<uint4*>(sAsc + ch * LBO_A)[row] = scale_hi(s.hi);
-            }
-        } else if (sub == NWQ - 1) {
-            const float v[8] = {xval(0), xval(1), 1.0f, 0.f, 0.f, 0.f, 0.f, 0.f};  // x16, x17, bias column
-            const HiLo8 s = split8_staged(v);
-            reinterpret_cast<uint4*>(sAhi + 2 * LBO_A)[row] = s.hi;
-            reinterpret_cast<uint4*>(sAlo + 2 * LBO_A)[row] = s.lo;
-            reinterpret_cast<uint4*>(sAsc + 2 * LBO_A)[row] = scale_hi(s.hi);
-        }
-    };
-    // layer 1: the layer-0 output of one (tile, t) is stored exactly in operand layout, hi part then lo part, 32 KB each:
-    //     h0[tile][t][hi|lo][chunk 16][row 128][8 halfs]
-    uint64_t* barS = bar + 2;                                        // "input part of A for the next step has landed"
-    constexpr uint32_t kPartBytes = 16u * kRows * 16u;               // 32 KB
-    const bool l2_prefetch = (dir_override >> 8) & 1;
-    const int npass = ((dir_override >> 16) & 3) ? ((dir_override >> 16) & 3) : 3;   // NSNP_PREC_F16X1: the hi.hi pass only
-    // the padding CTA of an odd tile count (clusters come in pairs) re-reads the last real tile: it must not touch memory
-    // past the layer-0 output (found by compute-sanitizer memcheck)
-    const size_t src_tile = min((size_t)blockIdx.x, (size_t)((n + kRows - 1) / kRows - 1));
-    auto stage_h0_bulk = [&](int t) {                                // one thread
-        const __half* src = h0_in + (src_tile * kT + t) * (2 * kPartBytes / 2);
-        mbar_expect_tx(barS, 2 * kPartBytes);
-        bulk_g2s(sAhi, src, kPartBytes, barS);
-        bulk_g2s(sAlo, src + kPartBytes / 2, kPartBytes, barS);
-        // the rows of the step after this one: pull them into L2 now, so that their bulk copy (issued when the operand
-        // buffer is free again, one step from now) pays L2 latency instead of DRAM latency
-        const int tp = dir == 0 ? t + 1 : t - 1;
-        if (l2_prefetch && tp >= 0 && tp < kT) bulk_prefetch_l2(h0_in + (src_tile * kT + tp) * (2 * kPartBytes / 2), 2 * kPartBytes);
-    };
-    constexpr int XB = IN / 16;                                  // k-blocks of the input part; the rest is the h part
-    constexpr uint32_t kTmemCols = LAYER == 1 ? 512 : 256;       // layer 1 double-buffers the accumulator
-    uint64_t* barH = bar;                                        // "gates of this step are complete"
-    uint64_t* barX = bar + 1;                                    // layer 1: "input part of the NEXT step is accumulated"
-    {
-        const int t0 = dir == 0 ? 0 : kT - 1;
-        load_x(t0); store_x();
-        fence_async_smem();
-    }
-
-    tc_fence_before();
-    if (CG == 2) cluster_sync_all(); else __syncthreads();         // barriers initialised, operands zeroed, TMEM allocated
-    tc_fence_after();
-    uint32_t phaseH = 0, phaseX = 0, phaseS = 0;
-    if (LAYER == 1) {
-        if (producer && lane == 0) stage_h0_bulk(dir == 0 ? 0 : kT - 1);
-        mbar_wait(barS, phaseS); phaseS ^= 1;
-        tc_fence_before();
-        if (CG == 2) cluster_sync_all(); else __syncthreads();     // both CTAs of the pair have their first input
-        tc_fence_after();
-    }
-    const uint32_t tmem_base = *tmem_slot;
-    const uint32_t a_hi = smem_u32(sAhi), a_lo = smem_u32(sAlo), a_sc = smem_u32(sAsc), b_hi = smem_u32(sBhi), b_lo = smem_u32(sBlo);
-    constexpr uint32_t idesc = make_idesc(128 * CG, 256);
-    const bool issuer = cta_rank == 0 && tid == 0;
-    // k-blocks [kb0, kb1) x three hi/lo passes into the accumulator at tmem_d
-    auto issue = [&](int kb0, int kb1, uint32_t tmem_d, uint32_t acc) {
-#pragma unroll 1
-        for (int pass = 0; pass < npass; ++pass) {
-#pragma unroll 1
-            for (int kb = kb0; kb < kb1; ++kb) {
-                // pass 0: a_hi.w_hi   pass 1: a_hi.w_lo (layer-0 counts: scaled copy)   pass 2: a_lo.w_hi
-                uint32_t aa = pass == 2 ? a_lo : a_hi;
-                if (LAYER == 0 && pass == 1 && kb < kTcIn0 / 16) aa = a_sc;
-                const uint32_t bb = pass == 1 ? b_lo : b_hi;
-                umma_f16<CG>(tmem_d, make_desc(aa + kb * 2 * LBO_A, LBO_A, SBO), make_desc(bb + kb * 2 * LBO_B, LBO_B, SBO), idesc, acc);
-                acc = 1;
-            }
-        }
-    };
-    if (LAYER == 1) {
-        // software pipeline: the input part of step t+1 (24 of 36 MMAs, independent of h_t) runs on the tensor core
-        // while the epilogue of step t runs on the SM; only the 12 h-part MMAs stay on the per-step critical path
-        if (issuer) { tc_fence_after(); issue(0, XB, tmem_base, 0); umma_commit<CG>(barX); }
-        if (producer) {
-            mbar_wait(barX, phaseX); phaseX ^= 1;
-            if (lane == 0 && C::STEPS > 1 && !DEBUG) stage_h0_bulk(dir == 0 ? 1 : kT - 2);
-        }
-    }
-
-    for (int step = 0; step < C::STEPS; ++step) {
-        const int t = dir == 0 ? step : (kT - 1 - step);
-        const int tn = dir == 0 ? step + 1 : (kT - 2 - step);
-        const bool more = !DEBUG && step + 1 < C::STEPS;
-        const uint32_t acc_cols = LAYER == 1 ? (uint32_t)(step & 1) * 256u : 0u;
-        // ---- operands written by the generic proxy -> visible to the tensor core; TMEM reads of the last step retired ----
-        if (LAYER == 1 && more) { mbar_wait(barS, phaseS); phaseS ^= 1; }      // the input rows of step t+1 have landed (their MMAs are issued below)
-        fence_async_smem();
-        tc_fence_before();
-        if (CG == 2) cluster_sync_exec(); else __syncthreads();
-        if (issuer) {
-            tc_fence_after();
-            if (LAYER == 1) {
-                issue(XB, KB, tmem_base + acc_cols, 1);                       // += W_hh . h_{t-1}
-                umma_commit<CG>(barH);
-                if (more) { issue(0, XB, tmem_base + (acc_cols ^ 256u), 0); umma_commit<CG>(barX); }
-            } else {
-                issue(0, KB, tmem_base, 0);
-                umma_commit<CG>(barH);
-            }
-        }
-        if (producer) {
-            // producer warp: once the input-part MMAs of step t+1 have completed, their operand region takes the rows of
-            // step t+2 (two 32 KB bulk copies); it never touches TMEM and skips the epilogue
-            if (more) {
-                mbar_wait(barX, phaseX); phaseX ^= 1;
-                if (lane == 0 && step + 2 < C::STEPS) stage_h0_bulk(dir == 0 ? step + 2 : kT - 3 - step);
-            }
-            if (DEBUG) break;
-            continue;
-        }
-        if (more) load_x(tn);                                       // global latency hides under the MMAs
-        mbar_wait(barH, phaseH);
-        phaseH ^= 1;
-        tc_fence_after();
-
-        if (DEBUG) {
-#pragma unroll 1
-            for (int jb = sub * UB; jb < sub * UB + UB; ++jb) {
-                float v[32];
-                tmem_ld32(tmem_base + acc_cols + ((uint32_t)(quad * 32) << 16) + jb * 32, v);
-                if (live) for (int i = 0; i < 32; ++i) dbg[(site0 + row) * 256 + jb * 32 + i] = v[i] + (LAYER == 1 ? sBias[jb * 32 + i] : 0.f);
-            }
-            break;
-        }
-
-        // ---- epilogue: UB blocks of 8 hidden units per thread, as 2*UB half blocks of 4 units whose TMEM loads are
-        //      software pipelined (the 16 columns of a half block are i,f,g,o of its 4 units) ----
-        uint32_t vb[2][16];
-        const uint32_t tacc = tmem_base + acc_cols + ((uint32_t)(quad * 32) << 16) + (uint32_t)(sub * UB) * 32u;
-        tmem_ld16_nowait(tacc, vb[0]);
-        tmem_wait_ld();
-        float hv[8];
-#pragma unroll
-        for (int hb = 0; hb < 2 * UB; ++hb) {
-            const int jl = hb >> 1, uh = hb & 1, jb = sub * UB + jl;
-            if (hb + 1 < 2 * UB) tmem_ld16_nowait(tacc + (hb + 1) * 16, vb[(hb + 1) & 1]);
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const uint32_t* v = vb[hb & 1];
-                // The packed weights carry the activation scales (pack_tc_weights): the accumulators are
-                //     xi = -log2e i,  xf = -log2e f,  xg = -2 log2e g,  xo = -log2e o
-                // so every exponential is a bare ex2, and the cell state is kept as cs = -2 log2e c, which makes the
-                // argument of tanh(c')'s exponential the state itself.
-                // Only the upper clamps are needed: a huge argument would give ex2 = +inf and inf * 0 below, a very negative
-                // one gives ex2 = 0, which is exact.  With the clamps every (1 + e) factor is <= 2^36 + 1, so the triple
-                // product stays below 2^108 and its reciprocal stays a normal float.  |c'| <= 33 after 33 steps, so
-                // ex2(cs') <= 2^96 needs no clamp; an overflowing (1 + eo) makes rcp return 0 = the exact limit.
-                const float* bq = sBias + jb * 32 + uh * 16 + u;              // layer 1 only: bias of gate columns i, f, g, o
-                const float bi_ = LAYER == 1 ? bq[0] : 0.f, bf_ = LAYER == 1 ? bq[4] : 0.f, bg_ = LAYER == 1 ? bq[8] : 0.f, bo_ = LAYER == 1 ? bq[12] : 0.f;
-                const float xi_ = fminf(__uint_as_float(v[u]) + bi_, 36.f), xf_ = fminf(__uint_as_float(v[4 + u]) + bf_, 36.f);
-                const float xg_ = fminf(__uint_as_float(v[8 + u]) + bg_, 36.f), xo_ = __uint_as_float(v[12 + u]) + bo_;
-                const float ei = ex2_approx(xi_), ef = ex2_approx(xf_), eg = ex2_approx(xg_), eo = ex2_approx(xo_);
-                const float pi = 1.f + ei, pf = 1.f + ef, pg = 1.f + eg;
-                // cs' = sigmoid(f) cs + K sigmoid(i) tanh(g), K = -2 log2e, over one common denominator
-                const float pig = pi * pg;
-                const float num = fmaf(c[jl][uh * 4 + u], pig, fmaf(eg, 2.f * kLog2e, -2.f * kLog2e) * pf);
-                const float cn = num * rcp_approx(pf * pig);
-                c[jl][uh * 4 + u] = cn;
-                const float ec = ex2_approx(cn);
-                hv[uh * 4 + u] = (1.f - ec) * rcp_approx((1.f + eo) * (1.f + ec));        // sigmoid(o) tanh(c')
-            }
-            if (hb + 1 < 2 * UB) tmem_wait_ld();
-            if (uh == 1) {
-                const HiLo8 s = split8(hv);
-                reinterpret_cast<uint4*>(sAhi + (IN / 8 + jb) * LBO_A)[row] = s.hi;
-                reinterpret_cast<uint4*>(sAlo + (IN / 8 + jb) * LBO_A)[row] = s.lo;
-                if (live) {
-                    if (LAYER == 0) {
-                        // layer-1 operand layout h0[tile][t][hi|lo][chunk][row][8]: a warp writes 512 contiguous bytes
-                        __half* o = h0_out + ((((size_t)blockIdx.x * kT + t) * 2) * 16 + (dir * 8 + jb)) * (kRows * 8) + row * 8;
-                        *reinterpret_cast<uint4*>(o) = s.hi;
-                        *reinterpret_cast<uint4*>(o + 16 * kRows * 8) = s.lo;
-                    } else if (step == C::STEPS - 1) {
-                        float4* o = reinterpret_cast<float4*>(h16 + site * 128 + dir * kH + jb * 8);
-                        o[0] = make_float4(hv[0], hv[1], hv[2], hv[3]); o[1] = make_float4(hv[4], hv[5], hv[6], hv[7]);
-                    }
-                }
-            }
-        }
-        if (more) store_x();
-    }
-
-    // ---- teardown: nobody may still be reading TMEM / the peer's shared memory ----
-    tc_fence_before();
-    if (CG == 2) cluster_sync_all(); else __syncthreads();
-    if (warp == 0) tmem_dealloc<CG>(tmem_base, kTmemCols);
 }
-
 
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
 // ------------------------------------------------------------------------------------------------------------------
-// Layer 0, "two groups per CTA" variant.  A clock64 trace of lstm_tc_kernel<0,2,2> (two independent CTAs per SM) shows a
-// step period of 8100 cycles while the two co-resident CTAs alternate (one waits for its MMAs while the other runs its
-// cell updates) and 10400 once later waves have drifted into phase: then both wait for the tensor pipe together and both
+// Layer 0, two groups per CTA.  A clock64 trace of two independent layer-0 CTAs per SM showed a step period of 8100 cycles
+// while the two co-resident CTAs alternate (one waits for its MMAs while the other runs its cell updates) and 10400 once
+// later waves have drifted into phase: then both wait for the tensor pipe together and both
 // fight for the MUFU pipe together.  Here the alternation is built in: one CTA per SM holds TWO 128-site groups
 // (16 warps, 2 x 256 TMEM columns, one copy of this CTA's half of W), still paired with a second CTA through
 // cta_group::2.  There is no cluster barrier: every warp reports "my part of the epilogue is done" on an mbarrier of the
 // leader CTA (remote arrive from the peer), the leader's thread 0 of the group issues the 18 MMAs and tcgen05.commit
 // multicasts completion to both CTAs.  A second pair of mbarriers passes a token between the two groups so that their
 // MMA bursts strictly alternate.
+// kGates (test aid, nsnp_debug_lstm_tc_gates): every tile runs its first step only, and the clusters of direction gates_dir
+// write the raw accumulators to gates[site][256] (TMEM column order) instead of the cell update.
 constexpr int kP2GroupThreads = 256, kP2Threads = 2 * kP2GroupThreads;
 struct P2Smem {
     static constexpr size_t b_bytes = (size_t)kTcK0 * 128 * 2;                  // this CTA's half of W, one of hi / lo
@@ -389,14 +120,16 @@ struct P2Smem {
     static constexpr size_t off_bhi = 0, off_blo = b_bytes, off_a = 2 * b_bytes, off_bar = off_a + 2 * a_stride, total = off_bar + 128;
 };
 
+template <bool kGates>
 __global__ void __launch_bounds__(kP2Threads, 1)
 lstm0_pair2_kernel(const unsigned char* __restrict__ blob, const int32_t* __restrict__ xi, const float* __restrict__ xf,
-                   __half* __restrict__ h0_out, int64_t n, const int32_t* __restrict__ pos, int64_t pos_bias, int npass)
+                   __half* __restrict__ h0_out, int64_t n, const int32_t* __restrict__ pos, int64_t pos_bias, int npass,
+                   float* __restrict__ gates, int gates_dir)
 {
     // pos != nullptr: xi is the region's count tensor [L][18] and site j's window is its contiguous row span starting at
     // pos[j] - pos_bias (pos_bias = region_start + 16): the [n][33][18] feature tensor is never materialised
     using S = P2Smem;
-    constexpr int K = kTcK0, IN = kTcIn0, KB = K / 16, RB = 128, UB = 4;
+    constexpr int K = kTcK0, IN = kTcIn0, KB = K / 16, RB = 128, UB = 4, kSteps = kGates ? 1 : kT;
     constexpr uint32_t LBO_A = kRows * 16, LBO_B = RB * 16, SBO = 128;
     extern __shared__ __align__(1024) unsigned char smem[];
     const int grp = (int)threadIdx.x / kP2GroupThreads;
@@ -420,7 +153,7 @@ lstm0_pair2_kernel(const unsigned char* __restrict__ blob, const int32_t* __rest
     const int n_quads = (int)((n + 4 * kRows - 1) / (4 * kRows));
     const int q0 = cluster_id >> 1;
     const int my_quads = q0 < n_quads ? (n_quads - q0 + quad_stride - 1) / quad_stride : 0;
-    const int total_g = my_quads * kT;                          // this group's stream of (quad, step) pairs
+    const int total_g = my_quads * kSteps;                      // this group's stream of (quad, step) pairs
     auto tile_of = [&](int qi) -> int64_t { return (int64_t)(q0 + qi * quad_stride) * 4 + (int64_t)cta_rank * 2 + grp; };
 
     if (threadIdx.x == 0) {
@@ -452,7 +185,7 @@ lstm0_pair2_kernel(const unsigned char* __restrict__ blob, const int32_t* __rest
     int2 xraw[8];
     int64_t win0 = 0;                                           // first row of this thread's window in the count tensor
     auto load_x = [&](int gstep) {                              // count row of stream element gstep
-        const int qi = gstep / kT, st = gstep - qi * kT;
+        const int qi = gstep / kSteps, st = gstep - qi * kSteps;
         const int t = dir == 0 ? st : (kT - 1 - st);
         int64_t site = tile_of(qi) * kRows + row;
         if (site >= n) site = n - 1;
@@ -556,23 +289,16 @@ lstm0_pair2_kernel(const unsigned char* __restrict__ blob, const int32_t* __rest
         for (int hb = 0; hb < 2 * UB; ++hb) {
             const int jl = hb >> 1, uh = hb & 1, jb = sub * UB + jl;
             if (hb + 1 < 2 * UB) tmem_ld16_nowait(tacc + (hb + 1) * 16, vb[(hb + 1) & 1]);
+            if (kGates) {
+                if (live && dir == gates_dir) {
 #pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const uint32_t* v = vb[hb & 1];
-                // same cell update as lstm_tc_kernel (scales folded into the weights, scaled cell state)
-                const float xi_ = fminf(__uint_as_float(v[u]), 36.f), xf_ = fminf(__uint_as_float(v[4 + u]), 36.f);
-                const float xg_ = fminf(__uint_as_float(v[8 + u]), 36.f), xo_ = __uint_as_float(v[12 + u]);
-                const float ei = ex2_approx(xi_), ef = ex2_approx(xf_), eg = ex2_approx(xg_), eo = ex2_approx(xo_);
-                const float pi = 1.f + ei, pf = 1.f + ef, pg = 1.f + eg;
-                const float pig = pi * pg;
-                const float num = fmaf(c[jl][uh * 4 + u], pig, fmaf(eg, 2.f * kLog2e, -2.f * kLog2e) * pf);
-                const float cn = num * rcp_approx(pf * pig);
-                c[jl][uh * 4 + u] = cn;
-                const float ec = ex2_approx(cn);
-                hv[uh * 4 + u] = (1.f - ec) * rcp_approx((1.f + eo) * (1.f + ec));
+                    for (int i = 0; i < 16; ++i) gates[(tile_idx * kRows + row) * 256 + sub * UB * 32 + hb * 16 + i] = __uint_as_float(vb[hb & 1][i]);
+                }
+            } else {
+                cell_update4<false>(vb[hb & 1], nullptr, c[jl] + uh * 4, hv + uh * 4);
             }
             if (hb + 1 < 2 * UB) tmem_wait_ld();
-            if (uh == 1) {
+            if (!kGates && uh == 1) {
                 const HiLo8 sp = split8(hv);
                 reinterpret_cast<uint4*>(sAhi + (IN / 8 + jb) * LBO_A)[row] = sp.hi;
                 if (npass == 3) reinterpret_cast<uint4*>(sAlo + (IN / 8 + jb) * LBO_A)[row] = sp.lo;
@@ -584,7 +310,7 @@ lstm0_pair2_kernel(const unsigned char* __restrict__ blob, const int32_t* __rest
             }
         }
         if (more) { store_x(); report_ready(); }
-        if (++step == kT) { step = 0; ++qi; }
+        if (++step == kSteps) { step = 0; ++qi; }
     }
 
     tc_fence_before();
@@ -595,12 +321,11 @@ lstm0_pair2_kernel(const unsigned char* __restrict__ blob, const int32_t* __rest
 // ------------------------------------------------------------------------------------------------------------------
 // Layer 1, single-pass (NSNP_PREC_F16X1) variant with the same two-groups-per-CTA alternation.  With one fp16 pass only the
 // hi halves of W and of the operands are needed: this CTA's half of W (48 KB) + two 128-site operand buffers (48 KB each) fit
-// one SM, and layer 1 stops being a serial "12 MMAs, then the cell update" chain per SM (lstm_tc_kernel<1> with one pass:
+// one SM, and layer 1 stops being a serial "12 MMAs, then the cell update" chain per SM (one group per CTA with one pass:
 // 2,300 + 4,150 cycles per step, MUFU pipe 55 % busy): one group's MMAs run under the other group's cell update.
 // The input rows of a step (layer-0 output, already in operand layout: 32 KB per tile and position) arrive by one bulk copy
 // per group and CTA, issued as soon as the MMAs that read the previous rows have completed; the warp that issued it waits for
-// the copy before it reports the group ready.  Same MMA order and cell arithmetic as lstm_tc_kernel<1> with npass = 1:
-// bit-identical output.
+// the copy before it reports the group ready.
 struct P2Smem1 {
     static constexpr size_t b_bytes = (size_t)kTcK1 * 128 * 2;                  // this CTA's half of W (hi)
     static constexpr size_t a_bytes = (size_t)kTcK1 * kRows * 2;               // one group's operand (hi): 128 input + 64 hidden columns
@@ -611,7 +336,7 @@ __global__ void __launch_bounds__(kP2Threads, 1)
 lstm1_pair2_kernel(const unsigned char* __restrict__ blob, const __half* __restrict__ h0_in, float* __restrict__ h16, int64_t n)
 {
     using S = P2Smem1;
-    constexpr int K = kTcK1, IN = kTcIn1, KB = K / 16, XB = IN / 16, RB = 128, UB = 4, kS = TcCfg<1>::STEPS;
+    constexpr int K = kTcK1, IN = kTcIn1, KB = K / 16, XB = IN / 16, RB = 128, UB = 4, kSteps = kSteps1;
     constexpr uint32_t LBO_A = kRows * 16, LBO_B = RB * 16, SBO = 128;
     constexpr uint32_t kPartBytes = 16u * kRows * 16u;              // 32 KB: the hi half of one (tile, position) of the layer-0 output
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -637,7 +362,7 @@ lstm1_pair2_kernel(const unsigned char* __restrict__ blob, const __half* __restr
     const int64_t last_tile = (n + kRows - 1) / kRows - 1;
     const int q0 = cluster_id >> 1;
     const int my_quads = q0 < n_quads ? (n_quads - q0 + quad_stride - 1) / quad_stride : 0;
-    const int total_g = my_quads * kS;                          // this group's stream of (quad, step) pairs
+    const int total_g = my_quads * kSteps;                      // this group's stream of (quad, step) pairs
     auto tile_of = [&](int qi) -> int64_t { return (int64_t)(q0 + qi * quad_stride) * 4 + (int64_t)cta_rank * 2 + grp; };
 
     if (threadIdx.x == 0) {
@@ -666,7 +391,7 @@ lstm1_pair2_kernel(const unsigned char* __restrict__ blob, const __half* __restr
 
     // input rows of stream element gstep: h0[tile][t][hi][16 chunks][128 rows][8]; a padding tile re-reads the last real one
     auto stage_in = [&](int gstep) {                            // one thread per group and CTA
-        const int qi = gstep / kS, st = gstep - qi * kS;
+        const int qi = gstep / kSteps, st = gstep - qi * kSteps;
         const int t = dir == 0 ? st : (kT - 1 - st);
         const int64_t tile = min(tile_of(qi), last_tile);
         mbar_expect_tx(barIn, kPartBytes);
@@ -731,27 +456,12 @@ lstm1_pair2_kernel(const unsigned char* __restrict__ blob, const __half* __restr
         for (int hb = 0; hb < 2 * UB; ++hb) {
             const int jl = hb >> 1, uh = hb & 1, jb = sub * UB + jl;
             if (hb + 1 < 2 * UB) tmem_ld16_nowait(tacc + (hb + 1) * 16, vb[(hb + 1) & 1]);
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const uint32_t* v = vb[hb & 1];
-                // same cell update as lstm_tc_kernel<1> (scales folded into the weights, scaled cell state, bias in the epilogue)
-                const float* bq = sBias + jb * 32 + uh * 16 + u;
-                const float xi_ = fminf(__uint_as_float(v[u]) + bq[0], 36.f), xf_ = fminf(__uint_as_float(v[4 + u]) + bq[4], 36.f);
-                const float xg_ = fminf(__uint_as_float(v[8 + u]) + bq[8], 36.f), xo_ = __uint_as_float(v[12 + u]) + bq[12];
-                const float ei = ex2_approx(xi_), ef = ex2_approx(xf_), eg = ex2_approx(xg_), eo = ex2_approx(xo_);
-                const float pi = 1.f + ei, pf = 1.f + ef, pg = 1.f + eg;
-                const float pig = pi * pg;
-                const float num = fmaf(c[jl][uh * 4 + u], pig, fmaf(eg, 2.f * kLog2e, -2.f * kLog2e) * pf);
-                const float cn = num * rcp_approx(pf * pig);
-                c[jl][uh * 4 + u] = cn;
-                const float ec = ex2_approx(cn);
-                hv[uh * 4 + u] = (1.f - ec) * rcp_approx((1.f + eo) * (1.f + ec));
-            }
+            cell_update4<true>(vb[hb & 1], sBias + jb * 32 + uh * 16, c[jl] + uh * 4, hv + uh * 4);
             if (hb + 1 < 2 * UB) tmem_wait_ld();
             if (uh == 1) {
                 const HiLo8 sp = split8(hv);
                 reinterpret_cast<uint4*>(sA + (IN / 8 + jb) * LBO_A)[row] = sp.hi;
-                if (live && step == kS - 1) {
+                if (live && step == kSteps - 1) {
                     float4* o = reinterpret_cast<float4*>(h16 + site * 128 + dir * kH + jb * 8);
                     o[0] = make_float4(hv[0], hv[1], hv[2], hv[3]); o[1] = make_float4(hv[4], hv[5], hv[6], hv[7]);
                 }
@@ -761,7 +471,7 @@ lstm1_pair2_kernel(const unsigned char* __restrict__ blob, const __half* __restr
             if (warp == 0) { mbar_wait(barIn, phaseIn); phaseIn ^= 1; }
             report_ready();
         }
-        if (++step == kS) { step = 0; ++qi; }
+        if (++step == kSteps) { step = 0; ++qi; }
     }
 
     tc_fence_before();
@@ -779,9 +489,9 @@ lstm1_pair2_kernel(const unsigned char* __restrict__ blob, const __half* __restr
 //             rows overlaps pass 2 and the 12 h-part MMAs;
 //     lo half (pass 2 reads it): empty once pass 2 of the input part has completed.
 // The full barriers exist per group (a group waits for its own rows only, one phase per step of that group); warp 0 of the
-// group waits for them before it reports the group ready, so barReady covers "both CTAs' input rows have landed".  Same MMA
-// order (input part: 3 passes over kb 0-7, then h part: 3 passes over kb 8-11) and cell arithmetic as lstm_tc_kernel<1>:
-// bit-identical output.
+// group waits for them before it reports the group ready, so barReady covers "both CTAs' input rows have landed".  MMA
+// order: input part (3 passes over kb 0-7), then h part (3 passes over kb 8-11).
+// kGates (test aid, nsnp_debug_lstm_tc_gates): as in lstm0_pair2_kernel, plus the bias.
 constexpr int kP2x3Threads = kP2Threads + 32;                   // + the producer warp
 struct P2Smem1x3 {
     static constexpr size_t b_bytes = (size_t)kTcK1 * 128 * 2;                  // this CTA's half of W, one of hi / lo
@@ -792,11 +502,13 @@ struct P2Smem1x3 {
 };
 static_assert(P2Smem1x3::total <= 232448, "lstm1_pair2x3_kernel: shared memory above the per-block opt-in limit");
 
+template <bool kGates>
 __global__ void __launch_bounds__(kP2x3Threads, 1)
-lstm1_pair2x3_kernel(const unsigned char* __restrict__ blob, const __half* __restrict__ h0_in, float* __restrict__ h16, int64_t n)
+lstm1_pair2x3_kernel(const unsigned char* __restrict__ blob, const __half* __restrict__ h0_in, float* __restrict__ h16, int64_t n,
+                     float* __restrict__ gates, int gates_dir)
 {
     using S = P2Smem1x3;
-    constexpr int K = kTcK1, IN = kTcIn1, KB = K / 16, XB = IN / 16, RB = 128, UB = 4, kS = TcCfg<1>::STEPS;
+    constexpr int K = kTcK1, IN = kTcIn1, KB = K / 16, XB = IN / 16, RB = 128, UB = 4, kSteps = kGates ? 1 : kSteps1;
     constexpr uint32_t LBO_A = kRows * 16, LBO_B = RB * 16, SBO = 128;
     constexpr uint32_t kPartBytes = 16u * kRows * 16u;              // 32 KB: the hi (or lo) half of one (tile, position) of the layer-0 output
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -827,7 +539,7 @@ lstm1_pair2x3_kernel(const unsigned char* __restrict__ blob, const __half* __res
     const int64_t last_tile = (n + kRows - 1) / kRows - 1;
     const int q0 = cluster_id >> 1;
     const int my_quads = q0 < n_quads ? (n_quads - q0 + quad_stride - 1) / quad_stride : 0;
-    const int total_g = my_quads * kS;                          // each group's stream of (quad, step) pairs; bursts alternate g0, g1, g0, ...
+    const int total_g = my_quads * kSteps;                      // each group's stream of (quad, step) pairs; bursts alternate g0, g1, g0, ...
     auto tile_of = [&](int qi, int g) -> int64_t { return (int64_t)(q0 + qi * quad_stride) * 4 + (int64_t)cta_rank * 2 + g; };
 
     if (threadIdx.x == 0) {
@@ -853,7 +565,7 @@ lstm1_pair2x3_kernel(const unsigned char* __restrict__ blob, const __half* __res
     // input rows of burst b (group b & 1, its stream element b >> 1): h0[tile][t][hi|lo][16 chunks][128 rows][8];
     // a padding tile re-reads the last real one
     auto rows_of = [&](int b) -> const __half* {
-        const int gs = b >> 1, qi = gs / kS, st = gs - qi * kS;
+        const int gs = b >> 1, qi = gs / kSteps, st = gs - qi * kSteps;
         const int t = dir == 0 ? st : (kT - 1 - st);
         const int64_t tile = min(tile_of(qi, b & 1), last_tile);
         return h0_in + ((size_t)tile * kT + t) * (size_t)kPartBytes;       // kPartBytes halfs = hi + lo per (tile, t)
@@ -970,28 +682,21 @@ lstm1_pair2x3_kernel(const unsigned char* __restrict__ blob, const __half* __res
             for (int hb = 0; hb < 2 * UB; ++hb) {
                 const int jl = hb >> 1, uh = hb & 1, jb = sub * UB + jl;
                 if (hb + 1 < 2 * UB) tmem_ld16_nowait(tacc + (hb + 1) * 16, vb[(hb + 1) & 1]);
+                if (kGates) {
+                    if (live && dir == gates_dir) {
 #pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    const uint32_t* v = vb[hb & 1];
-                    // same cell update as lstm_tc_kernel<1> (scales folded into the weights, scaled cell state, bias in the epilogue)
-                    const float* bq = sBias + jb * 32 + uh * 16 + u;
-                    const float xi_ = fminf(__uint_as_float(v[u]) + bq[0], 36.f), xf_ = fminf(__uint_as_float(v[4 + u]) + bq[4], 36.f);
-                    const float xg_ = fminf(__uint_as_float(v[8 + u]) + bq[8], 36.f), xo_ = __uint_as_float(v[12 + u]) + bq[12];
-                    const float ei = ex2_approx(xi_), ef = ex2_approx(xf_), eg = ex2_approx(xg_), eo = ex2_approx(xo_);
-                    const float pi = 1.f + ei, pf = 1.f + ef, pg = 1.f + eg;
-                    const float pig = pi * pg;
-                    const float num = fmaf(c[jl][uh * 4 + u], pig, fmaf(eg, 2.f * kLog2e, -2.f * kLog2e) * pf);
-                    const float cn = num * rcp_approx(pf * pig);
-                    c[jl][uh * 4 + u] = cn;
-                    const float ec = ex2_approx(cn);
-                    hv[uh * 4 + u] = (1.f - ec) * rcp_approx((1.f + eo) * (1.f + ec));
+                        for (int i = 0; i < 16; ++i)
+                            gates[site * 256 + sub * UB * 32 + hb * 16 + i] = __uint_as_float(vb[hb & 1][i]) + sBias[sub * UB * 32 + hb * 16 + i];
+                    }
+                } else {
+                    cell_update4<true>(vb[hb & 1], sBias + jb * 32 + uh * 16, c[jl] + uh * 4, hv + uh * 4);
                 }
                 if (hb + 1 < 2 * UB) tmem_wait_ld();
-                if (uh == 1) {
+                if (!kGates && uh == 1) {
                     const HiLo8 sp = split8(hv);
                     reinterpret_cast<uint4*>(sHhi + jb * LBO_A)[row] = sp.hi;
                     reinterpret_cast<uint4*>(sHlo + jb * LBO_A)[row] = sp.lo;
-                    if (live && step == kS - 1) {
+                    if (live && step == kSteps - 1) {
                         float4* o = reinterpret_cast<float4*>(out + jl * 8);
                         o[0] = make_float4(hv[0], hv[1], hv[2], hv[3]); o[1] = make_float4(hv[4], hv[5], hv[6], hv[7]);
                     }
@@ -1001,7 +706,7 @@ lstm1_pair2x3_kernel(const unsigned char* __restrict__ blob, const __half* __res
                 if (warp == 0) wait_input();
                 report_ready();
             }
-            if (++step == kS) { step = 0; ++qi; }
+            if (++step == kSteps) { step = 0; ++qi; }
         }
     }
 
@@ -1029,14 +734,17 @@ int launch_pair2(Kern kern, const char* name, size_t smem_bytes, int threads, in
     return NSNP_OK;
 }
 
-int launch_l0_pair2(const void* blob, const int32_t* xi, const float* xf, void* h0_out, int64_t m, const int32_t* pos, int64_t pos_bias, int npass, cudaStream_t stream) {
+template <bool kGates>
+int launch_l0_pair2(const void* blob, const int32_t* xi, const float* xf, void* h0_out, int64_t m, const int32_t* pos, int64_t pos_bias, int npass,
+                    float* gates, int gates_dir, cudaStream_t stream) {
     static bool attr_done = false;
     if (!attr_done) {
-        if (cudaFuncSetAttribute(lstm0_pair2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P2Smem::total) != cudaSuccess)
+        if (cudaFuncSetAttribute(lstm0_pair2_kernel<kGates>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P2Smem::total) != cudaSuccess)
             return cuda_status("cudaFuncSetAttribute(lstm0_pair2_kernel)");
         attr_done = true;
     }
-    return launch_pair2(lstm0_pair2_kernel, "lstm0_pair2_kernel", P2Smem::total, kP2Threads, m, stream, (const unsigned char*)blob, xi, xf, (__half*)h0_out, m, pos, pos_bias, npass);
+    return launch_pair2(lstm0_pair2_kernel<kGates>, "lstm0_pair2_kernel", P2Smem::total, kP2Threads, m, stream, (const unsigned char*)blob, xi, xf,
+                        (__half*)h0_out, m, pos, pos_bias, npass, gates, gates_dir);
 }
 
 int launch_l1_pair2(const void* blob, const void* h0_in, float* h16, int64_t m, cudaStream_t stream) {
@@ -1049,14 +757,16 @@ int launch_l1_pair2(const void* blob, const void* h0_in, float* h16, int64_t m, 
     return launch_pair2(lstm1_pair2_kernel, "lstm1_pair2_kernel", P2Smem1::total, kP2Threads, m, stream, (const unsigned char*)blob, (const __half*)h0_in, h16, m);
 }
 
-int launch_l1_pair2x3(const void* blob, const void* h0_in, float* h16, int64_t m, cudaStream_t stream) {
+template <bool kGates>
+int launch_l1_pair2x3(const void* blob, const void* h0_in, float* h16, int64_t m, float* gates, int gates_dir, cudaStream_t stream) {
     static bool attr_done = false;
     if (!attr_done) {
-        if (cudaFuncSetAttribute(lstm1_pair2x3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P2Smem1x3::total) != cudaSuccess)
+        if (cudaFuncSetAttribute(lstm1_pair2x3_kernel<kGates>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)P2Smem1x3::total) != cudaSuccess)
             return cuda_status("cudaFuncSetAttribute(lstm1_pair2x3_kernel)");
         attr_done = true;
     }
-    return launch_pair2(lstm1_pair2x3_kernel, "lstm1_pair2x3_kernel", P2Smem1x3::total, kP2x3Threads, m, stream, (const unsigned char*)blob, (const __half*)h0_in, h16, m);
+    return launch_pair2(lstm1_pair2x3_kernel<kGates>, "lstm1_pair2x3_kernel", P2Smem1x3::total, kP2x3Threads, m, stream, (const unsigned char*)blob,
+                        (const __half*)h0_in, h16, m, gates, gates_dir);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -1260,33 +970,6 @@ tail_tc_kernel(const unsigned char* __restrict__ blob, const float* __restrict__
     if (warp == 0) tmem_dealloc<1>(tmem_base, 512);
 }
 
-template <int LAYER, int CG, int NWQ, bool DEBUG>
-int launch_one(const void* blob, const int32_t* xi, const float* xf, const void* h0_in, void* h0_out, float* h16, float* dbg,
-               int64_t m, int dir_override, cudaStream_t stream)
-{
-    using S = TcSmem<LAYER, CG>;
-    auto kern = lstm_tc_kernel<LAYER, CG, NWQ, DEBUG>;
-    static bool attr_done = false;
-    if (!attr_done) {
-        if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)S::total) != cudaSuccess) return cuda_status("cudaFuncSetAttribute(lstm_tc_kernel)");
-        attr_done = true;
-    }
-    unsigned gx = (unsigned)((m + kRows - 1) / kRows);
-    if (CG == 2 && (gx & 1)) ++gx;                               // whole clusters; the padding CTA works on clamped rows
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(gx, DEBUG ? 1 : 2, 1);
-    cfg.blockDim = dim3(128 * NWQ + (LAYER == 1 ? 32 : 0), 1, 1);
-    cfg.dynamicSmemBytes = S::total;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = CG; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    const cudaError_t e = cudaLaunchKernelEx(&cfg, kern, (const unsigned char*)blob, xi, xf, (const __half*)h0_in, (__half*)h0_out, h16, dbg, m, dir_override);
-    if (e != cudaSuccess) return set_error(NSNP_E_CUDA, "lstm_tc_kernel<%d,%d,%d>: %s", LAYER, CG, NWQ, cudaGetErrorString(e));
-    return NSNP_OK;
-}
-
 }  // namespace
 
 int launch_tail_tc(const void* blob, const float* h16, int64_t n_max, const int32_t* n_dev, float* gt, float* zy, cudaStream_t stream) {
@@ -1304,30 +987,20 @@ int launch_tail_tc(const void* blob, const float* h16, int64_t n_max, const int3
 }
 
 int launch_lstm_tc(const void* blob, const int32_t* xi, const float* xf, void* h0, float* h16, int64_t m, const int32_t* pos, int64_t pos_bias, int npass, cudaStream_t stream) {
-    // layer 0: CTA pairs share W (53 KB each) so two CTAs fit per SM and one CTA's MMAs overlap the other's epilogue
+    // layer 0: CTA pairs share W (53 KB each); two alternating 128-site groups per CTA
     {
         ProfScope prof(NSNP_PROF_LSTM0, stream);
-        // default: two alternating groups per CTA (lstm0_pair2_kernel); NSNP_L0_VARIANT=0 selects two independent CTAs per SM
-        static const int variant = [] { const char* v = getenv("NSNP_L0_VARIANT"); return v ? atoi(v) : 1; }();
-        if (pos && variant != 1) return set_error(NSNP_E_UNSUPPORTED, "window reads from the count tensor need the default layer-0 kernel");
-        if (int e = variant == 1 ? launch_l0_pair2(blob, xi, xf, h0, m, pos, pos_bias, npass, stream)
-                                 : launch_one<0, 2, 2, false>(blob, xi, xf, nullptr, h0, nullptr, nullptr, m, npass << 16, stream)) return e;
+        if (int e = launch_l0_pair2<false>(blob, xi, xf, h0, m, pos, pos_bias, npass, nullptr, 0, stream)) return e;
     }
     // layer 1: W only fits split across a CTA pair (2 x 96 KB hi + lo); one CTA per SM
     ProfScope prof(NSNP_PROF_LSTM1, stream);
-    static const int pf = [] { const char* v = getenv("NSNP_L1_PREFETCH"); return v ? atoi(v) : 1; }();
-    // default: two alternating groups per CTA (lstm1_pair2x3_kernel, single pass: lstm1_pair2_kernel);
-    // NSNP_L1_VARIANT=0 keeps the one-group kernel lstm_tc_kernel<1,2,4> (A/B, tests)
-    static const int l1_variant = [] { const char* v = getenv("NSNP_L1_VARIANT"); return v ? atoi(v) : 1; }();
-    if (npass == 1 && l1_variant == 1) return launch_l1_pair2(blob, h0, h16, m, stream);
-    if (npass == 3 && l1_variant == 1) return launch_l1_pair2x3(blob, h0, h16, m, stream);
-    return launch_one<1, 2, 4, false>(blob, nullptr, nullptr, h0, nullptr, h16, nullptr, m, (pf << 8) | (npass << 16), stream);
+    return npass == 1 ? launch_l1_pair2(blob, h0, h16, m, stream) : launch_l1_pair2x3<false>(blob, h0, h16, m, nullptr, 0, stream);
 }
 
 int debug_tc_gates(const void* blob, const int32_t* xi, int layer, int dir, int cg, const void* h0, float* gates_out, int64_t m, cudaStream_t stream) {
-    if (layer == 0 && cg == 1) return launch_one<0, 1, 2, true>(blob, xi, nullptr, nullptr, nullptr, nullptr, gates_out, m, dir, stream);
-    if (layer == 0 && cg == 2) return launch_one<0, 2, 2, true>(blob, xi, nullptr, nullptr, nullptr, nullptr, gates_out, m, dir, stream);
-    if (layer == 1 && cg == 2) return launch_one<1, 2, 4, true>(blob, nullptr, nullptr, h0, nullptr, nullptr, gates_out, m, dir, stream);
+    // the production kernels, first step of every tile only (kGates)
+    if (layer == 0 && cg == 2) return launch_l0_pair2<true>(blob, xi, nullptr, nullptr, m, nullptr, 0, 3, gates_out, dir, stream);
+    if (layer == 1 && cg == 2) return launch_l1_pair2x3<true>(blob, h0, nullptr, m, gates_out, dir, stream);
     return set_error(NSNP_E_UNSUPPORTED, "debug_tc_gates: layer %d with cta_group %d is not built", layer, cg);
 }
 

@@ -6,7 +6,7 @@
 //
 //   read_scan_kernel   one warp per read: reference end, (ref,query) checkpoints every 32 CIGAR ops,
 //                      first/last read index per position tile.
-//   pileup_tile_kernel persistent CTAs, one position tile (T bp) at a time in shared memory:
+//   pileup_tile_kernel persistent CTAs, one position tile (kTile bp) at a time in shared memory:
 //       - one warp per overlapping read, ONE LANE PER CIGAR OP (warp scan gives each op its ref/query start)
 //       - an aligned run (M/=/X) costs two run-boundary increments (depth by prefix sum later) plus a
 //         bit-parallel 2-bit XOR against the reference tile, 16 bases per word: only MISMATCHES touch a
@@ -14,8 +14,7 @@
 //       - a deletion costs two boundary increments ('*'/'#' depth) plus one indel event
 //       - indel events are chained per position (exact grouping for I1/D1 by length / sequence identity)
 //       - epilogue: prefix sums -> 18 channels + AF gate (IEEE double, tensor_maker.cpp:195-228)
-//         -> rows staged in shared memory -> coalesced 16-byte stores of the int32 [T][18] block.
-#include <stdlib.h>
+//         -> rows staged in shared memory -> coalesced 16-byte stores of the int32 [kTile][18] block.
 #include <type_traits>
 #include "common.cuh"
 
@@ -24,6 +23,7 @@ namespace {
 
 constexpr int kCkShift = 5;                 // checkpoint every 32 ops
 constexpr int kReadList = 1024;             // overlapping reads handled per round
+constexpr int kTileShift = 10, kTile = 1 << kTileShift;     // position tile of pileup_tile_kernel (bp)
 
 struct Event {                               // 16 bytes, lives in the per-CTA global slab (L2 resident)
     uint32_t next;                           // previous event anchored at the same position (chain)
@@ -56,7 +56,6 @@ __device__ __forceinline__ uint32_t ld_cigar(const nsnp_reads_t& rd, int64_t i) 
 
 __device__ __forceinline__ bool op_ref(int op) { return op == 0 || op == 2 || op == 3 || op == 7 || op == 8; }
 __device__ __forceinline__ bool op_query(int op) { return op == 0 || op == 1 || op == 4 || op == 7 || op == 8; }
-__device__ __forceinline__ bool op_aligned(int op) { return op == 0 || op == 7 || op == 8; }
 
 __device__ __forceinline__ int warp_incl_scan(int v) {
     const int l = lane_id();
@@ -87,7 +86,7 @@ __device__ __forceinline__ uint32_t spread16(uint32_t x) {     // bit j -> bit 2
 
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) read_scan_kernel(nsnp_reads_t rd, nsnp_params_t prm, int64_t region_start,
-                                                        int64_t region_end, int tile_shift, Workspace ws, int32_t* status)
+                                                        int64_t region_end, Workspace ws, int32_t* status)
 {
     const int lane = lane_id();
     const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -139,7 +138,7 @@ __global__ void __launch_bounds__(256) read_scan_kernel(nsnp_reads_t rd, nsnp_pa
         const int64_t a = pos > region_start ? pos : region_start;
         const int64_t b = R < region_end ? R : region_end;
         if (a < b) {
-            const int t0 = (int)((a - region_start) >> tile_shift), t1 = (int)((b - 1 - region_start) >> tile_shift);
+            const int t0 = (int)((a - region_start) >> kTileShift), t1 = (int)((b - 1 - region_start) >> kTileShift);
             for (int t = t0 + lane; t <= t1; t += 32) { atomicMin(&ws.tile_lo[t], (int)r); atomicMax(&ws.tile_hi[t], (int)r + 1); }
         }
     }
@@ -232,25 +231,24 @@ constexpr uint32_t kBias = 0x40004000u; // packed signed boundary deltas: each u
 constexpr int kMaxOverlap = 16383;       // reads overlapping one tile (keeps the biased halves inside [1, 0x7FFF])
 constexpr uint32_t kNoEvent = 0xFFFFFFFFu;
 
-template <int T>
 struct TileSmem {
     // --- cleared to zero per tile (contiguous) ---
-    uint32_t base[4][T];          // mismatch counters, u16 pairs: [strand*2 + (b>>1)][p], half = b&1
-    uint32_t nn[T];               // read-N bases: fwd | rev << 16
-    uint32_t cnt4[T];             // indel events per class (I i D d), one byte each (exact while <= 255 reads overlap)
-    uint32_t dfast[T];            // deletions of length 1 / 2 per strand, one byte each: D1 D2 d1 d2
-    uint32_t ifast[2][T];         // 1-base insertions per strand, one byte per inserted base: A C G T
+    uint32_t base[4][kTile];          // mismatch counters, u16 pairs: [strand*2 + (b>>1)][p], half = b&1
+    uint32_t nn[kTile];               // read-N bases: fwd | rev << 16
+    uint32_t cnt4[kTile];             // indel events per class (I i D d), one byte each (exact while <= 255 reads overlap)
+    uint32_t dfast[kTile];            // deletions of length 1 / 2 per strand, one byte each: D1 D2 d1 d2
+    uint32_t ifast[2][kTile];         // 1-base insertions per strand, one byte per inserted base: A C G T
     // --- cleared to kBias ---
-    uint32_t ms[T];               // read-span boundary deltas (fwd | rev << 16, biased); after the scan: aligned depth
-    uint32_t ds[T];               // deletion-span boundary deltas;                      after the scan: '*' / '#' depth
+    uint32_t ms[kTile];               // read-span boundary deltas (fwd | rev << 16, biased); after the scan: aligned depth
+    uint32_t ds[kTile];               // deletion-span boundary deltas;                      after the scan: '*' / '#' depth
     // --- cleared to kNoEvent ---
-    uint32_t head[T];             // chain heads of the indel events that have no fast counter
-    uint32_t ref2[T / 16 + 2];    // 2-bit reference tile
-    uint32_t refx[T / 16 + 2];    // 01 at non-ACGT reference positions (forces a "mismatch" event)
-    uint32_t skipcov[T / 32];     // positions inside a reference skip (N op)
+    uint32_t head[kTile];             // chain heads of the indel events that have no fast counter
+    uint32_t ref2[kTile / 16 + 2];    // 2-bit reference tile
+    uint32_t refx[kTile / 16 + 2];    // 01 at non-ACGT reference positions (forces a "mismatch" event)
+    uint32_t skipcov[kTile / 32];     // positions inside a reference skip (N op)
     int32_t  thr_snp[kGateTab], thr_indel[kGateTab];   // smallest count c with (double)c / den >= min_af
-    int32_t  rlist[T];                                  // >= kReadList; reused as per-warp walk lists (T / warps each)
-    int32_t  warp_tot[T / 128][4];
+    int32_t  rlist[kTile];                              // >= kReadList; reused as per-warp walk lists (kTile / warps each)
+    int32_t  warp_tot[kTile / 128][4];
     int32_t  n_rlist, next_task, n_events, tile, ref_has_x, sub_end;
 };
 
@@ -262,189 +260,23 @@ __device__ __forceinline__ ReadMeta load_meta(const nsnp_reads_t& rd, const Work
     return m;
 }
 
+// ------------------------------------------------------------------------------------------------
+// The per-read walk: TWO consecutive CIGAR ops per lane (64 ops per warp iteration, one packed scan for both), 32-bit
+// read-relative sequence coordinates, and per-lane comparison loops with rolling word registers instead of a flattened
+// word list (its scan + binary search + four broadcasts cost more than the lanes it saved: ONT aligned runs average 14
+// bases, i.e. one or two 16-base words).  Runs longer than kSelfWords words -- HiFi-like reads -- finish
+// warp-cooperatively, one word per lane.  In strictly alternating CIGARs (M indel M indel ...) each of the two slots is
+// type-uniform across the warp, so the aligned-run code and the indel code run without divergence.
 // All coordinates are 32-bit: contig positions are int32 (BAM), query offsets are < 2^31; only the absolute base index
 // of the packed sequence array needs 64 bits (added last).
 // kEvOnly: the re-walk of a tile whose indel events overflowed the slab (see pileup_tile_kernel): only the chained events
 // anchored in [elo, ehi) are recorded, no counter is touched.  The first walk passes elo = ts, ehi = te.
-template <int T, bool kEvOnly>
-__device__ __forceinline__ void process_read(TileSmem<T>& sm, const nsnp_reads_t& rd, const Workspace& ws, Event* slab,
-                                             int r, const ReadMeta& meta, int ts, int te, int elo, int ehi, bool deep, int32_t* status)
-{
-    const int lane = lane_id();
-    const int rpos = meta.rpos;
-    const int64_t c0 = meta.c0, c1 = meta.c1;
-    const int64_t sbase = meta.sbase;
-    const int strand = meta.strand;
-    const uint32_t sinc = 1u << (16 * strand);
-    const int nchunks = (int)((c1 - c0 + 31) >> kCkShift);
-    const bool ref_has_x = sm.ref_has_x != 0;                       // tile-uniform
-    const int32_t* ckr = ws.ck_ref + ((c0 >> kCkShift) + r);
-    const int32_t* ckq = ws.ck_q + ((c0 >> kCkShift) + r);
-    // the read's reference span [rpos, rend): two boundary increments per read and tile.  Aligned depth = span depth
-    // minus deletion depth (minus reference skips, which close and reopen the span below): prefix sums in the epilogue.
-    if (!kEvOnly && lane == 0) atomicAdd(&sm.ms[max(rpos - ts, 0)], sinc);
-    if (!kEvOnly && lane == 1 && meta.rend < te) atomicSub(&sm.ms[meta.rend - ts], sinc);
-    // last chunk whose first op starts at or before the window start (32-ary search over the checkpoints)
-    int lo = 0, hi = nchunks;
-    if (rpos < elo) {
-        while (hi - lo > 1) {
-            const int step = (hi - lo + 31) >> 5;
-            const int c = lo + lane * step;
-            const bool le = c < hi && __ldg(ckr + c) <= elo;
-            const int cnt = __popc(__ballot_sync(0xffffffffu, le));      // monotone: lanes 0..cnt-1 are true, cnt >= 1
-            lo = lo + (cnt - 1) * step;
-            hi = min(hi, lo + step);
-        }
-    }
-    const int chunk = lo;
-    int R = __ldg(ckr + chunk), Q = __ldg(ckq + chunk);
-    const uint32_t* seqw = reinterpret_cast<const uint32_t*>(rd.seq2);
-    const uint32_t* nmw = reinterpret_cast<const uint32_t*>(rd.nmask);
-
-    int64_t cgp = c0 + ((int64_t)chunk << kCkShift);
-    int left = (int)(c1 - c0) - (chunk << kCkShift);                             // ops from this chunk to the end of the read
-    uint32_t cg_next = lane < left ? ld_cigar(rd, cgp + lane) : 6u;               // software-pipelined CIGAR loads
-    for (; left > 0 && R <= ehi; left -= 32, cgp += 32) {
-        const uint32_t cg = cg_next;
-        cg_next = (32 + lane < left) ? ld_cigar(rd, cgp + 32 + lane) : 6u;
-        const int op = cg & 15, len = cg >> 4;                          // 6 = pad: consumes nothing
-        const int rl = op_ref(op) ? len : 0, ql = op_query(op) ? len : 0;
-        int ri, qi;
-        if (!__any_sync(0xffffffffu, len >= 2048)) {                    // both prefix sums fit 16 bits: one packed scan
-            const int pk = warp_incl_scan(rl | (ql << 16));
-            ri = pk & 0xFFFF; qi = (int)((uint32_t)pk >> 16);
-        } else {
-            ri = warp_incl_scan(rl); qi = warp_incl_scan(ql);
-        }
-        const int rs = R + ri - rl;                                     // reference start of this lane's op
-        const int qs = Q + qi - ql;                                     // query start (relative to the read)
-        R += __shfl_sync(0xffffffffu, ri, 31);
-        Q += __shfl_sync(0xffffffffu, qi, 31);
-
-        // ---- phase 1: one lane per CIGAR op, straight-line predicated bookkeeping ----
-        const bool aligned = op_aligned(op), isdel = op == 2;
-        const int a = max(rs, ts), b = min(rs + len, te);                               // clipped reference span
-        // indel event anchored at the preceding reference position (appendix A.8 iii/iv); leading ops are never reported.
-        // Totals per class go to byte counters.  The multiplicity of the most frequent IDENTICAL indel (I1/D1) needs
-        // grouping by (length, sequence): the common groups -- deletions of 1 or 2 bases, 1-base insertions of A/C/G/T --
-        // have their own byte counters; everything else is chained per position and grouped exactly in the epilogue.
-        const int anchor = rs - 1;
-        const bool isins = op == 1;
-        const bool ev = (isins || isdel) && len <= NSNP_MAX_INDEL && rs > rpos && anchor >= elo && anchor < ehi;
-        const int64_t gq = sbase + qs;                                   // absolute base index of an inserted sequence
-        const bool ins1 = ev && isins && len == 1 && !deep;
-        // '*' / '#' depth: a counted 1- or 2-base deletion anchored inside the tile is covered by its fast counter (the
-        // epilogue adds D1[p-1] + D2[p-1] + D2[p-2]); every other deletion -- longer, leading, anchored in the previous
-        // tile, or any in a deep tile -- marks its clipped span with two boundary deltas
-        const bool fastdel = ev && isdel && len <= 2 && !deep;
-        if (!kEvOnly && isdel && a < b && !fastdel) {
-            atomicAdd(&sm.ds[a - ts], sinc);
-            if (b < te) atomicSub(&sm.ds[b - ts], sinc);
-        }
-        uint32_t iword = 0, inbit = 0;
-        if (ins1) { iword = __ldg(seqw + (gq >> 4)); if (nmw) inbit = (__ldg(nmw + (gq >> 5)) >> (gq & 31)) & 1u; }   // consumed after phase 2
-        if (ev) {
-            const int cls = (isdel ? 2 : 0) + strand;
-            const int ap = anchor - ts;
-            if (!kEvOnly) atomicAdd(&sm.cnt4[ap], deep ? 1u : 1u << (8 * cls));
-            if (fastdel) {
-                if (!kEvOnly) atomicAdd(&sm.dfast[ap], 1u << (8 * (2 * strand + len - 1)));
-            } else if (!ins1) {
-                const int e = atomicAdd(&sm.n_events, 1);
-                if (e < ws.slab_cap) {
-                    Event evr;
-                    evr.next = atomicExch(&sm.head[ap], (uint32_t)e);
-                    evr.info = (uint32_t)len | ((uint32_t)cls << 8);
-                    evr.seq = (uint64_t)gq;
-                    slab[e] = evr;
-                } else if (kEvOnly) {
-                    dev_fail(status, DEV_E_INDEL_SLAB, sm.tile);
-                }
-            }
-        }
-        if (!kEvOnly && op == 3 && a < b) {                                          // reference skip: covered, nothing counted
-            atomicSub(&sm.ms[a - ts], sinc);                             // close the span over the skip, reopen after it
-            if (b < te) atomicAdd(&sm.ms[b - ts], sinc);
-            for (int p = a; p < b; ++p) atomicOr(&sm.skipcov[(p - ts) >> 5], 1u << ((p - ts) & 31));
-        }
-
-        // ---- phase 2: mismatch detection, one lane per 16-base word of any aligned run of this chunk.  The words of
-        //      all 32 ops are flattened (warp scan) so long runs do not leave the other lanes idle. ----
-        const int n = (!kEvOnly && aligned && a < b) ? (b - a) : 0;
-        const int nw = (n + 15) >> 4;
-        const int winc = warp_incl_scan(nw);
-        const int W = __shfl_sync(0xffffffffu, winc, 31);
-        const int pa = a - ts;
-        const int qa = qs + (a - rs);                                    // query offset of the first clipped base
-        for (int wb = 0; wb < W; wb += 32) {
-            const int f = wb + lane;
-            // owner = number of lanes whose inclusive word count is <= f (binary search across lanes)
-            int j = 0;
-#pragma unroll
-            for (int stp = 16; stp >= 1; stp >>= 1) { const int v = __shfl_sync(0xffffffffu, winc, j + stp - 1); if (v <= f) j += stp; }
-            const int ex_j = __shfl_sync(0xffffffffu, winc - nw, j);
-            const int pa_j = __shfl_sync(0xffffffffu, pa, j);
-            const int n_j = __shfl_sync(0xffffffffu, n, j);
-            const int qa_j = __shfl_sync(0xffffffffu, qa, j);
-            if (f < W) {
-                const int o = (f - ex_j) << 4;
-                const int m = min(16, n_j - o);
-                const int64_t gw = sbase + (qa_j + o);
-                const int pw = pa_j + o;
-                const uint32_t sw = bases16_g(seqw, gw);
-                const uint32_t rw = bases16(sm.ref2, pw);
-                uint32_t x = sw ^ rw;
-                uint32_t mm = (x | (x >> 1)) & 0x55555555u;
-                if (ref_has_x) mm |= bases16(sm.refx, pw);
-                if (m < 16) mm &= (1u << (2 * m)) - 1u;
-                if (nmw) {
-                    uint32_t nb = bits16_g(nmw, gw);
-                    if (m < 16) nb &= (1u << m) - 1u;
-                    if (nb) {
-                        mm &= ~spread16(nb);
-                        while (nb) { const int q = __ffs(nb) - 1; nb &= nb - 1; atomicAdd(&sm.nn[pw + q], sinc); }
-                    }
-                }
-                while (mm) {
-                    const int j2 = __ffs(mm) - 1; mm &= mm - 1;
-                    const int bcode = (sw >> j2) & 3;
-                    atomicAdd(&sm.base[strand * 2 + (bcode >> 1)][pw + (j2 >> 1)], 1u << (16 * (bcode & 1)));
-                }
-            }
-        }
-        if (ins1) {                                                      // 1-base insertion: fast counter, or the chain when the base is N
-            if (!inbit) {
-                if (!kEvOnly) atomicAdd(&sm.ifast[strand][anchor - ts], 1u << (8 * ((iword >> (2 * (int)(gq & 15))) & 3u)));
-            } else {
-                const int e = atomicAdd(&sm.n_events, 1);
-                if (e < ws.slab_cap) {
-                    Event evr;
-                    evr.next = atomicExch(&sm.head[anchor - ts], (uint32_t)e);
-                    evr.info = 1u | ((uint32_t)strand << 8);
-                    evr.seq = (uint64_t)gq;
-                    slab[e] = evr;
-                } else if (kEvOnly) {
-                    dev_fail(status, DEV_E_INDEL_SLAB, sm.tile);
-                }
-            }
-        }
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Variant 2 of the per-read walk: TWO consecutive CIGAR ops per lane (64 ops per warp iteration, one packed scan for
-// both), 32-bit read-relative sequence coordinates, and per-lane comparison loops with rolling word registers instead of
-// the flattened word list (its scan + binary search + four broadcasts cost more than the lanes it saved: ONT aligned runs
-// average 14 bases, i.e. one or two 16-base words).  Runs longer than kSelfWords words -- HiFi-like reads -- finish
-// warp-cooperatively, one word per lane.  In strictly alternating CIGARs (M indel M indel ...) each of the two slots is
-// type-uniform across the warp, so the aligned-run code and the indel code run without divergence.
 constexpr uint32_t kRefOps = 0x18Du;        // M D N = X consume the reference   (bits 0 2 3 7 8)
 constexpr uint32_t kQryOps = 0x193u;        // M I S = X consume the query       (bits 0 1 4 7 8)
 constexpr uint32_t kAlnOps = 0x181u;        // M = X are aligned runs
 constexpr int kSelfWords = 8;
 
-template <int T>
-__device__ __forceinline__ void count_mismatches(TileSmem<T>& sm, uint32_t* __restrict__ bs, const uint32_t* __restrict__ nmr,
+__device__ __forceinline__ void count_mismatches(TileSmem& sm, uint32_t* __restrict__ bs, const uint32_t* __restrict__ nmr,
                                                  uint32_t sw, uint32_t rw, uint32_t xw, int pw, int qb, int m, bool ref_has_x, uint32_t sinc)
 {
     uint32_t x = sw ^ rw;
@@ -462,12 +294,12 @@ __device__ __forceinline__ void count_mismatches(TileSmem<T>& sm, uint32_t* __re
     while (mm) {
         const int j2 = __ffs(mm) - 1; mm &= mm - 1;
         const uint32_t bcode = (sw >> j2) & 3u;
-        atomicAdd(bs + (bcode >> 1) * T + pw + (j2 >> 1), 1u << (16 * (bcode & 1u)));
+        atomicAdd(bs + (bcode >> 1) * kTile + pw + (j2 >> 1), 1u << (16 * (bcode & 1u)));
     }
 }
 
-template <int T, bool kEvOnly>
-__device__ __forceinline__ void process_read2(TileSmem<T>& sm, const nsnp_reads_t& rd, const Workspace& ws, Event* slab,
+template <bool kEvOnly>
+__device__ __forceinline__ void process_read2(TileSmem& sm, const nsnp_reads_t& rd, const Workspace& ws, Event* slab,
                                               int r, const ReadMeta& meta, int ts, int te, int elo, int ehi, bool deep, int32_t* status)
 {
     const int lane = lane_id();
@@ -543,7 +375,7 @@ __device__ __forceinline__ void process_read2(TileSmem<T>& sm, const nsnp_reads_
                 for (int o = 0; o < ne; o += 16) {
                     ++sp; ++rp; ++xp;
                     const uint32_t s_hi = __ldg(sp), r_hi = rp[0], x_hi = ref_has_x ? xp[0] : 0u;
-                    count_mismatches<T>(sm, bs, nmr, __funnelshift_r(s_lo, s_hi, ssh), __funnelshift_r(r_lo, r_hi, rsh),
+                    count_mismatches(sm, bs, nmr, __funnelshift_r(s_lo, s_hi, ssh), __funnelshift_r(r_lo, r_hi, rsh),
                                         __funnelshift_r(x_lo, x_hi, rsh), pa + o, qa + o - sb_lo + nb_lo, n - o, ref_has_x, sinc);
                     s_lo = s_hi; r_lo = r_hi; x_lo = x_hi;
                 }
@@ -554,7 +386,7 @@ __device__ __forceinline__ void process_read2(TileSmem<T>& sm, const nsnp_reads_
                 const int pa_j = __shfl_sync(0xffffffffu, pa, j), n_j = __shfl_sync(0xffffffffu, n, j), qa_j = __shfl_sync(0xffffffffu, qa, j);
                 for (int o = 16 * (kSelfWords + lane); o < n_j; o += 16 * 32) {
                     const int pw = pa_j + o, qw = qa_j + o;
-                    count_mismatches<T>(sm, bs, nmr, bases16_g(seqr, qw), bases16(sm.ref2, pw), ref_has_x ? bases16(sm.refx, pw) : 0u,
+                    count_mismatches(sm, bs, nmr, bases16_g(seqr, qw), bases16(sm.ref2, pw), ref_has_x ? bases16(sm.refx, pw) : 0u,
                                         pw, qw - sb_lo + nb_lo, n_j - o, ref_has_x, sinc);
                 }
             }
@@ -636,16 +468,15 @@ __device__ __forceinline__ int min_count_for_af(double af, int den) {
     return c;
 }
 
-template <int T, int V>
-__global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads_t rd, nsnp_params_t prm, const uint8_t* __restrict__ ref,
+__global__ void __launch_bounds__(kTile / 4, 4096 / kTile) pileup_tile_kernel(nsnp_reads_t rd, nsnp_params_t prm, const uint8_t* __restrict__ ref,
                                                                int64_t region_start, int64_t region_len, int n_tiles,
                                                                Workspace ws, int32_t* __restrict__ counts,
                                                                uint8_t* __restrict__ flags, int32_t* status)
 {
-    constexpr int kThreads = T / 4, kWarps = kThreads / 32;       // one thread packs 4 reference bases
-    static_assert(T >= kReadList, "read list");
+    constexpr int kThreads = kTile / 4, kWarps = kThreads / 32;   // one thread packs 4 reference bases
+    static_assert(kTile >= kReadList, "read list");
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    TileSmem<T>& sm = *reinterpret_cast<TileSmem<T>*>(smem_raw);
+    TileSmem& sm = *reinterpret_cast<TileSmem*>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     Event* slab = ws.slabs + (int64_t)blockIdx.x * ws.slab_cap;
     const uint32_t* seqw = reinterpret_cast<const uint32_t*>(rd.seq2);
@@ -669,19 +500,19 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
         __syncthreads();
         const int tile = sm.tile;
         if (tile >= n_tiles) break;
-        const int ts = (int)region_start + tile * T;                          // contig coordinates are int32 (checked by the host)
-        const int te = (int)min((int64_t)ts + T, region_start + region_len);
+        const int ts = (int)region_start + tile * kTile;                      // contig coordinates are int32 (checked by the host)
+        const int te = (int)min((int64_t)ts + kTile, region_start + region_len);
         const int tn = te - ts;
 
         // ---- clear counters, stage the reference tile ----
         {
             uint4* z = reinterpret_cast<uint4*>(&sm.base[0][0]);
-            for (int i = tid; i < 9 * T / 4; i += kThreads) z[i] = make_uint4(0u, 0u, 0u, 0u);    // base, nn, cnt4, dfast, ifast
+            for (int i = tid; i < 9 * kTile / 4; i += kThreads) z[i] = make_uint4(0u, 0u, 0u, 0u);    // base, nn, cnt4, dfast, ifast
             uint4* zb = reinterpret_cast<uint4*>(&sm.ms[0]);
-            for (int i = tid; i < 2 * T / 4; i += kThreads) zb[i] = make_uint4(kBias, kBias, kBias, kBias);   // ms, ds
+            for (int i = tid; i < 2 * kTile / 4; i += kThreads) zb[i] = make_uint4(kBias, kBias, kBias, kBias);   // ms, ds
             uint4* zh = reinterpret_cast<uint4*>(&sm.head[0]);
-            for (int i = tid; i < T / 4; i += kThreads) zh[i] = make_uint4(kNoEvent, kNoEvent, kNoEvent, kNoEvent);
-            for (int i = tid; i < T / 32; i += kThreads) sm.skipcov[i] = 0u;
+            for (int i = tid; i < kTile / 4; i += kThreads) zh[i] = make_uint4(kNoEvent, kNoEvent, kNoEvent, kNoEvent);
+            for (int i = tid; i < kTile / 32; i += kThreads) sm.skipcov[i] = 0u;
             if (tid == 0) { sm.n_events = 0; }
             // 4 reference bases per thread -> one byte of the 2-bit tile and of the non-ACGT mask
             uint32_t r2 = 0, rx = 0;
@@ -694,7 +525,7 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
             }
             reinterpret_cast<uint8_t*>(sm.ref2)[tid] = (uint8_t)r2;
             reinterpret_cast<uint8_t*>(sm.refx)[tid] = (uint8_t)rx;
-            if (tid < 8) { reinterpret_cast<uint8_t*>(sm.ref2)[T / 4 + tid] = 0; reinterpret_cast<uint8_t*>(sm.refx)[T / 4 + tid] = 0x55; }
+            if (tid < 8) { reinterpret_cast<uint8_t*>(sm.ref2)[kTile / 4 + tid] = 0; reinterpret_cast<uint8_t*>(sm.refx)[kTile / 4 + tid] = 0x55; }
             const int any_x = __syncthreads_or(rx != 0u && tid * 4 < tn);
             if (tid == 0) sm.ref_has_x = any_x;
         }
@@ -733,8 +564,7 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
                     ReadMeta mnext = {};
                     int rn = 0;
                     if (tn < nr) { rn = sm.rlist[tn]; mnext = load_meta(rd, ws, rn); }
-                    if (V == 2) process_read2<T, kEv>(sm, rd, ws, slab, r, meta, ts, te, elo, ehi, deep, status);
-                    else process_read<T, kEv>(sm, rd, ws, slab, r, meta, ts, te, elo, ehi, deep, status);
+                    process_read2<kEv>(sm, rd, ws, slab, r, meta, ts, te, elo, ehi, deep, status);
                     t = tn; r = rn; meta = mnext;
                 }
             }
@@ -745,7 +575,7 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
 
         // ---- prefix sums: biased boundary deltas -> depths (fwd | rev << 16 stays valid: depths are <= kMaxOverlap) ----
         {
-            constexpr int K = T / kThreads;
+            constexpr int K = kTile / kThreads;
             constexpr int kB = (int)(kBias & 0xFFFFu);
             int s0 = 0, s1 = 0, s2 = 0, s3 = 0;          // read span fwd, span rev, del fwd, del rev
 #pragma unroll
@@ -793,9 +623,9 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
                 fsum = sum4(if0) | (sum4(if1) << 8) | ((d0 + d1) << 16) | ((d2 + d3) << 24);      // each <= 255 when not deep
                 fmax = max4(if0) | (max4(if1) << 8) | (max(d0, d1) << 16) | (max(d2, d3) << 24);
             };
-            int32_t* wl = sm.rlist + warp * (T / kWarps);          // the read list is dead here: 128 slots per warp
+            int32_t* wl = sm.rlist + warp * (kTile / kWarps);      // the read list is dead here: 128 slots per warp
             int nlist = 0;
-            for (int sb = warp * 32; sb < T; sb += kThreads) {
+            for (int sb = warp * 32; sb < kTile; sb += kThreads) {
                 const int p = sb + lane;
                 const uint32_t c4 = sm.cnt4[p];                    // zero beyond tn
                 uint32_t fsum, fmax;
@@ -876,14 +706,14 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
             __syncwarp();
         };
         if (sm.n_events <= ws.slab_cap) {
-            indel_channels(0, T);
+            indel_channels(0, kTile);
         } else {
             // The slab held only the first slab_cap chained events of this tile (the rest were not linked).  Re-walk the
             // reads once per anchor sub-range whose events fit the slab, each time rebuilding the chains of that range
             // and reducing them.  cnt4 bounds the chained events per position: in a deep tile it counts exactly them, else
             // its byte sum counts every event.  One position holds at most two events per read (an insertion and a
             // deletion after it), so with <= kMaxOverlap reads a single position always fits.  Tiles that fit never get here.
-            for (int i = tid; i < T; i += kThreads) sm.head[i] = kNoEvent;
+            for (int i = tid; i < kTile; i += kThreads) sm.head[i] = kNoEvent;
             for (int alo = 0; alo < tn;) {
                 __syncthreads();                            // heads reset / previous sub-range reduced, read list free
                 if (tid == 0) {
@@ -975,7 +805,7 @@ __global__ void __launch_bounds__(T / 4, 4096 / T) pileup_tile_kernel(nsnp_reads
 // One block, no per-interval launch: boundary deltas per interval (tile ranges of neighbouring intervals may overlap),
 // then a running sum and an ordered compaction over the tiles.  Count -> counters[6].
 __global__ void __launch_bounds__(1024) tile_list_kernel(Workspace ws, int n_iv, int64_t region_start, int64_t region_len,
-                                                         int tile_shift, int n_tiles)
+                                                         int n_tiles)
 {
     __shared__ int wtot[2][32];
     __shared__ int carry[2];
@@ -986,7 +816,7 @@ __global__ void __launch_bounds__(1024) tile_list_kernel(Workspace ws, int n_iv,
     for (int k = tid; k < n_iv; k += 1024) {
         const int64_t a = max((int64_t)ws.targets[2 * k] - NSNP_FLANK, region_start) - region_start;
         const int64_t b = min((int64_t)ws.targets[2 * k + 1] + NSNP_FLANK, region_start + region_len) - region_start;
-        if (a < b) { atomicAdd(&ws.tile_diff[a >> tile_shift], 1); atomicSub(&ws.tile_diff[((b - 1) >> tile_shift) + 1], 1); }
+        if (a < b) { atomicAdd(&ws.tile_diff[a >> kTileShift], 1); atomicSub(&ws.tile_diff[((b - 1) >> kTileShift) + 1], 1); }
     }
     __syncthreads();
     for (int base = 0; base < n_tiles; base += 1024) {
@@ -1011,13 +841,6 @@ __global__ void __launch_bounds__(1024) tile_list_kernel(Workspace ws, int n_iv,
     if (tid == 0) ws.counters[6] = carry[1];
 }
 
-int tile_shift_for(int64_t region_len) {                                    // T = 1024 (default) or 2048 (NSNP_PILEUP_TILE=2048)
-    (void)region_len;
-    static int shift = 0;
-    if (!shift) { const char* e = getenv("NSNP_PILEUP_TILE"); shift = (e && atoi(e) == 2048) ? 11 : 10; }
-    return shift;
-}
-
 }  // namespace
 }  // namespace nsnp
 
@@ -1028,10 +851,10 @@ static constexpr int kMaxCtas = kNumSMs * 4;
 static constexpr int64_t kSlabCapMax = 32768;
 
 // n_targets < 0: no target areas (the layout of nsnp_pileup_counts)
-static void carve(void* base, int64_t n_reads, int64_t n_cigar, int64_t region_len, int tile_shift, Workspace* w, size_t* total,
+static void carve(void* base, int64_t n_reads, int64_t n_cigar, int64_t region_len, Workspace* w, size_t* total,
                   int64_t n_targets = -1) {
     const int64_t n_slots = (n_cigar >> kCkShift) + n_reads + 2;
-    const int64_t n_tiles = (region_len + (1 << tile_shift) - 1) >> tile_shift;
+    const int64_t n_tiles = (region_len + kTile - 1) >> kTileShift;
     int64_t cap = n_cigar < kSlabCapMax ? n_cigar : kSlabCapMax; if (cap < 64) cap = 64;
     size_t off = 0;
     auto take = [&](size_t bytes) { void* p = base ? (char*)base + off : nullptr; off += align_up(bytes, 256); return p; };
@@ -1080,11 +903,10 @@ static int pileup_counts(const nsnp_reads_t* reads, const uint8_t* ref_dev, int6
     if (nsnp_device_count() == 0) return set_error(NSNP_E_NO_DEVICE, "no CUDA device (there is no CPU fallback)");
     if (region_len == 0) return NSNP_OK;
 
-    const int tile_shift = tile_shift_for(region_len);
     Workspace w; size_t need = 0;
-    carve(workspace_dev, reads->n_reads, reads->n_cigar, region_len, tile_shift, &w, &need, n_targets);
+    carve(workspace_dev, reads->n_reads, reads->n_cigar, region_len, &w, &need, n_targets);
     if (need > workspace_bytes) return set_error(NSNP_E_WORKSPACE, "pileup workspace: need %zu bytes, have %zu", need, workspace_bytes);
-    const int n_tiles = (int)((region_len + (1 << tile_shift) - 1) >> tile_shift);
+    const int n_tiles = (int)((region_len + kTile - 1) >> kTileShift);
 
     cudaMemsetAsync(w.tile_lo, 0x7f, (size_t)(n_tiles + 1) * 4, stream);
     cudaMemsetAsync(w.tile_hi, 0, (size_t)(n_tiles + 1) * 4, stream);
@@ -1094,14 +916,14 @@ static int pileup_counts(const nsnp_reads_t* reads, const uint8_t* ref_dev, int6
         cudaMemsetAsync(flags_dev, 0, (size_t)region_len, stream);
         if (n_targets > 0)
             cudaMemcpyAsync(w.targets, targets, (size_t)n_targets * 8, cudaMemcpyHostToDevice, stream);
-        tile_list_kernel<<<1, 1024, 0, stream>>>(w, (int)n_targets, region_start, region_len, tile_shift, n_tiles);
+        tile_list_kernel<<<1, 1024, 0, stream>>>(w, (int)n_targets, region_start, region_len, n_tiles);
         if (int e = cuda_status("tile_list_kernel")) return e;
     }
     if (reads->n_reads > 0) {
         const int64_t warps = reads->n_reads;
         int blocks = (int)((warps + 7) / 8); if (blocks > kNumSMs * 8) blocks = kNumSMs * 8;
         ProfScope prof(NSNP_PROF_READ_SCAN, stream);
-        read_scan_kernel<<<blocks, 256, 0, stream>>>(*reads, *params, region_start, region_start + region_len, tile_shift, w, status_dev);
+        read_scan_kernel<<<blocks, 256, 0, stream>>>(*reads, *params, region_start, region_start + region_len, w, status_dev);
         if (int e = cuda_status("read_scan_kernel")) return e;
         if (params->max_depth > 0) {
             cap_kernel<<<(int)((reads->n_reads / kCapStride + 8) / 8), 256, 0, stream>>>(*reads, w, params->max_depth);
@@ -1109,27 +931,21 @@ static int pileup_counts(const nsnp_reads_t* reads, const uint8_t* ref_dev, int6
         }
     }
     {
-        static int variant = -1;
-        if (variant < 0) { const char* e = getenv("NSNP_PILEUP_VARIANT"); variant = (e && atoi(e) == 1) ? 1 : 2; }
-        using kern_t = void (*)(nsnp_reads_t, nsnp_params_t, const uint8_t*, int64_t, int64_t, int, Workspace, int32_t*, uint8_t*, int32_t*);
-        const int T = 1 << tile_shift;
-        const kern_t kern = T == 2048 ? (variant == 1 ? (kern_t)pileup_tile_kernel<2048, 1> : (kern_t)pileup_tile_kernel<2048, 2>)
-                                      : (variant == 1 ? (kern_t)pileup_tile_kernel<1024, 1> : (kern_t)pileup_tile_kernel<1024, 2>);
-        const size_t smem = T == 2048 ? sizeof(TileSmem<2048>) : sizeof(TileSmem<1024>);
-        const int threads = T / 4;
+        constexpr size_t smem = sizeof(TileSmem);
+        constexpr int threads = kTile / 4;
         static bool attr_done = false;
         if (!attr_done) {
-            if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+            if (cudaFuncSetAttribute(pileup_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
                 return cuda_status("cudaFuncSetAttribute(pileup_tile_kernel)");
             attr_done = true;
         }
         int occ = 1;
-        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, smem);
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, pileup_tile_kernel, threads, smem);
         if (occ < 1) occ = 1; if (occ > 4) occ = 4;
         int grid = kNumSMs * occ; if (grid > n_tiles) grid = n_tiles; if (grid > kMaxCtas) grid = kMaxCtas;
         ProfScope prof(NSNP_PROF_PILEUP_TILE, stream);
-        kern<<<grid, threads, smem, stream>>>(*reads, *params, ref_dev, region_start, region_len, n_tiles, w,
-                                              counts_dev, flags_dev, status_dev);
+        pileup_tile_kernel<<<grid, threads, smem, stream>>>(*reads, *params, ref_dev, region_start, region_len, n_tiles, w,
+                                                            counts_dev, flags_dev, status_dev);
         if (int e = cuda_status("pileup_tile_kernel")) return e;
     }
     return NSNP_OK;
@@ -1139,7 +955,7 @@ extern "C" {
 
 size_t nsnp_pileup_workspace_bytes(int64_t n_reads, int64_t n_cigar, int64_t region_len) {
     Workspace w; size_t total = 0;
-    carve(nullptr, n_reads < 0 ? 0 : n_reads, n_cigar < 0 ? 0 : n_cigar, region_len < 0 ? 0 : region_len, tile_shift_for(region_len), &w, &total);
+    carve(nullptr, n_reads < 0 ? 0 : n_reads, n_cigar < 0 ? 0 : n_cigar, region_len < 0 ? 0 : region_len, &w, &total);
     return total;
 }
 
@@ -1153,7 +969,7 @@ int nsnp_pileup_counts(const nsnp_reads_t* reads, const uint8_t* ref_dev, int64_
 
 size_t nsnp_pileup_targets_workspace_bytes(int64_t n_reads, int64_t n_cigar, int64_t region_len, int64_t n_targets) {
     Workspace w; size_t total = 0;
-    carve(nullptr, n_reads < 0 ? 0 : n_reads, n_cigar < 0 ? 0 : n_cigar, region_len < 0 ? 0 : region_len, tile_shift_for(region_len), &w, &total,
+    carve(nullptr, n_reads < 0 ? 0 : n_reads, n_cigar < 0 ? 0 : n_cigar, region_len < 0 ? 0 : region_len, &w, &total,
           n_targets < 0 ? 0 : n_targets);
     return total;
 }

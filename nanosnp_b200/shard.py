@@ -79,9 +79,10 @@ def plan_target_units(contigs: Sequence[Tuple[str, int]], targets: Dict[str, np.
     return units, unit_iv
 
 
-def listed_tiles(region: Region, intervals: np.ndarray, tile: int = 1024) -> np.ndarray:
-    """The tiles (indices from region.start) the GPU computes for a unit: those holding any position of [start-16, end+16)
-    of an interval, clipped to the unit's computed span."""
+def listed_tiles(region: Region, intervals: np.ndarray) -> np.ndarray:
+    """The 1024-bp tiles (indices from region.start) the GPU computes for a unit: those holding any position of
+    [start-16, end+16) of an interval, clipped to the unit's computed span."""
+    tile = 1024                                                  # the pileup kernel's position tile (kTile, pileup.cu)
     iv = np.asarray(intervals, np.int64).reshape(-1, 2)
     a = np.maximum(iv[:, 0] - FLANK, region.start) - region.start
     b = np.minimum(iv[:, 1] + FLANK, region.end) - region.start

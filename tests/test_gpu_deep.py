@@ -254,7 +254,7 @@ def deep_inputs(deep_case):
     return {"x": np.ascontiguousarray(x[perm]), "onehot": onehot}
 
 
-@pytest.mark.parametrize("cg", [1, 2])
+@pytest.mark.parametrize("cg", [2])
 def test_layer0_gates_at_deep_counts(weights, golden_weights, deep_inputs, cg):
     """Raw layer-0 accumulators of step 0 (both directions) against float64, relative to sum |x w|: the three passes over the
     input k-blocks are exact enough that dropping the lo pass would exceed the bound by far on the one-hot rows."""

@@ -4,16 +4,12 @@ than 65 535 CIGAR ops.
 
 s1 (counts of covered rows, flags, candidates, windows) is bit-exact against the oracle chain: whole contig with 32- and 16-bit
 CIGAR words, region shards whose boundaries fall inside long ops (directly and through the host read slicing), target
-intervals inside deletion- and skip-only tiles, the depth cap at 8 / 144 / off, and the alternate pileup kernels
-(NSNP_PILEUP_VARIANT=1, NSNP_PILEUP_TILE=2048).  The CLI over plain and indexed BAMs (the long read in CG:B,I) writes the
-oracle's VCF rows.  s4 read matrices with group columns inside long D / N equal the pysam-emulator restatement.
-
-Run as a script (`python test_gpu_long_cigars.py in.npz out.npz`) it is the child of the alternate-kernel test: the pileup
-kernel switches are read once per process.
+intervals inside deletion- and skip-only tiles, and the depth cap at 8 / 144 / off.  The CLI over plain and indexed BAMs (the
+long read in CG:B,I) writes the oracle's VCF rows.  s4 read matrices with group columns inside long D / N equal the
+pysam-emulator restatement.
 """
 import os
 import re
-import subprocess
 import sys
 from pathlib import Path
 
@@ -27,10 +23,6 @@ if str(ROOT) not in sys.path:
 pytestmark = pytest.mark.gpu
 
 CTG = "ctg1"
-
-
-def _fields(rd):
-    return {f: getattr(rd, f) for f in ("pos", "flag", "mapq", "cigar_off", "cigar", "seq_off", "seq2", "nmask")}
 
 
 def _s1(engine, reads, ref, **kw):
@@ -224,60 +216,6 @@ def test_depth_cap_with_ultra_long_reads(fx, orc, oracle_res, max_depth):
     assert np.array_equal(pos + 1, res.positions) and np.array_equal(x, res.windows)
 
 
-def _child(inp, out):
-    """Alternate-kernel child: the fixture from inp, s1 of the whole contig and of two shards into out."""
-    import torch
-    from nanosnp_b200.pipeline import PileupEngine
-    from nanosnp_b200.reads import PackedReads, cigar16
-    z = np.load(inp)
-    ref = z["ref"]
-    res = {}
-    eng = PileupEngine("cuda:0")
-    for tag in ("", "16_"):
-        rd = PackedReads(*[z[tag + f] for f in ("pos", "flag", "mapq", "cigar_off", "cigar", "seq_off", "seq2", "nmask")])
-        if tag:
-            rd = cigar16(rd)
-        ref_t = z[tag + "ref"]
-        pos, x, counts, flags = _s1(eng, rd, ref_t)
-        res[tag + "pos"], res[tag + "x"], res[tag + "counts"], res[tag + "flags"] = pos, x, counts, flags
-    pos, x, counts, flags = _s1(eng, PackedReads(*[z[f] for f in ("pos", "flag", "mapq", "cigar_off", "cigar", "seq_off", "seq2", "nmask")]),
-                                ref, region_start=SHARDS[2] - 16, region_len=SHARDS[3] - SHARDS[2] + 32,
-                                emit_start=SHARDS[2], emit_end=SHARDS[3])
-    res["shard_pos"], res["shard_counts"], res["shard_flags"] = pos, counts, flags
-    torch.cuda.synchronize()
-    np.savez(out, **res)
-
-
-def test_alternate_pileup_kernels(fx, fx16, oracle_res, tmp_path):
-    """NSNP_PILEUP_VARIANT=1, NSNP_PILEUP_TILE=2048 and both: one process each (the switches are read once per process); every
-    output equals the default kernel's and the oracle's."""
-    ref, rd, _ = fx
-    ref16, rd16, _ = fx16
-    inp = tmp_path / "in.npz"
-    np.savez(inp, ref=ref, **_fields(rd), **{"16_" + k: v for k, v in _fields(rd16).items()}, **{"16_ref": ref16})
-    res, res16 = oracle_res("fx"), oracle_res("fx16")
-    outs = {}
-    for name, env in (("default", {}), ("v1", {"NSNP_PILEUP_VARIANT": "1"}), ("t2048", {"NSNP_PILEUP_TILE": "2048"}),
-                      ("v1_t2048", {"NSNP_PILEUP_VARIANT": "1", "NSNP_PILEUP_TILE": "2048"})):
-        e = {k: v for k, v in os.environ.items() if k not in ("NSNP_PILEUP_VARIANT", "NSNP_PILEUP_TILE")}
-        e.update(env, PYTHONPATH=str(ROOT))
-        out = tmp_path / f"{name}.npz"
-        r = subprocess.run([sys.executable, __file__, str(inp), str(out)], env=e, capture_output=True, text=True, timeout=1200)
-        assert r.returncode == 0, (name, r.stderr[-3000:])
-        outs[name] = dict(np.load(out))
-    base = outs["default"]
-    for name, o in outs.items():
-        for k in base:
-            assert np.array_equal(o[k], base[k]), (name, k)
-    for tag, rs in (("", res), ("16_", res16)):
-        _compare(rs, base[tag + "pos"], base[tag + "x"], base[tag + "counts"], base[tag + "flags"])
-        assert np.array_equal(base[tag + "pos"] + 1, rs.positions) and np.array_equal(base[tag + "x"], rs.windows)
-    lo = SHARDS[2] - 16
-    _compare(res, base["shard_pos"], None, base["shard_counts"], base["shard_flags"], lo, SHARDS[3] + 16)
-    want = res.positions - 1
-    assert np.array_equal(base["shard_pos"], want[(want >= SHARDS[2]) & (want < SHARDS[3])])
-
-
 # ------------------------------------------------------------------------------------------------ end to end
 def test_predict_cli_plain_and_indexed_bam(fx, oracle_res, golden_weights, tmp_path):
     """`python -m nanosnp_b200.predict` over a plain and an indexed BAM (the >65 535-op read stored in CG:B,I): the VCF equals the
@@ -437,6 +375,3 @@ def test_hap_group_matrices_inside_long_ops(tmp_path):
             n_checked += 1
     assert n_checked > 80
 
-
-if __name__ == "__main__":
-    _child(sys.argv[1], sys.argv[2])

@@ -36,9 +36,10 @@ def _col_scale():
     return np.where(((n >> 2) & 3) == 2, -2.0, -1.0) * np.log2(np.e)
 
 
-@pytest.mark.parametrize("layer,cg", [(0, 1), (0, 2), (1, 2)])
+@pytest.mark.parametrize("layer,cg", [(0, 2), (1, 2)])
 def test_umma_operand_layout_first_step_gates(weights, golden_weights, small_case, layer, cg):
-    """Raw TMEM accumulators of step 0 == W_ih . in + b (h = 0): validates descriptors, operand layout, hi/lo split."""
+    """Raw TMEM accumulators of step 0 == W_ih . in + b (h = 0), from the production kernels (lstm0_pair2_kernel,
+    lstm1_pair2x3_kernel) through the debug entry: validates descriptors, operand layout, hi/lo split."""
     import torch
     from nanosnp_b200 import _lib
     lib = _lib.load()

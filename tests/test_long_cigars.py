@@ -1,7 +1,7 @@
 """Long-read alignment geometry: kilobase deletions and reference skips, long soft clips and insertions, ultra-long reads.
 
 The seeded fixture built here (`long_fixture`) puts every long-op path of the s1 kernels to work: ops on both sides of the
-packed 16-bit prefix-scan switch (1024 for the default two-ops-per-lane walk, 2048 for variant 1), ops longer than a tile,
+packed 16-bit prefix-scan switch (1024 for the two-ops-per-lane walk, 2048 for a one-op-per-lane walk), ops longer than a tile,
 tiles that lie wholly inside one read's D or N, a stretch covered only by deletions and skips, ultra-long reads whose index
 range makes ordinary low-depth tiles deep, and one read with more than 65 535 CIGAR ops (stored in CG:B,I in a BAM).
 
@@ -198,8 +198,8 @@ def read_geometry(reads):
 
 def window_scans(reads, width, threshold):
     """For every walk window of `width` ops starting at a 32-op checkpoint: (max op length, sum of reference lengths).  The
-    kernel leaves the packed 16-bit scan for a window with any op >= threshold (64 / 1024 for the default walk, 32 / 2048
-    for variant 1)."""
+    kernel leaves the packed 16-bit scan for a window with any op >= threshold (64 / 1024 for the two-ops-per-lane walk,
+    32 / 2048 for a one-op-per-lane walk)."""
     g = read_geometry(reads)
     out = []
     for r in range(reads.n_reads):

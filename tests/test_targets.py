@@ -117,8 +117,8 @@ def test_whole_contig_targets_plan_like_plan_regions():
         assert units == plan_regions(contigs, rl)
 
 
-@pytest.mark.parametrize("tile", [1024, 2048])
-def test_listed_tiles_rule(tile):
+def test_listed_tiles_rule_at_the_pileup_tile():
+    tile = 1024                                                   # the pileup kernel's position tile (kTile, pileup.cu)
     rng = np.random.default_rng(tile)
     for trial in range(40):
         L = int(rng.integers(1, 40_000))
@@ -131,7 +131,7 @@ def test_listed_tiles_rule(tile):
             a, b = max(s - FLANK, rg.start), min(e + FLANK, rg.end)
             near[a - rg.start:b - rg.start] = True
         want = sorted({p // tile for p in np.nonzero(near)[0].tolist()})
-        assert listed_tiles(rg, iv, tile).tolist() == want
+        assert listed_tiles(rg, iv).tolist() == want
 
 
 def test_fetch_ranges_halo_merge():

@@ -1,5 +1,5 @@
 // LSTM cell-update epilogue in isolation: how close to the MUFU rate (16 ops/clk/SM) does the instruction stream of
-// lstm_tc_kernel get without the tensor core, TMEM and barriers, and which ingredient costs what?
+// lstm0_pair2_kernel get without the tensor core, TMEM and barriers, and which ingredient costs what?
 //   MODE 0: math only (gates from registers)      MODE 1: + fp16 hi/lo split and st.shared of h
 //   MODE 2: + fence.proxy.async + __syncthreads per step      MODE 3: + global stores of h (layer-0 output)
 #include <cstdio>
